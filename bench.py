@@ -2,6 +2,7 @@
 """bench.py — frame-pairs/sec of the hot path (match -> gather/back-project -> PnP-RANSAC -> pose).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c1|c2|c2r|c2tc|c3|c4|c5|default]
+                    [--dump-outputs DIR]
 
 Input = one synthetic SEQUENCE of P + 1 frames per GPU (synthetic.make_chain): pair i = (frame i, frame i+1), so a frame's
 descriptors / keypoints / depth map exist (and, in the e2e leg, cross the bus) once.  A step = R passes of the hot path
@@ -394,6 +395,9 @@ def run_ours(args, name):
     launches = ops.launch_count() - l0
     ms = agree_max(ms)
     value = world * P * R * args.steps / (ms / 1e3)
+    # what run_resident handed back in the last timed step (this rank's block of pairs), read before anything else runs
+    outputs = {f: getattr(out, f).cpu().numpy().astype(np.float64)
+               for f in ("T_rel", "rt", "n_matches", "n_corr", "n_inl", "status")} if args.dump_outputs else {}
 
     # ---- matcher variants of the same workload, resident, same pairs, same R (reported beside the headline, never as it):
     # c2: the Hamming distances on the tensor cores (bit-identical matches); c3 / c5: the split-fp16 form of the 3xTF32 GEMM
@@ -503,6 +507,10 @@ def run_ours(args, name):
 
     if rank != 0:
         return None
+    if outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for f, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}_{f}.npy"), a)
 
     # ---- roofline of the dominant kernel, from the per-stage event times of the timed region
     hbm_peak, bf16_peak, peak_kind = peaks()
@@ -754,7 +762,14 @@ def main():
     ap.add_argument("--no-api-rate", action="store_true", help="skip the frames/s measurement through process_frame / the device loop")
     ap.add_argument("--no-variants", action="store_true", help="skip the matcher variants measured beside the headline (hamming_tc, f16x3)")
     ap.add_argument("--allow-no-clocks", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's pipeline outputs (poses, rt, match / correspondence / inlier counts, status; "
+                         "float64) as DIR/<workload>_<name>.npy, so that two builds can be compared on identical seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     rank, _, world = env_rank()
     names = ["c2", "c3"] if args.workload == "default" else [args.workload]     # headline last
     if args.impl == "reference":

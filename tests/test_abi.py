@@ -2,11 +2,14 @@
 import ctypes
 import os
 import re
+import shutil
 import subprocess
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 HEADER = os.path.join(ROOT, "include", "vo_b200.h")
 LIB = os.path.join(ROOT, "visual-odometry-pipeline_b200", "libvo_b200.so")
+# the toolkit's bin/ need not be on PATH; csrc/build.sh finds nvcc under /usr/local/cuda the same way
+CUOBJDUMP = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
 
 
 def _declared():
@@ -46,7 +49,7 @@ def test_binding_prototypes_cover_the_header_and_abi_version():
 
 
 def test_sass_is_sm100a_only():
-    out = subprocess.run(["cuobjdump", "-lelf", LIB], capture_output=True, text=True).stdout
+    out = subprocess.run([CUOBJDUMP, "-lelf", LIB], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 

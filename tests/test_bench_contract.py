@@ -5,15 +5,27 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
              "vs_baseline", "dtype", "data", "config", "e2e", "gpu_launches", "cpu_baseline"}
 
 
+def _bench(*argv, env_extra=None):
+    env = dict(os.environ, **(env_extra or {}))
+    return subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *argv], capture_output=True, text=True, env=env, timeout=600)
+
+
 def _run(env_extra):
-    env = dict(os.environ, **env_extra)
-    return subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
-                           "--cpu-pairs", "2"], capture_output=True, text=True, env=env, timeout=600)
+    return _bench("--impl", "reference", "--steps", "1", "--warmup", "0", "--cpu-pairs", "2", env_extra=env_extra)
+
+
+def _line(r):
+    lines = [l for l in r.stdout.splitlines() if l.startswith("{")]
+    assert len(lines) == 1, r.stdout[-400:]
+    return json.loads(lines[0])
 
 
 def test_reference_arm_prints_one_contract_line():
@@ -37,6 +49,35 @@ def test_reference_arm_prints_one_contract_line():
 def test_reference_arm_is_silent_on_other_ranks():
     r = _run({"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2"})
     assert r.returncode == 0 and not [l for l in r.stdout.splitlines() if l.startswith("{")]
+
+
+def test_bad_arguments_are_refused_before_any_work():
+    for argv in (("--steps", "0"), ("--impl", "reference", "--dump-outputs", "unused")):
+        r = _bench(*argv)
+        assert r.returncode == 2 and "error" in r.stderr, (argv, r.stderr[-400:])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_step_and_repeat_run_to_run(tmp_path):
+    """--dump-outputs writes the timed path's outputs of its last step; two runs with the same arguments write the same
+    arrays, and --steps sets the number of timed steps (one pass per step here: launches scale with it)."""
+    small = ("--workload", "c1", "--pairs", "8", "--passes", "1", "--warmup", "1", "--no-cpu", "--no-api-rate",
+             "--no-variants", "--allow-no-clocks")
+    lines, dumps = [], []
+    for k, steps in enumerate((2, 2, 1)):
+        d = tmp_path / f"run{k}"
+        r = _bench(*small, "--steps", str(steps), "--dump-outputs", str(d))
+        assert r.returncode == 0, r.stderr[-800:]
+        lines.append(_line(r))
+        dumps.append({p.name: np.load(p) for p in sorted(d.iterdir())})
+    names = {f"c1_{f}.npy" for f in ("T_rel", "rt", "n_matches", "n_corr", "n_inl", "status")}
+    assert set(dumps[0]) == names
+    assert dumps[0]["c1_T_rel.npy"].shape == (8, 4, 4) and all(a.dtype == np.float64 for a in dumps[0].values())
+    assert (dumps[0]["c1_status.npy"] == 0).mean() >= 0.5 and (dumps[0]["c1_n_inl.npy"] > 20).any()
+    for dump in dumps[1:]:
+        assert set(dump) == names and all(np.array_equal(dumps[0][n], dump[n]) for n in names)
+    assert [l["steps"] for l in lines] == [2, 2, 1] and all(l["config"]["passes_per_step"] == 1 for l in lines)
+    assert lines[0]["gpu_launches"] == lines[1]["gpu_launches"] == 2 * lines[2]["gpu_launches"] > 0
 
 
 def test_committed_b200_line_has_the_roofline_and_clock_keys():

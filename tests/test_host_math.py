@@ -4,7 +4,6 @@ under a shared hypothesis set" claim; tests/test_gpu_pnp.py is the device half."
 import ctypes
 import os
 import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -13,8 +12,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 @pytest.fixture(scope="module")
-def hm():
-    so = os.path.join(tempfile.gettempdir(), "libvo_host_math_test.so")
+def hm(tmp_path_factory):
+    so = str(tmp_path_factory.mktemp("shim") / "libvo_host_math_test.so")
     subprocess.check_call(["g++", "-O2", "-ffp-contract=off", "-shared", "-fPIC", "-o", so,
                            os.path.join(HERE, "host_math_shim.cpp")])
     lib = ctypes.CDLL(so)

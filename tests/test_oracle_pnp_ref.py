@@ -10,7 +10,6 @@
 import ctypes
 import os
 import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -19,8 +18,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 @pytest.fixture(scope="module")
-def hm():
-    so = os.path.join(tempfile.gettempdir(), "libvo_host_math_ref_test.so")
+def hm(tmp_path_factory):
+    so = str(tmp_path_factory.mktemp("shim") / "libvo_host_math_ref_test.so")
     subprocess.check_call(["g++", "-O2", "-ffp-contract=off", "-shared", "-fPIC", "-o", so, os.path.join(HERE, "host_math_shim.cpp")])
     lib = ctypes.CDLL(so)
     lib.hm_ref_scan.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_double, ctypes.c_void_p, ctypes.c_void_p]

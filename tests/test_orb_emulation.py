@@ -4,7 +4,6 @@ half of the ORB front-end's parity claim; tests/test_gpu_orb_frontend.py is the 
 import ctypes
 import os
 import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -16,8 +15,8 @@ CAP = 8 * 4096
 
 
 @pytest.fixture(scope="module")
-def emu():
-    so = os.path.join(tempfile.gettempdir(), "libvo_orb_emu_test.so")
+def emu(tmp_path_factory):
+    so = str(tmp_path_factory.mktemp("shim") / "libvo_orb_emu_test.so")
     subprocess.check_call(["g++", "-x", "c++", "-std=c++17", "-O2", "-ffp-contract=off", "-pthread", "-Wno-unknown-pragmas",
                            "-Wno-subobject-linkage", "-shared", "-fPIC", '-DVO_HOST_EMU="cuda_emu.h"', "-I", HERE, "-o", so,
                            os.path.join(HERE, "orb_emu_shim.cpp")])

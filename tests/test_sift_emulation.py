@@ -4,7 +4,6 @@ kernels use plain fp32 (device expf / powf / atan polynomial), not OpenCV's oper
 import ctypes
 import os
 import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -17,8 +16,8 @@ CAP = 20000
 
 
 @pytest.fixture(scope="module")
-def emu():
-    so = os.path.join(tempfile.gettempdir(), "libvo_sift_emu_test.so")
+def emu(tmp_path_factory):
+    so = str(tmp_path_factory.mktemp("shim") / "libvo_sift_emu_test.so")
     subprocess.check_call(["g++", "-x", "c++", "-std=c++17", "-O2", "-ffp-contract=off", "-pthread", "-Wno-unknown-pragmas",
                            "-Wno-subobject-linkage", "-shared", "-fPIC", '-DVO_HOST_EMU="cuda_emu.h"', "-I", HERE, "-o", so,
                            os.path.join(HERE, "sift_emu_shim.cpp")])
