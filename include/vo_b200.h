@@ -118,7 +118,9 @@ VO_API int vo_match_u8(vo_ctx *ctx, const uint8_t *ref, const uint8_t *cur, int 
  *   param: ratio (RATIO, RATIO_MUTUAL) or similarity threshold (THRESH*); a double because the
  *   reference compares fp32 distances against Python doubles (0.85, 0.90)
  *   near_tie uint8 [B][n_stride] (may be NULL): 1 where the row's best and second best
- *   are within 1e-5 relative, i.e. the arg-min is not robust to rounding.
+ *   are within 1e-5 relative in distance terms, !(d2 - d1 > 1e-5f * d2) in fp32 with d the
+ *   L2 distance or, for VO_METRIC_COSINE, sqrt(2 - 2 sim), i.e. the arg-min is not robust to
+ *   rounding; 0 on rows without a second best and on rows past n_ref[b].
  */
 VO_API int vo_match_f32(vo_ctx *ctx, const float *ref, const float *cur, int B, int n_stride, int m_stride,
                  const int32_t *n_ref, const int32_t *n_cur, int dim, int metric, int mode, double param,

@@ -117,3 +117,33 @@ def test_device_loop_empty_frames_and_history_limit():
         loop.push(frames[0]["kp"], frames[0]["desc"], frames[0]["depth"], 4)               # history full
     p2, i2 = loop.poses(first=2, count=2)
     assert np.array_equal(p2, poses[2:]) and np.array_equal(i2, info[2:])
+
+
+def test_default_sift_loop_refuses_non_integer_descriptors():
+    """The default SIFT pass (F16X1) is exact for integers in 0..255 only: RootSIFT frames are refused, on the host and as
+    device tensors, and an explicit TF32X3 loop takes them and gives the poses of an explicit TF32X3 loop on the device
+    copies."""
+    import torch
+    import vo_b200  # noqa: F401
+    from vo_b200 import ops, synthetic, synthetic_sequence
+    from vo_b200.device_loop import DeviceLoop
+    frames, _ = synthetic_sequence.make_sequence(n_frames=4, n_kp=400, kind="sift", seed=5)
+    root = [np.sqrt(f["desc"] / np.maximum(f["desc"].sum(1, keepdims=True), 1)).astype(np.float32) for f in frames]
+    loop = DeviceLoop(synthetic.KITTI_K, synthetic.KITTI_WH, 512, kind="sift", n_hyp=128)
+    loop.push(frames[0]["kp"], frames[0]["desc"], frames[0]["depth"], 0)             # integer SIFT: accepted
+    with pytest.raises(ValueError, match="not integers"):
+        loop.push(frames[1]["kp"], root[1], frames[1]["depth"], 1)
+    loop.close()
+    loop = DeviceLoop(synthetic.KITTI_K, synthetic.KITTI_WH, 512, kind="sift", n_hyp=128)
+    with pytest.raises(ValueError, match="not integers"):
+        loop.push(frames[0]["kp"], torch.from_numpy(root[0]).cuda(), frames[0]["depth"], 0)
+    loop.close()
+    out = []
+    for dev in (False, True):
+        loop = DeviceLoop(synthetic.KITTI_K, synthetic.KITTI_WH, 512, kind="sift", n_hyp=128, precision=ops.VO_PREC_TF32X3)
+        for i, f in enumerate(frames):
+            loop.push(f["kp"], torch.from_numpy(root[i]).cuda() if dev else root[i], f["depth"], i)
+        out.append(loop.poses())
+        loop.close()
+    assert np.array_equal(out[0][0], out[1][0]) and np.array_equal(out[0][1], out[1][1])
+    assert (out[0][1][1:, 0] == 0).all(), out[0][1]                                   # the RootSIFT frames do match

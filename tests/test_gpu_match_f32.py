@@ -13,22 +13,6 @@ def _gpu(a):
     return torch.from_numpy(np.ascontiguousarray(a)).cuda()
 
 
-def _precisions():
-    from vo_b200 import ops
-    return [ops.VO_PREC_FP32_SIMT, ops.VO_PREC_TF32X3, ops.VO_PREC_TF32X1]
-
-
-def _check_pairs(orc, ref, cur, got, want, metric):
-    """equal, or each differing row is a near-tie in fp64; returns the number of recorded near-ties."""
-    gd, wd = {int(a): int(b) for a, b in got}, {int(a): int(b) for a, b in want}
-    ties = 0
-    for r in sorted(set(gd) | set(wd)):
-        if gd.get(r) == wd.get(r):
-            continue
-        ties += 1
-    return ties
-
-
 @pytest.mark.parametrize("prec", [2, 1, 0])
 def test_golden_sift_knn_bit_exact(golden, prec):
     from vo_b200 import ops

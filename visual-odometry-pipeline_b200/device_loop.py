@@ -27,9 +27,12 @@ class DeviceLoop:
             norm_or_metric = {"orb": ops.VO_NORM_L2_U8, "sift": ops.VO_METRIC_L2}.get(kind, ops.VO_METRIC_COSINE)
         if mode is None:
             mode = ops.VO_MODE_RATIO_MUTUAL if kind == "r2d2" else ops.VO_MODE_RATIO
+        # one 11-bit pass is exact only on integer-valued descriptors in 0..255 (OpenCV SIFT); unit-norm R2D2 descriptors need
+        # the split passes to reproduce the reference's fp32 `d1 @ d2.t()` decisions (R2D2.py:56-65).  A SIFT loop left on
+        # its default F16X1 pass checks that its descriptors are such integers (push), so RootSIFT or another normalised
+        # variant is refused instead of silently matched with 11-bit products.
+        self._check_int = precision is None and kind == "sift"
         if precision is None:
-            # one 11-bit pass is exact only on integer-valued descriptors (OpenCV SIFT); unit-norm R2D2 descriptors need
-            # the split passes to reproduce the reference's fp32 `d1 @ d2.t()` decisions (R2D2.py:56-65)
             precision = ops.VO_PREC_F16X1 if kind == "sift" else ops.VO_PREC_TF32X3
         if (f32 and norm_or_metric == ops.VO_METRIC_COSINE and precision in (ops.VO_PREC_TF32X1, ops.VO_PREC_F16X1)
                 and not allow_inexact):
@@ -76,6 +79,8 @@ class DeviceLoop:
             desc_a = np.ascontiguousarray(desc, dtype=self.desc_dtype)
         if tuple(desc_a.shape) != (n, self.desc_cols):
             raise ValueError(f"DeviceLoop.push: descriptors {tuple(desc_a.shape)} do not match {n} keypoints x {self.desc_cols}")
+        if self._check_int:
+            self._check_integer_descriptors(desc_a)
         if isinstance(depth, torch.Tensor):
             depth_a = depth.to(torch.float32).contiguous()
         else:
@@ -87,6 +92,22 @@ class DeviceLoop:
             stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
             check(self.ctx.lib.vo_seq_push(self.handle, self._ptr(desc_a), self._ptr(kp_a), n, self._ptr(depth_a),
                                            int(frame_no), stream), "vo_seq_push")
+
+    def _check_integer_descriptors(self, desc):
+        """The default SIFT pass (F16X1) is exact only for integers in 0..255.  Host arrays are checked on every push (no
+        device work).  Device tensors are checked on the first non-empty push only: the check needs a host read, which would stall
+        the otherwise asynchronous loop on every frame, and a device-side producer emits the same kind of descriptor on
+        every frame."""
+        if isinstance(desc, torch.Tensor):
+            if desc.is_cuda and desc.numel():
+                self._check_int = False
+            ok = bool(((desc == desc.round()) & (desc >= 0) & (desc <= 255)).all().item()) if desc.numel() else True
+        else:
+            ok = bool(np.all((desc == np.rint(desc)) & (desc >= 0) & (desc <= 255)))
+        if not ok:
+            raise ValueError("DeviceLoop.push: descriptors are not integers in 0..255 (RootSIFT or another normalised "
+                             "variant?); the default SIFT pass (F16X1, 11-bit operands) is exact only for those.  Create the "
+                             "loop with precision=ops.VO_PREC_TF32X3")
 
     def push_image(self, image, depth, frame_no, nfeatures=500, frontend=None):
         """Extract on the device and push — the image is the only per-frame upload besides the depth map; one host read of
