@@ -27,7 +27,9 @@
 extern "C" {
 #endif
 
-#define VO_ABI_VERSION 2   /* 2: vo_pipeline_args.u8_bytes, vo_pnp_ransac_ref, VO_NORM_HAMMING_TC, vo_orb_debug_read */
+#define VO_ABI_VERSION 3   /* 2: vo_pipeline_args.u8_bytes, vo_pnp_ransac_ref, VO_NORM_HAMMING_TC, vo_orb_debug_read
+                             3: vo_bootstrap, vo_pnp_ransac_ref_batch, VO_ST_BAD_INPUT, the pnp_mode / ref_* fields of
+                                vo_pipeline_args and vo_seq_config */
 
 #if defined(__GNUC__)
 #define VO_API __attribute__((visibility("default")))
@@ -46,6 +48,8 @@ extern "C" {
 #define VO_ST_NO_MODEL 1        /* no hypothesis reached min_inliers (reference: "NO IT IS A BAD PNP") */
 #define VO_ST_TOO_FEW_POINTS 2  /* fewer correspondences than a minimal sample */
 #define VO_ST_KP_OUT_OF_IMAGE 4 /* a matched keypoint truncates outside the depth map (reference: IndexError -> bad PnP) */
+#define VO_ST_BAD_INPUT 8       /* Mode R: n_pts[b] outside [0, cap] or a bootstrap index outside [0, n_pts[b]); set with
+                                   VO_ST_NO_MODEL, and the pair read no point */
 
 /* ---- matcher configuration ---------------------------------------------- */
 /* byte descriptors (ORB) */
@@ -74,6 +78,10 @@ extern "C" {
                                that need the column arg-max run the TF32X1 kernel (identical results there)      */
 #define VO_PREC_F16X3 4     /* tcgen05 kind::f16, x * 2^8 = hi + lo in fp16: the 22 operand bits of TF32X3 at twice the
                                MMA rate; for |x| < 255 (unit-norm R2D2 descriptors, SIFT)                         */
+
+/* PnP estimator of vo_pipeline / vo_seq (pnp_mode) */
+#define VO_PNP_THROUGHPUT 0 /* Mode T: counter-based P3P hypotheses (vo_hypotheses + vo_pnp_ransac)                      */
+#define VO_PNP_REFERENCE 1  /* Mode R: the reference's sampler (vo_bootstrap + vo_pnp_ransac_ref_batch)                 */
 
 typedef struct vo_ctx vo_ctx;
 
@@ -249,6 +257,13 @@ typedef struct vo_pipeline_args {
      * integers 0..255 held as uint8 (OpenCV SIFT: a quarter of the float32 bytes over the bus, same exact results) — with
      * VO_NORM_L2_U8 and a rule without a column side (VO_MODE_RATIO / VO_MODE_NN) only */
     int u8_bytes;
+    /* PnP estimator (VERSION 3; zero = Mode T as before).  VO_PNP_REFERENCE runs match -> gather/back-project ->
+     * vo_bootstrap(n_corr, ref_restarts, cap = n_stride, seed, pair0) -> vo_pnp_ransac_ref_batch(ref_iters, thr_px,
+     * ref_confidence, min_inliers, refine_iters): bit-identical to those calls in sequence; n_hyp is then ignored (any value).
+     * ref_restarts 0 = 3, ref_iters 0 = 100, ref_confidence 0 = 0.99 (the reference's values, :121-126). */
+    int pnp_mode;
+    int ref_restarts, ref_iters;
+    double ref_confidence;
 } vo_pipeline_args;
 
 VO_API int vo_pipeline(vo_ctx *ctx, const vo_pipeline_args *args, void *stream);
@@ -291,6 +306,11 @@ typedef struct vo_seq_config {
     double kf_max_dist;         /* 1.5  (:286) */
     int bad_pnp_limit;          /* 3    (:295) */
     int max_frames;             /* capacity of the pose / info history */
+    /* PnP estimator, as in vo_pipeline_args (VERSION 3; zero = Mode T).  A Mode R loop always launches plainly: VO_SEQ_GRAPH
+     * is ignored for it (its poses are the same either way); n_hyp is then ignored. */
+    int pnp_mode;
+    int ref_restarts, ref_iters;
+    double ref_confidence;
 } vo_seq_config;
 VO_API int vo_seq_create(vo_ctx *ctx, const vo_seq_config *cfg, vo_seq **out);
 VO_API void vo_seq_destroy(vo_seq *seq);
@@ -360,11 +380,46 @@ VO_API int vo_r2d2_extract(vo_r2d2 *net, const uint8_t *rgb, float rel_thr, floa
  * Parity: sampler, scoring and stopping rule reproduce cv2.solvePnPRansac exactly when driven with OpenCV's minimal solver
  * (tests/test_oracle_pnp_ref.py); OpenCV's five-point EPnP itself depends on an arbitrary null-space basis and is matched
  * statistically (csrc/pnp_ref_math.cuh, DESIGN 3.6).
+ * A bootstrap index outside [0, n) gives status VO_ST_NO_MODEL | VO_ST_BAD_INPUT and an identity pose; no point is read.
+ * Fewer than 5 points: VO_ST_NO_MODEL.  hyp_poses rows of iterations without a model are zero.  The sample table is built
+ * on the host and copied from a host array (not for stream capture: use vo_pnp_ransac_ref_batch there).
  */
 VO_API int vo_pnp_ransac_ref(vo_ctx *ctx, const float *xyz, const float *uv, int n, const double *K_h, const int32_t *boot_idx,
                       int restarts, int iters, float thr_px, double confidence, int min_inliers, int refine_iters, double *rt,
                       double *rvec_tvec, double *T_rel, int32_t *n_inl, int32_t *best, uint8_t *inlier_mask, int32_t *hyp_counts,
                       double *hyp_poses, int32_t *status, void *stream);
+
+/*
+ * Bootstrap rows for Mode R: boot int32 [B][restarts][cap], entry (b, r, i) uniform in [0, n_pts[b]) for i < n_pts[b] and -1
+ * for the padding i >= n_pts[b] (every entry of a pair with n_pts[b] <= 0).  Counter-based, keyed by (seed, pair0 + b, r, i):
+ * the pair key, not the batch position, decides a row, so rows do not depend on chunking, lanes or GPU count (as
+ * vo_hypotheses).  The restart enters through a domain constant that keeps the row keys apart from the hypothesis keys of the
+ * same seed and pair.  Range map: multiply-high of a 32-bit draw, ((uint64) u * n) >> 32, relative bias below n / 2^32.
+ * The draw replaces np.random.randint(0, n, n) of :122 by a reproducible stream (a different one: Mode R results with these
+ * rows match the reference statistically, not draw for draw).
+ */
+VO_API int vo_bootstrap(vo_ctx *ctx, const int32_t *n_pts, int B, int restarts, int cap, uint64_t seed, int64_t pair0,
+                 int32_t *boot, void *stream);
+
+/*
+ * Mode R over B frame pairs in one call, everything on the device (no host read of n_pts, no host-staged copy: capture-safe).
+ *   xyz float [B][cap][3], uv float [B][cap][2], n_pts int32 [B] (device); boot_idx int32 [B][restarts][cap]: pair b's rows,
+ *   stride cap, first n_pts[b] entries used (vo_bootstrap, or the caller's own rows); restarts <= 8, iters <= 1024.
+ *   Outputs: the single-pair entry's with a leading [B]: rt [B][12], rvec_tvec [B][6], T_rel [B][16], n_inl [B], best [B][3],
+ *   inlier_mask uint8 [B][cap] (first n_pts[b] entries), hyp_counts int32 [B][restarts][iters],
+ *   hyp_poses double [B][restarts][iters][12], status int32 [B]; all optional except T_rel / status.
+ *   Per pair: n_pts[b] outside [0, cap] or an index of the first n_pts[b] entries of a row outside [0, n_pts[b]) gives
+ *   VO_ST_NO_MODEL | VO_ST_BAD_INPUT, identity pose, zero inliers, a zero mask, and no point of that pair is read; neighbours
+ *   are unaffected.  n_pts[b] < 5: VO_ST_NO_MODEL, as the single-pair entry.  The sample table of each pair is OpenCV's
+ *   (a function of n_pts[b]), built on the device.
+ *   Parity: pair b's outputs are bit-identical to vo_pnp_ransac_ref on xyz[b][:n], uv[b][:n] and boot_idx[b][:, :n], whatever
+ *   its position in the batch and its neighbours (tests/test_gpu_pnp_ref_batch.py).
+ */
+VO_API int vo_pnp_ransac_ref_batch(vo_ctx *ctx, const float *xyz, const float *uv, const int32_t *n_pts, int B, int cap,
+                            const double *K_h, const int32_t *boot_idx, int restarts, int iters, float thr_px, double confidence,
+                            int min_inliers, int refine_iters, double *rt, double *rvec_tvec, double *T_rel, int32_t *n_inl,
+                            int32_t *best, uint8_t *inlier_mask, int32_t *hyp_counts, double *hyp_poses, int32_t *status,
+                            void *stream);
 
 /*
  * ORB front-end (SURVEY 8(f) rank 1): `extract_features_and_desc` of feature_extractors/ORB.py:10-21, i.e.

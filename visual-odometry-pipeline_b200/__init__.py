@@ -9,6 +9,6 @@ from . import _lib  # noqa: F401
 from ._lib import (VO_METRIC_COSINE, VO_METRIC_L2, VO_MODE_MUTUAL, VO_MODE_NN, VO_MODE_RATIO, VO_MODE_RATIO_MUTUAL,  # noqa: F401
                    VO_MODE_THRESH, VO_MODE_THRESH_MUTUAL, VO_NORM_HAMMING, VO_NORM_L2_U8, VO_PREC_F16X1, VO_PREC_F16X3, VO_PREC_FP32_SIMT,
                    VO_PREC_TF32X1, VO_PREC_TF32X3, VO_ST_KP_OUT_OF_IMAGE, VO_ST_NO_MODEL, VO_ST_OK,
-                   VO_ST_TOO_FEW_POINTS, VoError)
+                   VO_ST_TOO_FEW_POINTS, VO_ST_BAD_INPUT, VO_PNP_THROUGHPUT, VO_PNP_REFERENCE, VoError)
 
 __all__ = ["_lib", "ops", "synthetic", "sequence"]

@@ -12,14 +12,15 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("VO_B200_LIB") or os.path.join(_HERE, "libvo_b200.so")   # (override: A/B runs of two builds)
 
 # ---- constants mirrored from include/vo_b200.h ---------------------------------------------
-VO_ABI_VERSION = 2
+VO_ABI_VERSION = 3
 VO_OK, VO_ERR_ARG, VO_ERR_CUDA, VO_ERR_UNSUPPORTED = 0, -1, -2, -3
-VO_ST_OK, VO_ST_NO_MODEL, VO_ST_TOO_FEW_POINTS, VO_ST_KP_OUT_OF_IMAGE = 0, 1, 2, 4
+VO_ST_OK, VO_ST_NO_MODEL, VO_ST_TOO_FEW_POINTS, VO_ST_KP_OUT_OF_IMAGE, VO_ST_BAD_INPUT = 0, 1, 2, 4, 8
 VO_NORM_HAMMING, VO_NORM_L2_U8, VO_NORM_HAMMING_TC = 0, 1, 2
 VO_METRIC_L2, VO_METRIC_COSINE = 0, 1
 (VO_MODE_RATIO, VO_MODE_MUTUAL, VO_MODE_RATIO_MUTUAL, VO_MODE_THRESH_MUTUAL, VO_MODE_THRESH,
  VO_MODE_NN) = range(6)
 VO_PREC_TF32X3, VO_PREC_TF32X1, VO_PREC_FP32_SIMT, VO_PREC_F16X1, VO_PREC_F16X3 = 0, 1, 2, 3, 4
+VO_PNP_THROUGHPUT, VO_PNP_REFERENCE = 0, 1
 
 c_void_p, c_int, c_float, c_double = ctypes.c_void_p, ctypes.c_int, ctypes.c_float, ctypes.c_double
 c_u64, c_i64 = ctypes.c_uint64, ctypes.c_int64
@@ -52,6 +53,9 @@ class PipelineArgs(ctypes.Structure):
         ("n_matches", c_void_p), ("n_corr", c_void_p), ("n_inl", c_void_p), ("status", c_void_p),
         ("depth_kp", c_void_p),
         ("u8_bytes", c_int),
+        ("pnp_mode", c_int),
+        ("ref_restarts", c_int), ("ref_iters", c_int),
+        ("ref_confidence", c_double),
     ]
 
 
@@ -70,6 +74,9 @@ class SeqConfig(ctypes.Structure):
         ("kf_min_common", c_int), ("kf_min_inliers", c_int),
         ("kf_max_dist", c_double),
         ("bad_pnp_limit", c_int), ("max_frames", c_int),
+        ("pnp_mode", c_int),
+        ("ref_restarts", c_int), ("ref_iters", c_int),
+        ("ref_confidence", c_double),
     ]
 
 
@@ -115,6 +122,10 @@ PROTOTYPES = {
                               c_void_p, c_void_p, c_void_p]),
     "vo_pnp_ransac_ref": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_int, c_float, c_double, c_int, c_int,
                                   c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vo_bootstrap": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_u64, c_i64, c_void_p, c_void_p]),
+    "vo_pnp_ransac_ref_batch": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_float,
+                                        c_double, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                        c_void_p, c_void_p, c_void_p]),
     "vo_pipeline": (c_int, [c_void_p, ctypes.POINTER(PipelineArgs), c_void_p]),
     "vo_seq_create": (c_int, [c_void_p, ctypes.POINTER(SeqConfig), ctypes.POINTER(c_void_p)]),
     "vo_seq_destroy": (None, [c_void_p]),

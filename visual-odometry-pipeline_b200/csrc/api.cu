@@ -190,25 +190,31 @@ extern "C" int vo_match_f32(vo_ctx *ctx, const float *ref, const float *cur, int
 // ---------------------------------------------------------------- whole-path pipeline
 extern "C" int vo_pipeline(vo_ctx *ctx, const vo_pipeline_args *a, void *stream) { return vo::pipeline_impl(ctx, a, stream, nullptr); }
 
-// pair0_dev (optional, device): the hypothesis generator's pair offset read on the device instead of a->pair0 (vo_seq_*'s graph)
+// pair0_dev (optional, device): the hypothesis / bootstrap generator's pair offset read on the device instead of a->pair0
+// (vo_seq_*'s graph)
 int vo::pipeline_impl(vo_ctx *ctx, const vo_pipeline_args *a, void *stream, const long long *pair0_dev) {
     using namespace vo;
     VO_REQUIRE(ctx && a, "vo_pipeline: null argument");
     const bool u8 = a->ref_u8 && a->cur_u8, f32 = a->ref_f32 && a->cur_f32;
     VO_REQUIRE(u8 != f32, "vo_pipeline: give exactly one descriptor pair (u8 or f32)");
-    VO_REQUIRE(a->B >= 0 && a->n_stride > 0 && a->m_stride > 0 && a->n_hyp > 0, "vo_pipeline: bad size");
+    VO_REQUIRE(a->pnp_mode == VO_PNP_THROUGHPUT || a->pnp_mode == VO_PNP_REFERENCE, "vo_pipeline: unknown pnp_mode %d", a->pnp_mode);
+    const bool ref = a->pnp_mode == VO_PNP_REFERENCE;
+    VO_REQUIRE(a->B >= 0 && a->n_stride > 0 && a->m_stride > 0 && (ref || a->n_hyp > 0), "vo_pipeline: bad size");
+    VO_REQUIRE(a->ref_restarts >= 0 && a->ref_iters >= 0 && a->ref_confidence >= 0.0, "vo_pipeline: negative Mode R parameter");
     VO_REQUIRE(a->ref_kp && a->cur_kp && (a->depth || a->depth_kp) && a->K_h, "vo_pipeline: null geometry input");
     VO_REQUIRE(a->T_rel && a->n_matches && a->n_corr && a->n_inl && a->status, "vo_pipeline: null output");
     if (a->B == 0) return VO_OK;
     const int B = a->B, cap = a->n_stride, H = a->n_hyp;
-    // scratch: pairs | xyz | ref_uv | cur_uv | hyp
+    const int restarts = a->ref_restarts ? a->ref_restarts : 3, iters = a->ref_iters ? a->ref_iters : 100;
+    const double confidence = a->ref_confidence != 0.0 ? a->ref_confidence : 0.99;
+    // scratch: pairs | xyz | ref_uv | cur_uv | hyp (Mode T: [B][H][4]) or bootstrap rows (Mode R: [B][restarts][cap])
     const size_t off_pairs = 0;
     const size_t off_xyz = off_pairs + sizeof(int32_t) * 2 * (size_t)B * cap;
     const size_t off_ruv = off_xyz + sizeof(float) * 3 * (size_t)B * cap;
     const size_t off_cuv = off_ruv + sizeof(float) * 2 * (size_t)B * cap;
     size_t off_hyp = off_cuv + sizeof(float) * 2 * (size_t)B * cap;
     off_hyp = (off_hyp + 255) & ~(size_t)255;
-    const size_t total = off_hyp + sizeof(int32_t) * 4 * (size_t)B * H;
+    const size_t total = off_hyp + sizeof(int32_t) * (ref ? (size_t)B * restarts * cap : 4 * (size_t)B * H);
     char *ws;
     int rc;
     if ((rc = ws_get(ctx, WS_PIPE, total, (void **)&ws))) return rc;
@@ -229,6 +235,12 @@ int vo::pipeline_impl(vo_ctx *ctx, const vo_pipeline_args *a, void *stream, cons
                                       a->min_flow_px, a->z_min, a->z_max, xyz, ruv, cuv, nullptr, a->n_corr, a->status,
                                       stream)))
         return rc;
+    if (ref) {
+        if ((rc = bootstrap_impl(ctx, a->n_corr, B, restarts, cap, a->seed, a->pair0, pair0_dev, hyp, stream))) return rc;
+        return pnp_ransac_ref_impl(ctx, xyz, cuv, a->n_corr, 0, B, cap, a->K_h, hyp, restarts, iters, a->thr_px, confidence,
+                                   a->min_inliers, a->refine_iters, a->rt, nullptr, a->T_rel, a->n_inl, nullptr, nullptr, nullptr,
+                                   nullptr, a->status, 1, stream);
+    }
     if ((rc = hypotheses_impl(ctx, a->n_corr, B, H, a->seed, a->pair0, pair0_dev, hyp, stream))) return rc;
     return pnp_ransac_impl(ctx, xyz, cuv, a->n_corr, B, cap, a->K_h, hyp, H, a->thr_px, a->min_inliers,
                            a->refine_iters, a->rt, nullptr, a->T_rel, a->n_inl, nullptr, nullptr, nullptr, a->status,

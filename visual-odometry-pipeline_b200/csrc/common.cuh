@@ -144,6 +144,13 @@ int pick_split(vo_ctx *ctx, int B, int row_blocks, int col_tiles, int min_tiles_
 int hypotheses_impl(vo_ctx *ctx, const int32_t *n_pts, int B, int H, uint64_t seed, int64_t pair0, const long long *pair0_dev,
                     int32_t *hyp, void *stream);
 int pipeline_impl(vo_ctx *ctx, const vo_pipeline_args *a, void *stream, const long long *pair0_dev);
+int bootstrap_impl(vo_ctx *ctx, const int32_t *n_pts, int B, int restarts, int cap, uint64_t seed, int64_t pair0,
+                   const long long *pair0_dev, int32_t *boot, void *stream);
+int pnp_ransac_ref_impl(vo_ctx *ctx, const float *xyz, const float *uv, const int32_t *n_pts, int n_fixed, int B, int cap,
+                        const double *K_h, const int32_t *boot_idx, int restarts, int iters, float thr_px, double confidence,
+                        int min_inliers, int refine_iters, double *rt, double *rvec_tvec, double *T_rel, int32_t *n_inl,
+                        int32_t *best, uint8_t *inlier_mask, int32_t *hyp_counts, double *hyp_poses, int32_t *status,
+                        int accumulate_status, void *stream);
 int pnp_ransac_impl(vo_ctx *ctx, const float *xyz, const float *uv, const int32_t *n_pts, int B, int cap,
                     const double *K_h, const int32_t *hyp, int H, float thr_px, int min_inliers, int refine_iters,
                     double *rt, double *rvec_tvec, double *T_rel, int32_t *n_inl, int32_t *best_h,

@@ -854,25 +854,71 @@ __device__ void jacobi12_warp(double (*A)[12], double (*V)[12], double *d, doubl
 // on lanes 0, 1, 2 at once.  Same operations in the same order per element as the serial refpnp::epnp5: identical results.
 // (One thread per solve, the first version, took 1.05 ms per frame pair for the 300 solves — a chain of dependent f64
 // operations on local-memory arrays; the warp-wide Jacobi brought it to 0.56 ms.)
+//
+// Batching: pair b of B owns xyz + b*cap*3, uv + b*cap*2, the bootstrap rows boot + b*restarts*cap (row stride cap) and the
+// sample table table + b*table_stride (stride 0: one table shared by the batch, the single-pair entry's host-built one).
+// pn[b] is the pair's point count once ref_prepare_kernel has checked it, -1 for a pair with bad input; pairs with fewer
+// than EP_N points (or bad input) solve nothing and read no point.  Every kernel indexes (b, restart, iteration) the same way,
+// so B = 1 with cap = n is exactly the single-pair computation.
+constexpr int RP_PREP_THREADS = 128;
+constexpr int32_t RP_BAD = -1;
+
+// one CTA per pair: n_pts[b] (n_fixed when n_pts is NULL) must lie in [0, cap] and every index of the first n entries of each
+// bootstrap row in [0, n); the verdict goes to pn[b].  With `table` set, thread 0 then builds the pair's OpenCV sample table
+// (refpnp::mwc_table: one thread stepping the multiply-with-carry generator, 87 us at iters = 100) — on the device, so the
+// batched entry needs no host staging and its table follows n_pts without a host read.
+__global__ void __launch_bounds__(RP_PREP_THREADS)
+ref_prepare_kernel(const int32_t *__restrict__ n_pts, int n_fixed, int cap, const int32_t *__restrict__ boot, int restarts,
+                   int iters, int32_t *__restrict__ table, int32_t *__restrict__ pn) {
+    const int b = blockIdx.x;
+    const int n = n_pts ? n_pts[b] : n_fixed;
+    int bad = (n < 0 || n > cap) ? 1 : 0;
+    if (!bad) {                                 // block-uniform
+        const int32_t *rows = boot + (size_t)b * restarts * cap;
+        for (int r = 0; r < restarts; ++r)
+            for (int i = threadIdx.x; i < n; i += RP_PREP_THREADS) {
+                const int32_t v = rows[(size_t)r * cap + i];
+                bad |= (v < 0 || v >= n) ? 1 : 0;
+            }
+    }
+    bad = __syncthreads_or(bad);
+    if (threadIdx.x == 0) {
+        pn[b] = bad ? RP_BAD : n;
+        if (table && !bad && n >= refpnp::EP_N) refpnp::mwc_table(n, iters, table + (size_t)b * iters * refpnp::EP_N);
+    }
+}
+
+// The warps cover B x restarts x iterations; an iteration without a model (pair without a solve, repeated point, no finite
+// candidate) writes valid 0 and a zero pose.
 constexpr int RP_WARPS = 4;
 __global__ void __launch_bounds__(32 * RP_WARPS)
-ref_epnp_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, const int32_t *__restrict__ boot, int n,
-                const int32_t *__restrict__ table, int restarts, int iters, IntrD kd, double *__restrict__ poses,
-                int32_t *__restrict__ valid) {
+ref_epnp_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, const int32_t *__restrict__ boot,
+                const int32_t *__restrict__ pn, int B, int cap, const int32_t *__restrict__ table, int table_stride, int restarts,
+                int iters, IntrD kd, double *__restrict__ poses, int32_t *__restrict__ valid) {
     __shared__ double sA[RP_WARPS][12][12], sV[RP_WARPS][12][12], sd[RP_WARPS][12], sX[RP_WARPS][refpnp::EP_N][3], sv[RP_WARPS][4][12];
     __shared__ refpnp::EpnpState sS[RP_WARPS];
     __shared__ int s_mode[RP_WARPS];            // 0: repeated point (no model), 1: regular, 2: coplanar
     __shared__ double s_cs[RP_WARPS][6][2];     // the (cos, sin) of a Jacobi round's six rotations
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int per = restarts * iters;
     const int id = blockIdx.x * RP_WARPS + w;
-    if (id >= restarts * iters) return;         // warp-uniform
-    const int r = id / iters, h = id % iters;
+    if (id >= B * per) return;                  // warp-uniform
+    const int b = id / per, r = (id % per) / iters, h = id % iters;
+    if (pn[b] < refpnp::EP_N) {                 // warp-uniform: too few points, or bad input
+        if (lane == 0) valid[id] = 0;
+        if (lane < 12) poses[(size_t)id * 12 + lane] = 0.0;
+        return;
+    }
+    xyz += (size_t)b * cap * 3;
+    uv += (size_t)b * cap * 2;
+    const int32_t *row = boot + ((size_t)b * restarts + r) * cap;
+    const int32_t *tab = table + (size_t)b * table_stride;
     if (lane == 0) {
         double q[refpnp::EP_N][2];
         int src[refpnp::EP_N];
         bool repeated = false;
         for (int j = 0; j < refpnp::EP_N; ++j) {
-            const int idx = boot[(size_t)r * n + table[h * refpnp::EP_N + j]];
+            const int idx = row[tab[h * refpnp::EP_N + j]];
             for (int k = 0; k < j; ++k) repeated = repeated || (src[k] == idx);
             src[j] = idx;
             for (int k = 0; k < 3; ++k) sX[w][j][k] = (double)xyz[(size_t)idx * 3 + k];
@@ -914,23 +960,28 @@ ref_epnp_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, con
         for (int k = 0; k < 9; ++k) poses[(size_t)id * 12 + k] = p.R[k];
         for (int k = 0; k < 3; ++k) poses[(size_t)id * 12 + 9 + k] = p.t[k];
     }
+    if (pick < 0 && lane < 12) poses[(size_t)id * 12 + lane] = 0.0;
 }
 
-// one warp per (restart, iteration): inlier count over the n points of the restart's resample
+// one warp per (pair, restart, iteration): inlier count over the n points of the restart's resample
 __global__ void __launch_bounds__(256)
-ref_score_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, const int32_t *__restrict__ boot, int n,
-                 int restarts, int iters, IntrD kd, float thr2, const double *__restrict__ poses,
-                 const int32_t *__restrict__ valid, int32_t *__restrict__ counts) {
+ref_score_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, const int32_t *__restrict__ boot,
+                 const int32_t *__restrict__ pn, int B, int cap, int restarts, int iters, IntrD kd, float thr2,
+                 const double *__restrict__ poses, const int32_t *__restrict__ valid, int32_t *__restrict__ counts) {
     const int id = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (id >= restarts * iters) return;
-    if (!valid[id]) {
+    const int per = restarts * iters;
+    if (id >= B * per) return;
+    if (!valid[id]) {                           // (every iteration of a pair without a solve)
         if (lane == 0) counts[id] = -1;
         return;
     }
+    const int pb = id / per, n = pn[pb];
+    xyz += (size_t)pb * cap * 3;
+    uv += (size_t)pb * cap * 2;
     refpnp::Pose p;
     for (int k = 0; k < 9; ++k) p.R[k] = poses[(size_t)id * 12 + k];
     for (int k = 0; k < 3; ++k) p.t[k] = poses[(size_t)id * 12 + 9 + k];
-    const int32_t *b = boot + (size_t)(id / iters) * n;
+    const int32_t *b = boot + ((size_t)pb * restarts + (id % per) / iters) * cap;
     int c = 0;
     for (int i = lane; i < n; i += 32) {
         const int idx = b[i];
@@ -943,18 +994,36 @@ ref_score_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, co
 }
 
 // stopping rule per restart, best of the restarts, inlier mask of the winning minimal model, Gauss-Newton refit on those
-// inliers (what cv2.solvePnP(ITERATIVE) converges to, SURVEY 3.4.1), Rodrigues vector and the pose the reference stores
+// inliers (what cv2.solvePnP(ITERATIVE) converges to, SURVEY 3.4.1), Rodrigues vector and the pose the reference stores.
+// One CTA per pair.  accumulate_status: OR into the soft bits an earlier stage set (vo_pipeline) instead of overwriting them.
 __global__ void __launch_bounds__(RF_THREADS)
-ref_select_refit_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, const int32_t *__restrict__ boot, int n,
-                        int restarts, int iters, IntrD kd, float thr2, double confidence, int min_inliers, int refine_iters,
-                        const double *__restrict__ poses, const int32_t *__restrict__ counts, double *__restrict__ rt_out,
-                        double *__restrict__ rvec_tvec, double *__restrict__ T_rel, int32_t *__restrict__ n_inl_out,
-                        int32_t *__restrict__ best_out, uint8_t *__restrict__ mask_out, int32_t *__restrict__ status) {
+ref_select_refit_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, const int32_t *__restrict__ boot,
+                        const int32_t *__restrict__ pn, int cap, int restarts, int iters, IntrD kd, float thr2, double confidence,
+                        int min_inliers, int refine_iters, const double *__restrict__ poses, const int32_t *__restrict__ counts,
+                        double *__restrict__ rt_out, double *__restrict__ rvec_tvec, double *__restrict__ T_rel,
+                        int32_t *__restrict__ n_inl_out, int32_t *__restrict__ best_out, uint8_t *__restrict__ mask_out,
+                        int32_t *__restrict__ status, int accumulate_status) {
     __shared__ int s_best[RP_MAX_RESTARTS], s_cnt[RP_MAX_RESTARTS], s_run[RP_MAX_RESTARTS];
     __shared__ int s_r, s_h, s_stop, s_bad;
     __shared__ double sR[9], st[3], sRp[9], stp[3], s_cost;
     __shared__ double sacc[RF_THREADS / 32][RF_ACC];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int pb = blockIdx.x, per = restarts * iters;
+    const int n_chk = pn[pb];
+    const bool bad_input = n_chk == RP_BAD;
+    const int n = bad_input ? 0 : n_chk;
+    xyz += (size_t)pb * cap * 3;
+    uv += (size_t)pb * cap * 2;
+    boot += (size_t)pb * restarts * cap;
+    poses += (size_t)pb * per * 12;
+    counts += (size_t)pb * per;
+    if (rt_out) rt_out += (size_t)pb * 12;
+    if (rvec_tvec) rvec_tvec += (size_t)pb * 6;
+    if (T_rel) T_rel += (size_t)pb * 16;
+    if (n_inl_out) n_inl_out += pb;
+    if (best_out) best_out += (size_t)pb * 3;
+    if (mask_out) mask_out += (size_t)pb * cap;
+    if (status) status += pb;
     if (threadIdx.x < restarts) {
         int run = 0, cnt = 0;
         s_best[threadIdx.x] = refpnp::ransac_scan(counts + threadIdx.x * iters, n, iters, confidence, &run, &cnt);
@@ -978,11 +1047,12 @@ ref_select_refit_kernel(const float *__restrict__ xyz, const float *__restrict__
     }
     __syncthreads();
     const int rsel = s_r, hsel = s_h;
-    if (rsel < 0) {
+    if (rsel < 0) {                                         // (always so for a pair with bad input: all its counts are -1)
         if (mask_out)
-            for (int i = threadIdx.x; i < n; i += RF_THREADS) mask_out[i] = 0;
+            for (int i = threadIdx.x; i < (bad_input ? cap : n); i += RF_THREADS) mask_out[i] = 0;
         if (threadIdx.x == 0) {
-            if (status) status[0] = VO_ST_NO_MODEL;
+            if (status)
+                status[0] = (accumulate_status ? status[0] : 0) | VO_ST_NO_MODEL | (bad_input ? VO_ST_BAD_INPUT : 0);
             if (n_inl_out) n_inl_out[0] = 0;
             if (best_out) { best_out[0] = -1; best_out[1] = -1; best_out[2] = 0; }
             for (int j = 0; j < 16; ++j)
@@ -994,7 +1064,7 @@ ref_select_refit_kernel(const float *__restrict__ xyz, const float *__restrict__
         }
         return;
     }
-    const int32_t *b = boot + (size_t)rsel * n;
+    const int32_t *b = boot + (size_t)rsel * cap;
     refpnp::Pose pm;                                        // the winning minimal model: its mask selects the refit's points
     for (int j = 0; j < 9; ++j) pm.R[j] = sR[j];
     for (int j = 0; j < 3; ++j) pm.t[j] = st[j];
@@ -1102,7 +1172,7 @@ ref_select_refit_kernel(const float *__restrict__ xyz, const float *__restrict__
             for (int j = 0; j < 9; ++j) sR[j] = (j % 4 == 0) ? 1.0 : 0.0;
             for (int j = 0; j < 3; ++j) st[j] = 0.0;
         }
-        if (status) status[0] = s_bad ? VO_ST_NO_MODEL : VO_ST_OK;
+        if (status) status[0] = (accumulate_status ? status[0] : 0) | (s_bad ? VO_ST_NO_MODEL : VO_ST_OK);
         if (n_inl_out) n_inl_out[0] = s_cnt[rsel];
         if (best_out) { best_out[0] = rsel; best_out[1] = hsel; best_out[2] = s_run[rsel]; }
         if (rt_out) {
@@ -1125,55 +1195,121 @@ ref_select_refit_kernel(const float *__restrict__ xyz, const float *__restrict__
     }
 }
 
+// ---------------------------------------------------------------- bootstrap rows
+// boot[b][r][i] = draw_bootstrap(seed, pair0 + b, r, i, n_pts[b]) for i < n_pts[b] (pnp_math.cuh: keyed like the hypotheses,
+// a pure function of the pair, not of its batch position), -1 for the padding i >= n_pts[b].
+__global__ void bootstrap_kernel(const int32_t *__restrict__ n_pts, int B, int restarts, int cap, uint64_t seed, int64_t pair0,
+                                 const long long *__restrict__ pair0_dev, int32_t *__restrict__ boot) {
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= (long long)B * restarts * cap) return;
+    const int i = (int)(gid % cap), r = (int)((gid / cap) % restarts), b = (int)(gid / ((long long)cap * restarts));
+    const int n = n_pts[b];
+    if (pair0_dev) pair0 = (int64_t)*pair0_dev;
+    boot[gid] = i < n ? draw_bootstrap(seed, pair0 + b, r, i, n) : -1;
+}
+
 }  // namespace
+
+int bootstrap_impl(vo_ctx *ctx, const int32_t *n_pts, int B, int restarts, int cap, uint64_t seed, int64_t pair0,
+                   const long long *pair0_dev, int32_t *boot, void *stream) {
+    VO_REQUIRE(ctx && n_pts && boot, "vo_bootstrap: null argument");
+    VO_REQUIRE(B >= 0 && restarts >= 0 && cap >= 0, "vo_bootstrap: negative size");
+    const long long total = (long long)B * restarts * cap;
+    if (total == 0) return VO_OK;
+    VO_PROF(ctx, (cudaStream_t)stream, VO_STAGE_HYP);
+    bootstrap_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n_pts, B, restarts, cap, seed, pair0,
+                                                                                      pair0_dev, boot);
+    VO_LAUNCH_CHECK(ctx);
+    VO_PROF(ctx, (cudaStream_t)stream, -1);
+    return VO_OK;
+}
+
+// Both Mode R entries.  n_pts NULL: one pair (B = 1) of n_fixed points whose bootstrap rows have stride cap = n_fixed, with the
+// sample table built on the host; otherwise B pairs, n_pts on the device, one table per pair built on the device.
+int pnp_ransac_ref_impl(vo_ctx *ctx, const float *xyz, const float *uv, const int32_t *n_pts, int n_fixed, int B, int cap,
+                        const double *K_h, const int32_t *boot_idx, int restarts, int iters, float thr_px, double confidence,
+                        int min_inliers, int refine_iters, double *rt, double *rvec_tvec, double *T_rel, int32_t *n_inl,
+                        int32_t *best, uint8_t *inlier_mask, int32_t *hyp_counts, double *hyp_poses, int32_t *status,
+                        int accumulate_status, void *stream) {
+    VO_REQUIRE(B >= 0 && cap >= 0 && restarts >= 1 && restarts <= RP_MAX_RESTARTS && iters >= 1 && iters <= RP_MAX_ITERS,
+               "vo_pnp_ransac_ref: bad size (B %d, cap %d, restarts %d, iterations %d)", B, cap, restarts, iters);
+    VO_REQUIRE(K_h[0] != 0.0 && K_h[4] != 0.0, "vo_pnp_ransac_ref: zero focal length");
+    VO_REQUIRE((long long)B * restarts * iters <= 0x7fffffffLL, "vo_pnp_ransac_ref: %d pairs x %d x %d models exceed 2^31", B,
+               restarts, iters);
+    if (B == 0) return VO_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    const bool host_table = n_pts == nullptr;
+    const size_t per = (size_t)restarts * iters, total = (size_t)B * per;
+    // workspace: sample tables | checked point counts | validity | counts | poses
+    char *ws;
+    int rc;
+    const size_t table_ints = (size_t)(host_table ? 1 : B) * iters * refpnp::EP_N;
+    const size_t off_pn = sizeof(int32_t) * table_ints, off_valid = off_pn + sizeof(int32_t) * (size_t)B,
+                 off_counts = off_valid + sizeof(int32_t) * total;
+    const size_t off_poses = (off_counts + sizeof(int32_t) * total + 15) & ~(size_t)15;
+    if ((rc = ws_get(ctx, WS_POSES, off_poses + sizeof(double) * 12 * total, (void **)&ws))) return rc;
+    int32_t *table = reinterpret_cast<int32_t *>(ws), *pn = reinterpret_cast<int32_t *>(ws + off_pn);
+    int32_t *valid = reinterpret_cast<int32_t *>(ws + off_valid), *counts = reinterpret_cast<int32_t *>(ws + off_counts);
+    double *poses = reinterpret_cast<double *>(ws + off_poses);
+    const IntrD kd{K_h[0], K_h[4], K_h[2], K_h[5]};
+    const float thr2 = (float)((double)thr_px * (double)thr_px);      // findInliers: float t = (float)(thresh * thresh)
+    VO_PROF(ctx, st, VO_STAGE_HYP);
+    if (host_table && n_fixed >= refpnp::EP_N) {
+        // OpenCV's sample table is a function of the point count alone.  One pair: built on the host (the same
+        // refpnp::mwc_table; on the device it is one thread, 87 us of the 470 us call) and copied in stream order — a
+        // pageable source is staged by the driver before cudaMemcpyAsync returns, so the array may die here.  (Not
+        // capture-safe; the batched entry builds its tables on the device.)
+        int32_t table_h[RP_MAX_ITERS * refpnp::EP_N];
+        refpnp::mwc_table(n_fixed, iters, table_h);
+        VO_CUDA(cudaMemcpyAsync(table, table_h, sizeof(int32_t) * (size_t)iters * refpnp::EP_N, cudaMemcpyHostToDevice, st));
+    }
+    ref_prepare_kernel<<<B, RP_PREP_THREADS, 0, st>>>(n_pts, n_fixed, cap, boot_idx, restarts, iters, host_table ? nullptr : table, pn);
+    VO_LAUNCH_CHECK(ctx);
+    VO_PROF(ctx, st, VO_STAGE_P3P);
+    const int table_stride = host_table ? 0 : iters * refpnp::EP_N;
+    ref_epnp_kernel<<<(unsigned)((total + RP_WARPS - 1) / RP_WARPS), 32 * RP_WARPS, 0, st>>>(xyz, uv, boot_idx, pn, B, cap, table,
+                                                                                            table_stride, restarts, iters, kd, poses, valid);
+    VO_LAUNCH_CHECK(ctx);
+    VO_PROF(ctx, st, VO_STAGE_SCORE);
+    ref_score_kernel<<<(unsigned)((total + 7) / 8), 256, 0, st>>>(xyz, uv, boot_idx, pn, B, cap, restarts, iters, kd, thr2,
+                                                                            poses, valid, counts);
+    VO_LAUNCH_CHECK(ctx);
+    VO_PROF(ctx, st, VO_STAGE_REFIT);
+    ref_select_refit_kernel<<<B, RF_THREADS, 0, st>>>(xyz, uv, boot_idx, pn, cap, restarts, iters, kd, thr2, confidence, min_inliers,
+                                                      refine_iters, poses, counts, rt, rvec_tvec, T_rel, n_inl, best, inlier_mask,
+                                                      status, accumulate_status);
+    VO_LAUNCH_CHECK(ctx);
+    VO_PROF(ctx, st, -1);
+    if (hyp_counts) VO_CUDA(cudaMemcpyAsync(hyp_counts, counts, sizeof(int32_t) * total, cudaMemcpyDeviceToDevice, st));
+    if (hyp_poses) VO_CUDA(cudaMemcpyAsync(hyp_poses, poses, sizeof(double) * 12 * total, cudaMemcpyDeviceToDevice, st));
+    return VO_OK;
+}
+
 }  // namespace vo
 
 extern "C" int vo_pnp_ransac_ref(vo_ctx *ctx, const float *xyz, const float *uv, int n, const double *K_h, const int32_t *boot_idx,
                                  int restarts, int iters, float thr_px, double confidence, int min_inliers, int refine_iters,
                                  double *rt, double *rvec_tvec, double *T_rel, int32_t *n_inl, int32_t *best, uint8_t *inlier_mask,
                                  int32_t *hyp_counts, double *hyp_poses, int32_t *status, void *stream) {
-    using namespace vo;
     VO_REQUIRE(ctx && xyz && uv && K_h && boot_idx, "vo_pnp_ransac_ref: null argument");
-    VO_REQUIRE(n >= 0 && restarts >= 1 && restarts <= RP_MAX_RESTARTS && iters >= 1 && iters <= RP_MAX_ITERS,
-               "vo_pnp_ransac_ref: bad size (n %d, restarts %d, iterations %d)", n, restarts, iters);
-    VO_REQUIRE(K_h[0] != 0.0 && K_h[4] != 0.0, "vo_pnp_ransac_ref: zero focal length");
-    cudaStream_t st = (cudaStream_t)stream;
-    const int total = restarts * iters;
-    // workspace: sample table | validity | counts | poses
-    char *ws;
-    int rc;
-    const size_t off_valid = sizeof(int32_t) * (size_t)iters * refpnp::EP_N, off_counts = off_valid + sizeof(int32_t) * total;
-    const size_t off_poses = (off_counts + sizeof(int32_t) * total + 15) & ~(size_t)15;
-    if ((rc = ws_get(ctx, WS_POSES, off_poses + sizeof(double) * 12 * (size_t)total, (void **)&ws))) return rc;
-    int32_t *table = reinterpret_cast<int32_t *>(ws), *valid = reinterpret_cast<int32_t *>(ws + off_valid);
-    int32_t *counts = reinterpret_cast<int32_t *>(ws + off_counts);
-    double *poses = reinterpret_cast<double *>(ws + off_poses);
-    const IntrD kd{K_h[0], K_h[4], K_h[2], K_h[5]};
-    const float thr2 = (float)((double)thr_px * (double)thr_px);      // findInliers: float t = (float)(thresh * thresh)
-    if (n < refpnp::EP_N) {                                            // RANSAC needs at least the model points: "no model"
-        VO_CUDA(cudaMemsetAsync(counts, 0xff, sizeof(int32_t) * total, st));
-    } else {
-        VO_PROF(ctx, st, VO_STAGE_P3P);
-        // OpenCV's sample table is a function of the point count alone: built on the host (the same refpnp::mwc_table; the device
-        // kernel that did it took 87 us of the 470 us call, one thread stepping a multiply-with-carry generator) and copied in
-        // stream order — a pageable source is staged by the driver before cudaMemcpyAsync returns, so the array may die here
-        {
-            int32_t table_h[RP_MAX_ITERS * refpnp::EP_N];
-            refpnp::mwc_table(n, iters, table_h);
-            VO_CUDA(cudaMemcpyAsync(table, table_h, sizeof(int32_t) * (size_t)iters * refpnp::EP_N, cudaMemcpyHostToDevice, st));
-        }
-        ref_epnp_kernel<<<ceil_div(total, RP_WARPS), 32 * RP_WARPS, 0, st>>>(xyz, uv, boot_idx, n, table, restarts, iters, kd, poses, valid);
-        VO_LAUNCH_CHECK(ctx);
-        VO_PROF(ctx, st, VO_STAGE_SCORE);
-        ref_score_kernel<<<ceil_div(total, 8), 256, 0, st>>>(xyz, uv, boot_idx, n, restarts, iters, kd, thr2, poses, valid, counts);
-        VO_LAUNCH_CHECK(ctx);
-    }
-    VO_PROF(ctx, st, VO_STAGE_REFIT);
-    ref_select_refit_kernel<<<1, RF_THREADS, 0, st>>>(xyz, uv, boot_idx, n, restarts, iters, kd, thr2, confidence, min_inliers, refine_iters,
-                                                      poses, counts, rt, rvec_tvec, T_rel, n_inl, best, inlier_mask, status);
-    VO_LAUNCH_CHECK(ctx);
-    VO_PROF(ctx, st, -1);
-    if (hyp_counts) VO_CUDA(cudaMemcpyAsync(hyp_counts, counts, sizeof(int32_t) * total, cudaMemcpyDeviceToDevice, st));
-    if (hyp_poses) VO_CUDA(cudaMemcpyAsync(hyp_poses, poses, sizeof(double) * 12 * (size_t)total, cudaMemcpyDeviceToDevice, st));
-    return VO_OK;
+    VO_REQUIRE(n >= 0, "vo_pnp_ransac_ref: bad size (n %d)", n);
+    return vo::pnp_ransac_ref_impl(ctx, xyz, uv, nullptr, n, 1, n, K_h, boot_idx, restarts, iters, thr_px, confidence, min_inliers,
+                                   refine_iters, rt, rvec_tvec, T_rel, n_inl, best, inlier_mask, hyp_counts, hyp_poses, status, 0,
+                                   stream);
+}
+
+extern "C" int vo_pnp_ransac_ref_batch(vo_ctx *ctx, const float *xyz, const float *uv, const int32_t *n_pts, int B, int cap,
+                                       const double *K_h, const int32_t *boot_idx, int restarts, int iters, float thr_px,
+                                       double confidence, int min_inliers, int refine_iters, double *rt, double *rvec_tvec,
+                                       double *T_rel, int32_t *n_inl, int32_t *best, uint8_t *inlier_mask, int32_t *hyp_counts,
+                                       double *hyp_poses, int32_t *status, void *stream) {
+    VO_REQUIRE(ctx && xyz && uv && n_pts && K_h && boot_idx && T_rel && status, "vo_pnp_ransac_ref_batch: null argument");
+    return vo::pnp_ransac_ref_impl(ctx, xyz, uv, n_pts, 0, B, cap, K_h, boot_idx, restarts, iters, thr_px, confidence, min_inliers,
+                                   refine_iters, rt, rvec_tvec, T_rel, n_inl, best, inlier_mask, hyp_counts, hyp_poses, status, 0,
+                                   stream);
+}
+
+extern "C" int vo_bootstrap(vo_ctx *ctx, const int32_t *n_pts, int B, int restarts, int cap, uint64_t seed, int64_t pair0,
+                            int32_t *boot, void *stream) {
+    return vo::bootstrap_impl(ctx, n_pts, B, restarts, cap, seed, pair0, nullptr, boot, stream);
 }

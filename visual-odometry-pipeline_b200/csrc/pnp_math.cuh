@@ -40,6 +40,17 @@ VO_HD uint64_t mix64(uint64_t z) {
     return z ^ (z >> 31);
 }
 
+// Mode R bootstrap entry i of restart r of pair `pair`, uniform in [0, n); requires n >= 1.  The pair key is the hypothesis
+// generator's; the restart is mixed in XOR-ed into a domain constant whose high word is set, so no row key equals a hypothesis
+// key of the same (seed, pair) (mix64 is a bijection and a hypothesis mixes in h < 2^32).  Range map: multiply-high of the high
+// word u, (u * n) >> 32, which gives every value floor or ceil of 2^32 / n of the 2^32 words: relative bias below n / 2^32.
+VO_HD int32_t draw_bootstrap(uint64_t seed, int64_t pair, int r, int i, int n) {
+    uint64_t key = mix64(seed + 0x9E3779B97F4A7C15ull * (uint64_t)(pair + 1));
+    key = mix64(key ^ 0xB0075742A9B5D0E1ull ^ (uint64_t)(uint32_t)r);
+    const uint32_t u = (uint32_t)(mix64(key + (uint64_t)(uint32_t)i * 0xD1B54A32D192ED03ull) >> 32);
+    return (int32_t)(((uint64_t)u * (uint64_t)(uint32_t)n) >> 32);
+}
+
 // 4 distinct indices in [0, n) for hypothesis h of pair `pair`; requires n >= 4.
 VO_HD void draw_hypothesis(uint64_t seed, int64_t pair, int h, int n, int32_t out[4]) {
     uint64_t key = mix64(seed + 0x9E3779B97F4A7C15ull * (uint64_t)(pair + 1));

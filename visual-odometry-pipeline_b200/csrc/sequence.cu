@@ -135,7 +135,10 @@ extern "C" int vo_seq_create(vo_ctx *ctx, const vo_seq_config *cfg, vo_seq **out
     using namespace vo;
     VO_REQUIRE(ctx && cfg && out, "vo_seq_create: null argument");
     *out = nullptr;
-    VO_REQUIRE(cfg->n_cap > 0 && cfg->H > 0 && cfg->W > 0 && cfg->kp_stride >= 2 && cfg->n_hyp > 0 && cfg->max_frames > 0,
+    VO_REQUIRE(cfg->pnp_mode == VO_PNP_THROUGHPUT || cfg->pnp_mode == VO_PNP_REFERENCE, "vo_seq_create: unknown pnp_mode %d",
+               cfg->pnp_mode);
+    VO_REQUIRE(cfg->n_cap > 0 && cfg->H > 0 && cfg->W > 0 && cfg->kp_stride >= 2 &&
+                   (cfg->n_hyp > 0 || cfg->pnp_mode == VO_PNP_REFERENCE) && cfg->max_frames > 0,
                "vo_seq_create: bad size");
     vo_seq *s = (vo_seq *)calloc(1, sizeof(vo_seq));
     VO_REQUIRE(s, "vo_seq_create: out of host memory");
@@ -214,6 +217,7 @@ extern "C" int vo_seq_push(vo_seq *seq, const void *desc, const float *kp, int n
             a.min_flow_px = c.min_flow_px; a.z_min = c.z_min; a.z_max = c.z_max;
             a.n_hyp = c.n_hyp; a.seed = c.seed; a.pair0 = slot - 1;
             a.thr_px = c.thr_px; a.min_inliers = c.min_inliers; a.refine_iters = c.refine_iters;
+            a.pnp_mode = c.pnp_mode; a.ref_restarts = c.ref_restarts; a.ref_iters = c.ref_iters; a.ref_confidence = c.ref_confidence;
             a.T_rel = seq->T_rel; a.rt = seq->rt;
             a.n_matches = seq->out4 + 0; a.n_corr = seq->out4 + 1; a.n_inl = seq->out4 + 2; a.status = seq->out4 + 3;
             int rc = pipeline_impl(ctx, &a, stream, &seq->st->pair0);
@@ -228,8 +232,9 @@ extern "C" int vo_seq_push(vo_seq *seq, const void *desc, const float *kp, int n
         VO_LAUNCH_CHECK(ctx);
         return VO_OK;
     };
-    // frames 0 and 1 run plainly (frame 1 sizes every workspace: nothing may allocate during capture); frame 2 captures
-    if (slot >= 2 && seq->graph_state == 0 && !ctx->prof_on && getenv("VO_SEQ_GRAPH")) {
+    // frames 0 and 1 run plainly (frame 1 sizes every workspace: nothing may allocate during capture); frame 2 captures.
+    // A Mode R loop always runs plainly (its graph is not captured).
+    if (slot >= 2 && seq->graph_state == 0 && !ctx->prof_on && c.pnp_mode == VO_PNP_THROUGHPUT && getenv("VO_SEQ_GRAPH")) {
         cudaGraph_t g = nullptr;
         const long long l0 = ctx->launches;
         seq->graph_state = -1;

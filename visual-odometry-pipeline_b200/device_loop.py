@@ -19,7 +19,10 @@ class DeviceLoop:
     def __init__(self, K, wh, n_cap, *, kind="orb", kp_stride=2, norm_or_metric=None, mode=None, match_param=0.85,
                  precision=None, allow_inexact=False, n_hyp=512, seed=8214, thr_px=1.5, min_inliers=20, refine_iters=10,
                  min_flow_px=3.0, z_range=(0.0, 50.0), max_step_m=1.5, kf_min_common=200, kf_min_inliers=100,
-                 kf_max_dist=1.5, bad_pnp_limit=3, max_frames=4096, device=None):
+                 kf_max_dist=1.5, bad_pnp_limit=3, max_frames=4096, device=None, pnp_mode="throughput", ref_restarts=3,
+                 ref_iters=100, ref_confidence=0.99):
+        """pnp_mode "reference": every frame runs Mode R (vo_bootstrap keyed by the frame's history slot - 1, then the batched
+        reference-sampler RANSAC with B = 1); such a loop always launches plainly (VO_SEQ_GRAPH does not apply to it)."""
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.ctx = ops.context(self.device)
         f32 = kind != "orb"
@@ -48,6 +51,12 @@ class DeviceLoop:
         c.min_inliers, c.refine_iters = int(min_inliers), int(refine_iters)
         c.max_step_m, c.kf_min_common, c.kf_min_inliers = float(max_step_m), int(kf_min_common), int(kf_min_inliers)
         c.kf_max_dist, c.bad_pnp_limit, c.max_frames = float(kf_max_dist), int(bad_pnp_limit), int(max_frames)
+        c.pnp_mode = ops.pnp_mode_id(pnp_mode)
+        if c.pnp_mode == ops.VO_PNP_REFERENCE:
+            if not 1 <= int(ref_restarts) <= ops.REF_MAX_RESTARTS or not 1 <= int(ref_iters) <= ops.REF_MAX_ITERS:
+                raise ValueError(f"DeviceLoop: ref_restarts {ref_restarts} must be in 1..{ops.REF_MAX_RESTARTS}, ref_iters "
+                                 f"{ref_iters} in 1..{ops.REF_MAX_ITERS}")
+            c.ref_restarts, c.ref_iters, c.ref_confidence = int(ref_restarts), int(ref_iters), float(ref_confidence)
         self.cfg = c
         self.desc_dtype = np.float32 if f32 else np.uint8
         self.desc_cols = 128 if f32 else 32

@@ -10,7 +10,8 @@ import torch
 from . import _lib
 from ._lib import (KnnOut, PipelineArgs, VO_METRIC_COSINE, VO_METRIC_L2, VO_MODE_MUTUAL, VO_MODE_NN, VO_MODE_RATIO,
                    VO_MODE_RATIO_MUTUAL, VO_MODE_THRESH, VO_MODE_THRESH_MUTUAL, VO_NORM_HAMMING, VO_NORM_HAMMING_TC, VO_NORM_L2_U8,
-                   VO_PREC_F16X1, VO_PREC_F16X3, VO_PREC_FP32_SIMT, VO_PREC_TF32X1, VO_PREC_TF32X3, check)
+                   VO_PNP_REFERENCE, VO_PNP_THROUGHPUT, VO_PREC_F16X1, VO_PREC_F16X3, VO_PREC_FP32_SIMT, VO_PREC_TF32X1,
+                   VO_PREC_TF32X3, VO_ST_BAD_INPUT, check)
 
 _contexts = {}
 
@@ -307,6 +308,73 @@ def pnp_ransac_ref(xyz, uv, n, K, boot_idx, iters=100, thr_px=1.5, confidence=0.
     return PnpRefResult(rt, rv, T, n_inl, best, mask, counts, poses, status)
 
 
+REF_MAX_RESTARTS, REF_MAX_ITERS = 8, 1024
+
+
+def bootstrap(n_pts, restarts, cap, seed=8214, pair0=0):
+    """Mode R bootstrap rows int32 [B, restarts, cap] (vo_bootstrap): entry [b, r, i] uniform in [0, n_pts[b]) for
+    i < n_pts[b], -1 past it; keyed by (seed, pair0 + b, r, i), so a pair's rows do not depend on its batch position."""
+    _chk(n_pts, torch.int32, "n_pts")
+    B = n_pts.shape[0]
+    boot = torch.empty((B, int(restarts), int(cap)), dtype=torch.int32, device=n_pts.device)
+    ctx = context(n_pts.device)
+    with torch.cuda.device(n_pts.device):
+        check(ctx.lib.vo_bootstrap(ctx.handle, _ptr(n_pts), B, int(restarts), int(cap), int(seed), int(pair0), _ptr(boot),
+                                   _stream()), "vo_bootstrap")
+    return boot
+
+
+def pnp_ransac_ref_batch(xyz, uv, n_pts, K, boot_idx, iters=100, thr_px=1.5, confidence=0.99, min_inliers=20, refine_iters=20,
+                         want_hyp=False):
+    """Reference-sampler PnP-RANSAC over B pairs (vo_pnp_ransac_ref_batch): xyz [B,cap,3], uv [B,cap,2] float32, n_pts int32 [B]
+    (device: no host read), boot_idx int32 [B,restarts,cap] (bootstrap(), or the caller's rows; first n_pts[b] entries used).
+    Pair b's outputs equal pnp_ransac_ref on its first n_pts[b] rows bit for bit; a pair with n_pts[b] outside [0, cap] or an
+    index outside [0, n_pts[b]) gets status VO_ST_NO_MODEL | VO_ST_BAD_INPUT and reads nothing."""
+    _chk(xyz, torch.float32, "xyz")
+    _chk(uv, torch.float32, "uv")
+    _chk(n_pts, torch.int32, "n_pts")
+    _chk(boot_idx, torch.int32, "boot_idx")
+    if xyz.dim() != 3 or xyz.shape[2] != 3:
+        raise ValueError(f"pnp_ransac_ref_batch: xyz must be [B, cap, 3], got {tuple(xyz.shape)}")
+    B, cap = int(xyz.shape[0]), int(xyz.shape[1])
+    if tuple(uv.shape) != (B, cap, 2) or tuple(n_pts.shape) != (B,):
+        raise ValueError(f"pnp_ransac_ref_batch: uv {tuple(uv.shape)} / n_pts {tuple(n_pts.shape)} do not match xyz {tuple(xyz.shape)}")
+    if boot_idx.dim() != 3 or boot_idx.shape[0] != B or boot_idx.shape[2] != cap:
+        raise ValueError(f"pnp_ransac_ref_batch: boot_idx must be [{B}, restarts, {cap}], got {tuple(boot_idx.shape)}")
+    restarts = int(boot_idx.shape[1])
+    if not 1 <= restarts <= REF_MAX_RESTARTS or not 1 <= int(iters) <= REF_MAX_ITERS:
+        raise ValueError(f"pnp_ransac_ref_batch: restarts {restarts} must be in 1..{REF_MAX_RESTARTS}, iters {iters} in "
+                         f"1..{REF_MAX_ITERS}")
+    dev = xyz.device
+    rt = torch.empty((B, 12), dtype=torch.float64, device=dev)
+    rv = torch.empty((B, 6), dtype=torch.float64, device=dev)
+    T = torch.empty((B, 4, 4), dtype=torch.float64, device=dev)
+    n_inl = torch.zeros((B,), dtype=torch.int32, device=dev)
+    best = torch.zeros((B, 3), dtype=torch.int32, device=dev)
+    mask = torch.zeros((B, max(cap, 1)), dtype=torch.uint8, device=dev)
+    counts = torch.zeros((B, restarts, int(iters)), dtype=torch.int32, device=dev) if want_hyp else None
+    poses = torch.zeros((B, restarts, int(iters), 12), dtype=torch.float64, device=dev) if want_hyp else None
+    status = torch.zeros((B,), dtype=torch.int32, device=dev)
+    ctx = context(dev)
+    kh, kp = _k_host(K)
+    with torch.cuda.device(dev):
+        check(ctx.lib.vo_pnp_ransac_ref_batch(ctx.handle, _ptr(xyz), _ptr(uv), _ptr(n_pts), B, cap, kp, _ptr(boot_idx), restarts,
+                                              int(iters), float(thr_px), float(confidence), int(min_inliers), int(refine_iters),
+                                              _ptr(rt), _ptr(rv), _ptr(T), _ptr(n_inl), _ptr(best), _ptr(mask), _ptr(counts),
+                                              _ptr(poses), _ptr(status), _stream()), "vo_pnp_ransac_ref_batch")
+    return PnpRefResult(rt, rv, T, n_inl, best, mask, counts, poses, status)
+
+
+_PNP_MODES = {"throughput": VO_PNP_THROUGHPUT, "reference": VO_PNP_REFERENCE}
+
+
+def pnp_mode_id(pnp_mode):
+    """"throughput" (Mode T, the default) or "reference" (Mode R) -> VO_PNP_*."""
+    if pnp_mode not in _PNP_MODES:
+        raise ValueError(f"pnp_mode must be 'throughput' or 'reference', got {pnp_mode!r}")
+    return _PNP_MODES[pnp_mode]
+
+
 class PipelineResult:
     def __init__(self, T_rel, rt, n_matches, n_corr, n_inl, status):
         self.T_rel, self.rt, self.n_matches, self.n_corr, self.n_inl, self.status = T_rel, rt, n_matches, n_corr, n_inl, status
@@ -327,8 +395,10 @@ class PipelineBuffers:
 def pipeline(ref_desc, cur_desc, ref_kp, cur_kp, depth, K, *, norm_or_metric, mode, match_param=0.85,
              precision=VO_PREC_TF32X3, n_ref=None, n_cur=None, n_hyp=1024, seed=8214, pair0=0, thr_px=1.5,
              min_inliers=20, refine_iters=10, min_flow_px=3.0, z_min=0.0, z_max=50.0, out=None, depth_kp=None, hw=None,
-             lane=0):
+             lane=0, pnp_mode="throughput", ref_restarts=3, ref_iters=100, ref_confidence=0.99):
     """match -> gather/back-project -> hypotheses -> PnP-RANSAC -> T_rel for a batch of pairs (vo_pipeline).
+    pnp_mode "reference" runs Mode R instead of the hypotheses and P3P RANSAC: bootstrap(n_corr, ref_restarts, N, seed, pair0)
+    -> pnp_ransac_ref_batch(ref_iters, thr_px, ref_confidence, min_inliers, refine_iters); n_hyp is then ignored.
     `depth` is the reference frames' dense map [B,H,W], on the device or in pinned host memory (then only the pixels
     under the matched reference keypoints cross the bus, read zero-copy by the gather kernel); alternatively pass
     `depth_kp` [B,N] (sample_depth) and `hw=(H, W)`.  `lane` selects the vo_ctx (see context())."""
@@ -367,6 +437,12 @@ def pipeline(ref_desc, cur_desc, ref_kp, cur_kp, depth, K, *, norm_or_metric, mo
     a.min_flow_px, a.z_min, a.z_max = float(min_flow_px), float(z_min), float(z_max)
     a.n_hyp, a.seed, a.pair0 = int(n_hyp), int(seed), int(pair0)
     a.thr_px, a.min_inliers, a.refine_iters = float(thr_px), int(min_inliers), int(refine_iters)
+    a.pnp_mode = pnp_mode_id(pnp_mode)
+    if a.pnp_mode == VO_PNP_REFERENCE:
+        if not 1 <= int(ref_restarts) <= REF_MAX_RESTARTS or not 1 <= int(ref_iters) <= REF_MAX_ITERS:
+            raise ValueError(f"pipeline: ref_restarts {ref_restarts} must be in 1..{REF_MAX_RESTARTS}, ref_iters {ref_iters} in "
+                             f"1..{REF_MAX_ITERS}")
+        a.ref_restarts, a.ref_iters, a.ref_confidence = int(ref_restarts), int(ref_iters), float(ref_confidence)
     a.T_rel, a.rt = out.T_rel.data_ptr(), out.rt.data_ptr()
     a.n_matches, a.n_corr = out.n_matches.data_ptr(), out.n_corr.data_ptr()
     a.n_inl, a.status = out.n_inl.data_ptr(), out.status.data_ptr()

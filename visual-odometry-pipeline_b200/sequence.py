@@ -133,10 +133,16 @@ class FrameSequence:
 
 
 class PipelineConfig:
+    """Keyword arguments of ops.pipeline shared by every chunk.  pnp_mode "reference" selects Mode R (the reference's sampler,
+    bootstrap rows keyed by the pair like the hypotheses: results do not depend on chunk or lanes); the default is Mode T."""
     def __init__(self, norm_or_metric, mode, match_param=0.85, precision=ops.VO_PREC_TF32X3, n_hyp=1024, seed=8214,
-                 thr_px=1.5, min_inliers=20, refine_iters=10):
+                 thr_px=1.5, min_inliers=20, refine_iters=10, pnp_mode="throughput", ref_restarts=3, ref_iters=100,
+                 ref_confidence=0.99):
+        ops.pnp_mode_id(pnp_mode)
         self.kw = dict(norm_or_metric=norm_or_metric, mode=mode, match_param=match_param, precision=precision,
                        n_hyp=n_hyp, seed=seed, thr_px=thr_px, min_inliers=min_inliers, refine_iters=refine_iters)
+        if pnp_mode != "throughput":
+            self.kw.update(pnp_mode=pnp_mode, ref_restarts=ref_restarts, ref_iters=ref_iters, ref_confidence=ref_confidence)
 
 
 _LANE_STREAMS = {}
