@@ -445,105 +445,35 @@ __device__ bool solve6(const double Hu[21], const double g[6], double x[6]) {
     return true;
 }
 
-__global__ void __launch_bounds__(RF_THREADS)
-refit_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, const int32_t *__restrict__ n_pts, int cap,
-             const float *__restrict__ poses, int H, IntrF kf, IntrD kd, float thr, int min_inliers, int iters,
-             const unsigned long long *__restrict__ bestkey, double *__restrict__ rt_out,
-             double *__restrict__ rvec_tvec, double *__restrict__ T_rel, int32_t *__restrict__ n_inl_out,
-             int32_t *__restrict__ best_h_out, uint8_t *__restrict__ mask_out, int32_t *__restrict__ status,
-             int accumulate_status) {
-    const int b = blockIdx.x;
-    const int n = min(n_pts[b], cap);
-    const unsigned long long key = bestkey[b];
-    const int count = (int)(uint32_t)(key >> 32);
-    const int h = (int)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
-    const bool have = (n >= 4) && (key != 0ull) && (count > min_inliers);
+// Shared state of refit_pose; the kernel declares it __shared__.
+struct RefitShared {
+    double R[9], t[3];                    // current pose, seeded with the winning minimal model
+    double Rp[9], tp[3], cost;            // last accepted pose and its cost
+    double acc[RF_THREADS / 32][RF_ACC];  // per-warp partial sums of the normal equations
+    int stop, bad;
+};
+
+// Gauss-Newton with a guard (the refined pose is chained into every later global pose, so it must never be worse
+// than what RANSAC found): every pass evaluates the cost at the current pose first; a pose that is not finite or
+// whose cost exceeds that of the last accepted pose is dropped for the last accepted one (at worst the minimal
+// model itself) and the iteration stops.  One extra evaluate-only pass checks the last step.
+// inlier(i, X, Y, Z, u, v) fetches correspondence i < n and says whether it is an inlier of the winning minimal model; only
+// those enter the refit.  On entry s.R / s.t hold that model and s.stop = s.bad = 0, visible to every thread.  On return
+// s.R / s.t hold the refined pose; a minimal model that is not finite sets s.bad and leaves the identity there instead (for
+// thread 0, which writes the outputs).
+template <class Inlier>
+__device__ __forceinline__ void refit_pose(RefitShared &s, int n, int iters, IntrD kd, const Inlier &inlier) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const float *pxyz = xyz + (size_t)b * cap * 3;
-    const float *puv = uv + (size_t)b * cap * 2;
-
-    __shared__ double sR[9], st[3], sRp[9], stp[3], s_cost;
-    __shared__ double sacc[RF_THREADS / 32][RF_ACC];
-    __shared__ int s_stop, s_bad;
-
-    if (!have) {
-        if (mask_out)
-            for (int i = threadIdx.x; i < cap; i += RF_THREADS) mask_out[(size_t)b * cap + i] = 0;
-        if (threadIdx.x == 0) {
-            int stt = (status && accumulate_status) ? status[b] : 0;
-            stt |= (n < 4) ? VO_ST_TOO_FEW_POINTS : VO_ST_NO_MODEL;
-            if (status) status[b] = stt;
-            if (n_inl_out) n_inl_out[b] = (n >= 4 && key != 0ull) ? count : 0;
-            if (best_h_out) best_h_out[b] = (n >= 4 && key != 0ull) ? h : -1;
-            for (int j = 0; j < 16; ++j) {
-                if (T_rel) T_rel[(size_t)b * 16 + j] = (j % 5 == 0) ? 1.0 : 0.0;
-            }
-            for (int j = 0; j < 12; ++j)
-                if (rt_out) rt_out[(size_t)b * 12 + j] = (j == 0 || j == 4 || j == 8) ? 1.0 : 0.0;
-            for (int j = 0; j < 6; ++j)
-                if (rvec_tvec) rvec_tvec[(size_t)b * 6 + j] = 0.0;
-        }
-        return;
-    }
-
-    PoseF p;
-    {
-        const float *src = poses + ((size_t)b * H + h) * 12;
-        for (int j = 0; j < 9; ++j) p.r[j] = src[j];
-        for (int j = 0; j < 3; ++j) p.t[j] = src[9 + j];
-    }
-    const ScoreModel sm = score_model(p, kf);
-    if (threadIdx.x == 0) {
-        // f64 start: the winning fp32 pose, rotation re-orthonormalised by two Newton polar steps
-        double R[9];
-        for (int j = 0; j < 9; ++j) R[j] = (double)p.r[j];
-        for (int it = 0; it < 2; ++it) {
-            double G[9];  // G = R^T R
-            for (int i = 0; i < 3; ++i)
-                for (int j = 0; j < 3; ++j) G[3 * i + j] = R[i] * R[j] + R[3 + i] * R[3 + j] + R[6 + i] * R[6 + j];
-            double N[9];  // R (3I - G) / 2
-            for (int i = 0; i < 3; ++i)
-                for (int j = 0; j < 3; ++j) {
-                    double s = 0.0;
-                    for (int q = 0; q < 3; ++q) s += R[3 * i + q] * ((q == j ? 3.0 : 0.0) - G[3 * q + j]);
-                    N[3 * i + j] = 0.5 * s;
-                }
-            for (int j = 0; j < 9; ++j) R[j] = N[j];
-        }
-        for (int j = 0; j < 9; ++j) sR[j] = R[j];
-        for (int j = 0; j < 3; ++j) st[j] = (double)p.t[j];
-        s_stop = 0;
-        s_bad = 0;
-    }
-    // inlier mask of the winning minimal model: identical arithmetic to score_kernel
-    // (per-thread flags are recomputed in the refit loop instead of being stored per point)
-    if (mask_out) {
-        for (int i = threadIdx.x; i < cap; i += RF_THREADS) {
-            uint8_t m = 0;
-            if (i < n) {
-                m = is_inlier(sm, thr, pxyz[i * 3], pxyz[i * 3 + 1], pxyz[i * 3 + 2], VO_FSUBF(puv[i * 2], kf.cx),
-                              VO_FSUBF(puv[i * 2 + 1], kf.cy)) ? 1 : 0;
-            }
-            mask_out[(size_t)b * cap + i] = m;
-        }
-    }
-    __syncthreads();
-
-    // Gauss-Newton with a guard (the refined pose is chained into every later global pose, so it must never be worse
-    // than what RANSAC found): every pass evaluates the cost at the current pose first; a pose that is not finite or
-    // whose cost exceeds that of the last accepted pose is dropped for the last accepted one (at worst the minimal
-    // model itself) and the iteration stops.  One extra evaluate-only pass checks the last step.
     for (int it = 0; it <= iters; ++it) {
         double acc[RF_ACC];
 #pragma unroll
         for (int j = 0; j < RF_ACC; ++j) acc[j] = 0.0;
         double R[9], t[3];
-        for (int j = 0; j < 9; ++j) R[j] = sR[j];
-        for (int j = 0; j < 3; ++j) t[j] = st[j];
+        for (int j = 0; j < 9; ++j) R[j] = s.R[j];
+        for (int j = 0; j < 3; ++j) t[j] = s.t[j];
         for (int i = threadIdx.x; i < n; i += RF_THREADS) {
-            const float Xf = pxyz[i * 3], Yf = pxyz[i * 3 + 1], Zf = pxyz[i * 3 + 2];
-            const float uf = puv[i * 2], vf = puv[i * 2 + 1];
-            if (!is_inlier(sm, thr, Xf, Yf, Zf, VO_FSUBF(uf, kf.cx), VO_FSUBF(vf, kf.cy))) continue;
+            float Xf, Yf, Zf, uf, vf;
+            if (!inlier(i, Xf, Yf, Zf, uf, vf)) continue;
             const double X = Xf, Y = Yf, Z = Zf;
             const double xr = R[0] * X + R[1] * Y + R[2] * Z;
             const double yr = R[3] * X + R[4] * Y + R[5] * Z;
@@ -568,33 +498,33 @@ refit_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, const 
         }
 #pragma unroll
         for (int j = 0; j < RF_ACC; ++j) {
-            const double s = warp_sum(acc[j]);
-            if (lane == 0) sacc[warp][j] = s;
+            const double v = warp_sum(acc[j]);
+            if (lane == 0) s.acc[warp][j] = v;
         }
         __syncthreads();
         if (threadIdx.x == 0) {
             double tot[RF_ACC];
             for (int j = 0; j < RF_ACC; ++j) {
-                double s = 0.0;
-                for (int w = 0; w < RF_THREADS / 32; ++w) s += sacc[w][j];
-                tot[j] = s;
+                double v = 0.0;
+                for (int w = 0; w < RF_THREADS / 32; ++w) v += s.acc[w][j];
+                tot[j] = v;
             }
             const double cost = tot[27];
             bool finite = cost == cost && cost < 1e300;
-            for (int j = 0; j < 9; ++j) finite = finite && sR[j] == sR[j] && fabs(sR[j]) < 2.0;
-            for (int j = 0; j < 3; ++j) finite = finite && st[j] == st[j] && fabs(st[j]) < 1e300;
-            if (it == 0 && !finite) {        // the minimal model itself is unusable: report "no model" below
-                s_bad = 1;
-                s_stop = 1;
-            } else if (it > 0 && !(finite && cost <= s_cost * (1.0 + 1e-12))) {   // worse than the last accepted pose: take that one back
-                for (int j = 0; j < 9; ++j) sR[j] = sRp[j];
-                for (int j = 0; j < 3; ++j) st[j] = stp[j];
-                s_stop = 1;
+            for (int j = 0; j < 9; ++j) finite = finite && s.R[j] == s.R[j] && fabs(s.R[j]) < 2.0;
+            for (int j = 0; j < 3; ++j) finite = finite && s.t[j] == s.t[j] && fabs(s.t[j]) < 1e300;
+            if (it == 0 && !finite) {        // the minimal model itself is unusable: report "no model"
+                s.bad = 1;
+                s.stop = 1;
+            } else if (it > 0 && !(finite && cost <= s.cost * (1.0 + 1e-12))) {   // worse than the last accepted pose: take that one back
+                for (int j = 0; j < 9; ++j) s.R[j] = s.Rp[j];
+                for (int j = 0; j < 3; ++j) s.t[j] = s.tp[j];
+                s.stop = 1;
             } else {
-                s_cost = cost;
-                for (int j = 0; j < 9; ++j) sRp[j] = sR[j];
-                for (int j = 0; j < 3; ++j) stp[j] = st[j];
-                if (it == iters) s_stop = 1;
+                s.cost = cost;
+                for (int j = 0; j < 9; ++j) s.Rp[j] = s.R[j];
+                for (int j = 0; j < 3; ++j) s.tp[j] = s.t[j];
+                if (it == iters) s.stop = 1;
             }
             double g[6], d[6];
             for (int j = 0; j < 6; ++j) g[j] = -tot[21 + j];
@@ -604,52 +534,147 @@ refit_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, const 
                 tot[dq] += 1e-12 * tot[dq] + 1e-300;
                 dq += 6 - r;
             }
-            if (s_stop) {
+            if (s.stop) {
             } else if (solve6(tot, g, d)) {
                 double dR[9], Rn[9];
                 so3_exp(d, dR);
                 for (int i = 0; i < 3; ++i)
                     for (int j = 0; j < 3; ++j)
-                        Rn[3 * i + j] = dR[3 * i] * sR[j] + dR[3 * i + 1] * sR[3 + j] + dR[3 * i + 2] * sR[6 + j];
-                for (int j = 0; j < 9; ++j) sR[j] = Rn[j];
-                for (int j = 0; j < 3; ++j) st[j] += d[3 + j];
+                        Rn[3 * i + j] = dR[3 * i] * s.R[j] + dR[3 * i + 1] * s.R[3 + j] + dR[3 * i + 2] * s.R[6 + j];
+                for (int j = 0; j < 9; ++j) s.R[j] = Rn[j];
+                for (int j = 0; j < 3; ++j) s.t[j] += d[3 + j];
                 double mx = 0.0;
                 for (int j = 0; j < 6; ++j) mx = fmax(mx, fabs(d[j]));
-                if (mx < 1e-11) s_stop = 1;
+                if (mx < 1e-11) s.stop = 1;
             } else {
-                s_stop = 1;
+                s.stop = 1;
             }
         }
         __syncthreads();
-        if (s_stop) break;
+        if (s.stop) break;
+    }
+    if (threadIdx.x == 0 && s.bad) {
+        for (int j = 0; j < 9; ++j) s.R[j] = (j % 4 == 0) ? 1.0 : 0.0;
+        for (int j = 0; j < 3; ++j) s.t[j] = 0.0;
+    }
+}
+
+// The pose outputs of one pair: rt = [R|t], rvec_tvec = (Rodrigues vector, t), T_rel = [R|t]^-1.  A null output is skipped.
+// (The identity written through here gets T_rel[3], [7], [11] = -0.0; write_no_pose writes +0.0.)
+__device__ __forceinline__ void write_pose(const double *R, const double *t, double *rt, double *rvec_tvec, double *T_rel) {
+    if (rt) {
+        for (int j = 0; j < 9; ++j) rt[j] = R[j];
+        for (int j = 0; j < 3; ++j) rt[9 + j] = t[j];
+    }
+    if (rvec_tvec) {
+        double w[3];
+        so3_log(R, w);
+        for (int j = 0; j < 3; ++j) rvec_tvec[j] = w[j];
+        for (int j = 0; j < 3; ++j) rvec_tvec[3 + j] = t[j];
+    }
+    if (T_rel) {  // inverse of [R|t]: [R^T | -R^T t]  (pose.pose = pose.inv_pose, :143)
+        for (int i = 0; i < 3; ++i) {
+            for (int j = 0; j < 3; ++j) T_rel[4 * i + j] = R[3 * j + i];
+            T_rel[4 * i + 3] = -(R[i] * t[0] + R[3 + i] * t[1] + R[6 + i] * t[2]);
+        }
+        T_rel[12] = 0.0; T_rel[13] = 0.0; T_rel[14] = 0.0; T_rel[15] = 1.0;
+    }
+}
+
+// The pose outputs of a pair without a model: identity rotation, zero translation and Rodrigues vector.
+__device__ __forceinline__ void write_no_pose(double *rt, double *rvec_tvec, double *T_rel) {
+    for (int j = 0; j < 16; ++j)
+        if (T_rel) T_rel[j] = (j % 5 == 0) ? 1.0 : 0.0;
+    for (int j = 0; j < 12; ++j)
+        if (rt) rt[j] = (j == 0 || j == 4 || j == 8) ? 1.0 : 0.0;
+    for (int j = 0; j < 6; ++j)
+        if (rvec_tvec) rvec_tvec[j] = 0.0;
+}
+
+__global__ void __launch_bounds__(RF_THREADS)
+refit_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, const int32_t *__restrict__ n_pts, int cap,
+             const float *__restrict__ poses, int H, IntrF kf, IntrD kd, float thr, int min_inliers, int iters,
+             const unsigned long long *__restrict__ bestkey, double *__restrict__ rt_out,
+             double *__restrict__ rvec_tvec, double *__restrict__ T_rel, int32_t *__restrict__ n_inl_out,
+             int32_t *__restrict__ best_h_out, uint8_t *__restrict__ mask_out, int32_t *__restrict__ status,
+             int accumulate_status) {
+    const int b = blockIdx.x;
+    const int n = min(n_pts[b], cap);
+    const unsigned long long key = bestkey[b];
+    const int count = (int)(uint32_t)(key >> 32);
+    const int h = (int)(0xffffffffu - (uint32_t)(key & 0xffffffffull));
+    const bool have = (n >= 4) && (key != 0ull) && (count > min_inliers);
+    const float *pxyz = xyz + (size_t)b * cap * 3;
+    const float *puv = uv + (size_t)b * cap * 2;
+    if (rt_out) rt_out += (size_t)b * 12;
+    if (rvec_tvec) rvec_tvec += (size_t)b * 6;
+    if (T_rel) T_rel += (size_t)b * 16;
+    if (mask_out) mask_out += (size_t)b * cap;
+
+    __shared__ RefitShared s;
+
+    if (!have) {
+        if (mask_out)
+            for (int i = threadIdx.x; i < cap; i += RF_THREADS) mask_out[i] = 0;
+        if (threadIdx.x == 0) {
+            int stt = (status && accumulate_status) ? status[b] : 0;
+            stt |= (n < 4) ? VO_ST_TOO_FEW_POINTS : VO_ST_NO_MODEL;
+            if (status) status[b] = stt;
+            if (n_inl_out) n_inl_out[b] = (n >= 4 && key != 0ull) ? count : 0;
+            if (best_h_out) best_h_out[b] = (n >= 4 && key != 0ull) ? h : -1;
+            write_no_pose(rt_out, rvec_tvec, T_rel);
+        }
+        return;
     }
 
+    PoseF p;
+    {
+        const float *src = poses + ((size_t)b * H + h) * 12;
+        for (int j = 0; j < 9; ++j) p.r[j] = src[j];
+        for (int j = 0; j < 3; ++j) p.t[j] = src[9 + j];
+    }
+    const ScoreModel sm = score_model(p, kf);
     if (threadIdx.x == 0) {
-        if (s_bad) {                                              // non-finite minimal model: identity + VO_ST_NO_MODEL
-            for (int j = 0; j < 9; ++j) sR[j] = (j % 4 == 0) ? 1.0 : 0.0;
-            for (int j = 0; j < 3; ++j) st[j] = 0.0;
-            if (status) status[b] = (accumulate_status ? status[b] : 0) | VO_ST_NO_MODEL;
-        } else if (status && !accumulate_status) status[b] = VO_ST_OK;  // else: keep the soft bits set upstream
+        // f64 start: the winning fp32 pose, rotation re-orthonormalised by two Newton polar steps
+        double R[9];
+        for (int j = 0; j < 9; ++j) R[j] = (double)p.r[j];
+        for (int it = 0; it < 2; ++it) {
+            double G[9];  // G = R^T R
+            for (int i = 0; i < 3; ++i)
+                for (int j = 0; j < 3; ++j) G[3 * i + j] = R[i] * R[j] + R[3 + i] * R[3 + j] + R[6 + i] * R[6 + j];
+            double N[9];  // R (3I - G) / 2
+            for (int i = 0; i < 3; ++i)
+                for (int j = 0; j < 3; ++j) {
+                    double v = 0.0;
+                    for (int q = 0; q < 3; ++q) v += R[3 * i + q] * ((q == j ? 3.0 : 0.0) - G[3 * q + j]);
+                    N[3 * i + j] = 0.5 * v;
+                }
+            for (int j = 0; j < 9; ++j) R[j] = N[j];
+        }
+        for (int j = 0; j < 9; ++j) s.R[j] = R[j];
+        for (int j = 0; j < 3; ++j) s.t[j] = (double)p.t[j];
+        s.stop = 0;
+        s.bad = 0;
+    }
+    // identical arithmetic to score_kernel
+    auto inlier = [&](int i, float &X, float &Y, float &Z, float &u, float &v) {
+        X = pxyz[i * 3]; Y = pxyz[i * 3 + 1]; Z = pxyz[i * 3 + 2];
+        u = puv[i * 2]; v = puv[i * 2 + 1];
+        return is_inlier(sm, thr, X, Y, Z, VO_FSUBF(u, kf.cx), VO_FSUBF(v, kf.cy));
+    };
+    // inlier mask of the winning minimal model (the refit recomputes the flags instead of storing them per point)
+    if (mask_out)
+        for (int i = threadIdx.x; i < cap; i += RF_THREADS) {
+            float X, Y, Z, u, v;
+            mask_out[i] = (i < n && inlier(i, X, Y, Z, u, v)) ? 1 : 0;
+        }
+    __syncthreads();
+    refit_pose(s, n, iters, kd, inlier);
+    if (threadIdx.x == 0) {
+        if (status) status[b] = (accumulate_status ? status[b] : 0) | (s.bad ? VO_ST_NO_MODEL : VO_ST_OK);
         if (n_inl_out) n_inl_out[b] = count;
         if (best_h_out) best_h_out[b] = h;
-        if (rt_out) {
-            for (int j = 0; j < 9; ++j) rt_out[(size_t)b * 12 + j] = sR[j];
-            for (int j = 0; j < 3; ++j) rt_out[(size_t)b * 12 + 9 + j] = st[j];
-        }
-        if (rvec_tvec) {
-            double w[3];
-            so3_log(sR, w);
-            for (int j = 0; j < 3; ++j) rvec_tvec[(size_t)b * 6 + j] = w[j];
-            for (int j = 0; j < 3; ++j) rvec_tvec[(size_t)b * 6 + 3 + j] = st[j];
-        }
-        if (T_rel) {  // inverse of [R|t]: [R^T | -R^T t]  (pose.pose = pose.inv_pose, :143)
-            double *T = T_rel + (size_t)b * 16;
-            for (int i = 0; i < 3; ++i) {
-                for (int j = 0; j < 3; ++j) T[4 * i + j] = sR[3 * j + i];
-                T[4 * i + 3] = -(sR[i] * st[0] + sR[3 + i] * st[1] + sR[6 + i] * st[2]);
-            }
-            T[12] = 0.0; T[13] = 0.0; T[14] = 0.0; T[15] = 1.0;
-        }
+        write_pose(s.R, s.t, rt_out, rvec_tvec, T_rel);
     }
 }
 
@@ -1004,10 +1029,8 @@ ref_select_refit_kernel(const float *__restrict__ xyz, const float *__restrict__
                         int32_t *__restrict__ n_inl_out, int32_t *__restrict__ best_out, uint8_t *__restrict__ mask_out,
                         int32_t *__restrict__ status, int accumulate_status) {
     __shared__ int s_best[RP_MAX_RESTARTS], s_cnt[RP_MAX_RESTARTS], s_run[RP_MAX_RESTARTS];
-    __shared__ int s_r, s_h, s_stop, s_bad;
-    __shared__ double sR[9], st[3], sRp[9], stp[3], s_cost;
-    __shared__ double sacc[RF_THREADS / 32][RF_ACC];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    __shared__ int s_r, s_h;
+    __shared__ RefitShared s;
     const int pb = blockIdx.x, per = restarts * iters;
     const int n_chk = pn[pb];
     const bool bad_input = n_chk == RP_BAD;
@@ -1037,12 +1060,12 @@ ref_select_refit_kernel(const float *__restrict__ xyz, const float *__restrict__
             if (s_best[r] >= 0 && s_cnt[r] > best && s_cnt[r] > min_inliers) { best = s_cnt[r]; rsel = r; }
         s_r = rsel;
         s_h = rsel >= 0 ? s_best[rsel] : -1;
-        s_stop = 0;
-        s_bad = 0;
+        s.stop = 0;
+        s.bad = 0;
         if (rsel >= 0) {
             const double *p = poses + ((size_t)rsel * iters + s_h) * 12;
-            for (int j = 0; j < 9; ++j) sR[j] = p[j];
-            for (int j = 0; j < 3; ++j) st[j] = p[9 + j];
+            for (int j = 0; j < 9; ++j) s.R[j] = p[j];
+            for (int j = 0; j < 3; ++j) s.t[j] = p[9 + j];
         }
     }
     __syncthreads();
@@ -1055,19 +1078,14 @@ ref_select_refit_kernel(const float *__restrict__ xyz, const float *__restrict__
                 status[0] = (accumulate_status ? status[0] : 0) | VO_ST_NO_MODEL | (bad_input ? VO_ST_BAD_INPUT : 0);
             if (n_inl_out) n_inl_out[0] = 0;
             if (best_out) { best_out[0] = -1; best_out[1] = -1; best_out[2] = 0; }
-            for (int j = 0; j < 16; ++j)
-                if (T_rel) T_rel[j] = (j % 5 == 0) ? 1.0 : 0.0;
-            for (int j = 0; j < 12; ++j)
-                if (rt_out) rt_out[j] = (j == 0 || j == 4 || j == 8) ? 1.0 : 0.0;
-            for (int j = 0; j < 6; ++j)
-                if (rvec_tvec) rvec_tvec[j] = 0.0;
+            write_no_pose(rt_out, rvec_tvec, T_rel);
         }
         return;
     }
     const int32_t *b = boot + (size_t)rsel * cap;
     refpnp::Pose pm;                                        // the winning minimal model: its mask selects the refit's points
-    for (int j = 0; j < 9; ++j) pm.R[j] = sR[j];
-    for (int j = 0; j < 3; ++j) pm.t[j] = st[j];
+    for (int j = 0; j < 9; ++j) pm.R[j] = s.R[j];
+    for (int j = 0; j < 3; ++j) pm.t[j] = s.t[j];
     auto inlier = [&](int i, float &X, float &Y, float &Z, float &u, float &v) {
         const int idx = b[i];
         X = xyz[(size_t)idx * 3]; Y = xyz[(size_t)idx * 3 + 1]; Z = xyz[(size_t)idx * 3 + 2];
@@ -1079,119 +1097,12 @@ ref_select_refit_kernel(const float *__restrict__ xyz, const float *__restrict__
             float X, Y, Z, u, v;
             mask_out[i] = inlier(i, X, Y, Z, u, v) ? 1 : 0;
         }
-    for (int it = 0; it <= refine_iters; ++it) {             // same guarded Gauss-Newton as refit_kernel
-        double acc[RF_ACC];
-#pragma unroll
-        for (int j = 0; j < RF_ACC; ++j) acc[j] = 0.0;
-        double R[9], t[3];
-        for (int j = 0; j < 9; ++j) R[j] = sR[j];
-        for (int j = 0; j < 3; ++j) t[j] = st[j];
-        for (int i = threadIdx.x; i < n; i += RF_THREADS) {
-            float Xf, Yf, Zf, uf, vf;
-            if (!inlier(i, Xf, Yf, Zf, uf, vf)) continue;
-            const double X = Xf, Y = Yf, Z = Zf;
-            const double xr = R[0] * X + R[1] * Y + R[2] * Z;
-            const double yr = R[3] * X + R[4] * Y + R[5] * Z;
-            const double zr = R[6] * X + R[7] * Y + R[8] * Z;
-            const double xc = xr + t[0], yc = yr + t[1], zc = zr + t[2];
-            const double iz = 1.0 / zc;
-            const double x = xc * iz, y = yc * iz;
-            const double ru = kd.fx * x + kd.cx - (double)uf;
-            const double rv = kd.fy * y + kd.cy - (double)vf;
-            const double a0 = kd.fx * iz, a2 = -kd.fx * x * iz;
-            const double b1 = kd.fy * iz, b2 = -kd.fy * y * iz;
-            const double ju[6] = {a2 * yr, a0 * zr - a2 * xr, -a0 * yr, a0, 0.0, a2};
-            const double jv[6] = {-b1 * zr + b2 * yr, -b2 * xr, b1 * xr, 0.0, b1, b2};
-            int q = 0;
-#pragma unroll
-            for (int r = 0; r < 6; ++r)
-#pragma unroll
-                for (int c = r; c < 6; ++c) acc[q++] += ju[r] * ju[c] + jv[r] * jv[c];
-#pragma unroll
-            for (int r = 0; r < 6; ++r) acc[21 + r] += ju[r] * ru + jv[r] * rv;
-            acc[27] += ru * ru + rv * rv;
-        }
-#pragma unroll
-        for (int j = 0; j < RF_ACC; ++j) {
-            const double s = warp_sum(acc[j]);
-            if (lane == 0) sacc[warp][j] = s;
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            double tot[RF_ACC];
-            for (int j = 0; j < RF_ACC; ++j) {
-                double s = 0.0;
-                for (int w = 0; w < RF_THREADS / 32; ++w) s += sacc[w][j];
-                tot[j] = s;
-            }
-            const double cost = tot[27];
-            bool finite = cost == cost && cost < 1e300;
-            for (int j = 0; j < 9; ++j) finite = finite && sR[j] == sR[j] && fabs(sR[j]) < 2.0;
-            for (int j = 0; j < 3; ++j) finite = finite && st[j] == st[j] && fabs(st[j]) < 1e300;
-            if (it == 0 && !finite) {
-                s_bad = 1;
-                s_stop = 1;
-            } else if (it > 0 && !(finite && cost <= s_cost * (1.0 + 1e-12))) {
-                for (int j = 0; j < 9; ++j) sR[j] = sRp[j];
-                for (int j = 0; j < 3; ++j) st[j] = stp[j];
-                s_stop = 1;
-            } else {
-                s_cost = cost;
-                for (int j = 0; j < 9; ++j) sRp[j] = sR[j];
-                for (int j = 0; j < 3; ++j) stp[j] = st[j];
-                if (it == refine_iters) s_stop = 1;
-            }
-            double g[6], d[6];
-            for (int j = 0; j < 6; ++j) g[j] = -tot[21 + j];
-            int dq = 0;
-            for (int r = 0; r < 6; ++r) {
-                tot[dq] += 1e-12 * tot[dq] + 1e-300;
-                dq += 6 - r;
-            }
-            if (s_stop) {
-            } else if (solve6(tot, g, d)) {
-                double dR[9], Rn[9];
-                so3_exp(d, dR);
-                for (int i = 0; i < 3; ++i)
-                    for (int j = 0; j < 3; ++j)
-                        Rn[3 * i + j] = dR[3 * i] * sR[j] + dR[3 * i + 1] * sR[3 + j] + dR[3 * i + 2] * sR[6 + j];
-                for (int j = 0; j < 9; ++j) sR[j] = Rn[j];
-                for (int j = 0; j < 3; ++j) st[j] += d[3 + j];
-                double mx = 0.0;
-                for (int j = 0; j < 6; ++j) mx = fmax(mx, fabs(d[j]));
-                if (mx < 1e-11) s_stop = 1;
-            } else {
-                s_stop = 1;
-            }
-        }
-        __syncthreads();
-        if (s_stop) break;
-    }
+    refit_pose(s, n, refine_iters, kd, inlier);
     if (threadIdx.x == 0) {
-        if (s_bad) {
-            for (int j = 0; j < 9; ++j) sR[j] = (j % 4 == 0) ? 1.0 : 0.0;
-            for (int j = 0; j < 3; ++j) st[j] = 0.0;
-        }
-        if (status) status[0] = (accumulate_status ? status[0] : 0) | (s_bad ? VO_ST_NO_MODEL : VO_ST_OK);
+        if (status) status[0] = (accumulate_status ? status[0] : 0) | (s.bad ? VO_ST_NO_MODEL : VO_ST_OK);
         if (n_inl_out) n_inl_out[0] = s_cnt[rsel];
         if (best_out) { best_out[0] = rsel; best_out[1] = hsel; best_out[2] = s_run[rsel]; }
-        if (rt_out) {
-            for (int j = 0; j < 9; ++j) rt_out[j] = sR[j];
-            for (int j = 0; j < 3; ++j) rt_out[9 + j] = st[j];
-        }
-        if (rvec_tvec) {
-            double w[3];
-            so3_log(sR, w);
-            for (int j = 0; j < 3; ++j) rvec_tvec[j] = w[j];
-            for (int j = 0; j < 3; ++j) rvec_tvec[3 + j] = st[j];
-        }
-        if (T_rel) {  // inverse of [R|t]: [R^T | -R^T t]  (pose.pose = pose.inv_pose, :143)
-            for (int i = 0; i < 3; ++i) {
-                for (int j = 0; j < 3; ++j) T_rel[4 * i + j] = sR[3 * j + i];
-                T_rel[4 * i + 3] = -(sR[i] * st[0] + sR[3 + i] * st[1] + sR[6 + i] * st[2]);
-            }
-            T_rel[12] = 0.0; T_rel[13] = 0.0; T_rel[14] = 0.0; T_rel[15] = 1.0;
-        }
+        write_pose(s.R, s.t, rt_out, rvec_tvec, T_rel);
     }
 }
 
