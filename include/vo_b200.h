@@ -27,9 +27,11 @@
 extern "C" {
 #endif
 
-#define VO_ABI_VERSION 3   /* 2: vo_pipeline_args.u8_bytes, vo_pnp_ransac_ref, VO_NORM_HAMMING_TC, vo_orb_debug_read
+#define VO_ABI_VERSION 4   /* 2: vo_pipeline_args.u8_bytes, vo_pnp_ransac_ref, VO_NORM_HAMMING_TC, vo_orb_debug_read
                              3: vo_bootstrap, vo_pnp_ransac_ref_batch, VO_ST_BAD_INPUT, the pnp_mode / ref_* fields of
-                                vo_pipeline_args and vo_seq_config */
+                                vo_pipeline_args and vo_seq_config
+                             4: vo_seq_config.n_seqs / seeds, vo_seq_push_all, vo_seq_read_at, vo_seq_frames_at, vo_seq_graph_captures,
+                                vo_workspace_generation */
 
 #if defined(__GNUC__)
 #define VO_API __attribute__((visibility("default")))
@@ -94,6 +96,9 @@ VO_API int vo_abi_version(void);
 VO_API const char *vo_last_error(void);
 /* Number of this library's kernels launched through `ctx` since creation. */
 VO_API long long vo_launch_count(const vo_ctx *ctx);
+/* Number of workspace (re)allocations of `ctx` since creation (VERSION 4).  Each one frees the old block, so work captured
+ * before it (a CUDA graph holding workspace pointers) is stale once this value has changed. */
+VO_API unsigned long long vo_workspace_generation(const vo_ctx *ctx);
 
 /* Optional raw k-NN outputs shared by both matchers (any pointer may be NULL).
  *   row_idx  int32 [B][n_stride][2]  nearest / second-nearest cur index (-1 if absent)
@@ -285,6 +290,23 @@ VO_API int vo_pipeline(vo_ctx *ctx, const vo_pipeline_args *args, void *stream);
  *                                  reference stores in global_poses (:293)
  *     info_h   int32  [count][6]   status bits | n_matches | n_corr ("common_pts") | n_inl |
  *                                  keyframe id the frame was matched against | 1 if it became the keyframe
+ *
+ * S independent sequences in lock-step (VERSION 4): n_seqs = S > 1 makes one loop of S sequences whose step is ONE
+ * vo_pipeline batch of B = S pairs (sequence q's current frame against its own keyframe); the policy and the promotion
+ * run per sequence on the device and never look at a neighbour.  Sequence q draws its hypotheses / bootstrap rows from
+ * (seeds[q], its history slot - 1), so its poses and info equal, bit for bit, those of a one-sequence loop created with
+ * seed = seeds[q] and fed the same frames.
+ *   vo_seq_push_all: desc (uint8 [S][n_cap][32] or float [S][n_cap][128]), kp float [S][n_cap][kp_stride], depth float
+ *   [S][H][W], device or (pinned) host memory, each copied with one cudaMemcpyAsync; n_kp_h, frame_id_h host int32 [S],
+ *   read before the call returns.  n_kp_h[q] < 0: sequence q has no frame at this step (its state is not touched); a
+ *   sequence's first frame installs its keyframe whenever it arrives.  Every check (counts <= n_cap, no pushing sequence's
+ *   history full) comes before anything is enqueued: one bad sequence refuses the whole step.
+ *   vo_seq_read_at / vo_seq_frames_at: vo_seq_read / vo_seq_frames of sequence q.  vo_seq_push, vo_seq_read and
+ *   vo_seq_frames act on sequence 0; vo_seq_push on a loop with S > 1 is an error.
+ * VO_SEQ_GRAPH=1 (environment, Mode T only): every step after the first one that ran the pipeline is one CUDA-graph
+ * launch.  The graph holds the vo_ctx workspace pointers; when any call on the same vo_ctx has reallocated a workspace
+ * since capture, the next step re-captures.  vo_seq_graph_captures: how many times the loop captured its step (0 when
+ * it launches plainly; one more for every re-capture).  n_seqs is at most 65535.
  */
 typedef struct vo_seq vo_seq;
 typedef struct vo_seq_config {
@@ -311,6 +333,9 @@ typedef struct vo_seq_config {
     int pnp_mode;
     int ref_restarts, ref_iters;
     double ref_confidence;
+    /* sequences in lock-step (VERSION 4): 0 or 1 = one sequence */
+    int n_seqs;
+    const uint64_t *seeds;      /* host uint64 [n_seqs] (copied at create); NULL = seed + q */
 } vo_seq_config;
 VO_API int vo_seq_create(vo_ctx *ctx, const vo_seq_config *cfg, vo_seq **out);
 VO_API void vo_seq_destroy(vo_seq *seq);
@@ -318,6 +343,11 @@ VO_API int vo_seq_push(vo_seq *seq, const void *desc, const float *kp, int n_kp,
                 void *stream);
 VO_API int vo_seq_frames(const vo_seq *seq);
 VO_API int vo_seq_read(vo_seq *seq, int first, int count, double *poses_h, int32_t *info_h, void *stream);
+VO_API int vo_seq_push_all(vo_seq *seq, const void *desc, const float *kp, const int32_t *n_kp_h, const float *depth,
+                    const int32_t *frame_id_h, void *stream);
+VO_API int vo_seq_frames_at(const vo_seq *seq, int q);
+VO_API int vo_seq_read_at(vo_seq *seq, int q, int first, int count, double *poses_h, int32_t *info_h, void *stream);
+VO_API int vo_seq_graph_captures(const vo_seq *seq);
 
 /*
  * "Same" 2-D convolution on the tensor cores (3xTF32 implicit GEMM; TMA zero fill is the padding): the layer type of

@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("VO_B200_LIB") or os.path.join(_HERE, "libvo_b200.so")   # (override: A/B runs of two builds)
 
 # ---- constants mirrored from include/vo_b200.h ---------------------------------------------
-VO_ABI_VERSION = 3
+VO_ABI_VERSION = 4
 VO_OK, VO_ERR_ARG, VO_ERR_CUDA, VO_ERR_UNSUPPORTED = 0, -1, -2, -3
 VO_ST_OK, VO_ST_NO_MODEL, VO_ST_TOO_FEW_POINTS, VO_ST_KP_OUT_OF_IMAGE, VO_ST_BAD_INPUT = 0, 1, 2, 4, 8
 VO_NORM_HAMMING, VO_NORM_L2_U8, VO_NORM_HAMMING_TC = 0, 1, 2
@@ -77,6 +77,8 @@ class SeqConfig(ctypes.Structure):
         ("pnp_mode", c_int),
         ("ref_restarts", c_int), ("ref_iters", c_int),
         ("ref_confidence", c_double),
+        ("n_seqs", c_int),
+        ("seeds", c_void_p),
     ]
 
 
@@ -105,6 +107,7 @@ PROTOTYPES = {
     "vo_abi_version": (c_int, []),
     "vo_last_error": (ctypes.c_char_p, []),
     "vo_launch_count": (ctypes.c_longlong, [c_void_p]),
+    "vo_workspace_generation": (ctypes.c_ulonglong, [c_void_p]),
     "vo_match_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_int,
                             c_int, c_double, c_void_p, c_void_p, c_void_p, ctypes.POINTER(KnnOut), c_void_p]),
     "vo_match_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_int,
@@ -132,6 +135,10 @@ PROTOTYPES = {
     "vo_seq_push": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p]),
     "vo_seq_frames": (c_int, [c_void_p]),
     "vo_seq_read": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "vo_seq_push_all": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vo_seq_frames_at": (c_int, [c_void_p, c_int]),
+    "vo_seq_read_at": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "vo_seq_graph_captures": (c_int, [c_void_p]),
     "vo_conv2d": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int,
                           c_void_p, c_void_p]),
     "vo_r2d2_create": (c_int, [c_void_p, ctypes.POINTER(R2d2Config), ctypes.POINTER(c_void_p)]),

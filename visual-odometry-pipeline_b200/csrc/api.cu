@@ -29,6 +29,7 @@ int ws_get(vo_ctx *ctx, int slot, size_t bytes, void **out) {
         }
         size_t cap = bytes + bytes / 4;
         cap = (cap + 255) & ~(size_t)255;
+        ctx->ws_gen++;
         VO_CUDA(cudaMalloc(&ctx->ws[slot], cap));
         ctx->ws_bytes[slot] = cap;
     }
@@ -73,6 +74,7 @@ int pick_split(vo_ctx *ctx, int B, int row_blocks, int col_tiles, int min_tiles_
 extern "C" int vo_abi_version(void) { return VO_ABI_VERSION; }
 extern "C" const char *vo_last_error(void) { return vo::get_error(); }
 extern "C" long long vo_launch_count(const vo_ctx *ctx) { return ctx ? ctx->launches : 0; }
+extern "C" unsigned long long vo_workspace_generation(const vo_ctx *ctx) { return ctx ? ctx->ws_gen : 0; }
 
 extern "C" int vo_create(int device, vo_ctx **out) {
     using namespace vo;
@@ -190,9 +192,9 @@ extern "C" int vo_match_f32(vo_ctx *ctx, const float *ref, const float *cur, int
 // ---------------------------------------------------------------- whole-path pipeline
 extern "C" int vo_pipeline(vo_ctx *ctx, const vo_pipeline_args *a, void *stream) { return vo::pipeline_impl(ctx, a, stream, nullptr); }
 
-// pair0_dev (optional, device): the hypothesis / bootstrap generator's pair offset read on the device instead of a->pair0
-// (vo_seq_*'s graph)
-int vo::pipeline_impl(vo_ctx *ctx, const vo_pipeline_args *a, void *stream, const long long *pair0_dev) {
+// keys (optional, device vo_pair_key[B]): the hypothesis / bootstrap generator key of each pair, read on the device instead of
+// (a->seed, a->pair0 + b) (vo_seq_*: one key per sequence)
+int vo::pipeline_impl(vo_ctx *ctx, const vo_pipeline_args *a, void *stream, const vo_pair_key *keys) {
     using namespace vo;
     VO_REQUIRE(ctx && a, "vo_pipeline: null argument");
     const bool u8 = a->ref_u8 && a->cur_u8, f32 = a->ref_f32 && a->cur_f32;
@@ -236,12 +238,12 @@ int vo::pipeline_impl(vo_ctx *ctx, const vo_pipeline_args *a, void *stream, cons
                                       stream)))
         return rc;
     if (ref) {
-        if ((rc = bootstrap_impl(ctx, a->n_corr, B, restarts, cap, a->seed, a->pair0, pair0_dev, hyp, stream))) return rc;
+        if ((rc = bootstrap_impl(ctx, a->n_corr, B, restarts, cap, a->seed, a->pair0, keys, hyp, stream))) return rc;
         return pnp_ransac_ref_impl(ctx, xyz, cuv, a->n_corr, 0, B, cap, a->K_h, hyp, restarts, iters, a->thr_px, confidence,
                                    a->min_inliers, a->refine_iters, a->rt, nullptr, a->T_rel, a->n_inl, nullptr, nullptr, nullptr,
                                    nullptr, a->status, 1, stream);
     }
-    if ((rc = hypotheses_impl(ctx, a->n_corr, B, H, a->seed, a->pair0, pair0_dev, hyp, stream))) return rc;
+    if ((rc = hypotheses_impl(ctx, a->n_corr, B, H, a->seed, a->pair0, keys, hyp, stream))) return rc;
     return pnp_ransac_impl(ctx, xyz, cuv, a->n_corr, B, cap, a->K_h, hyp, H, a->thr_px, a->min_inliers,
                            a->refine_iters, a->rt, nullptr, a->T_rel, a->n_inl, nullptr, nullptr, nullptr, a->status,
                            1, stream);

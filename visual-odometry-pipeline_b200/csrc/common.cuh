@@ -106,6 +106,9 @@ struct vo_ctx {
     void *encode_tiled;  // PFN_cuTensorMapEncodeTiled
     void *prof;          // vo::Profiler* when profiling was ever enabled
     int prof_on;
+    // bumped by every workspace (re)allocation: a CUDA graph that baked in ws pointers is stale once it differs from the
+    // value stored at capture
+    unsigned long long ws_gen;
 };
 
 namespace vo {
@@ -141,11 +144,18 @@ int match_bits_tc(vo_ctx *ctx, const uint8_t *ref, const uint8_t *cur, int B, in
                   const int32_t *n_cur, int need_cols, int need_second, vo_row_partial **part_out, int *n_split_out,
                   unsigned long long *colkey, cudaStream_t st);
 int pick_split(vo_ctx *ctx, int B, int row_blocks, int col_tiles, int min_tiles_per_split);
-int hypotheses_impl(vo_ctx *ctx, const int32_t *n_pts, int B, int H, uint64_t seed, int64_t pair0, const long long *pair0_dev,
+// Generator key of one pair: hypotheses and bootstrap rows of pair b are drawn from (keys[b].seed, keys[b].pair).  The
+// *_impl entries take an optional device array keys[B]; NULL means (seed, pair0 + b).  The keyframe loop passes one key per
+// sequence (its own seed, its history slot - 1), written on the device, so a captured graph replays with fresh keys.
+struct vo_pair_key {
+    uint64_t seed;
+    int64_t pair;
+};
+int hypotheses_impl(vo_ctx *ctx, const int32_t *n_pts, int B, int H, uint64_t seed, int64_t pair0, const vo_pair_key *keys,
                     int32_t *hyp, void *stream);
-int pipeline_impl(vo_ctx *ctx, const vo_pipeline_args *a, void *stream, const long long *pair0_dev);
+int pipeline_impl(vo_ctx *ctx, const vo_pipeline_args *a, void *stream, const vo_pair_key *keys);
 int bootstrap_impl(vo_ctx *ctx, const int32_t *n_pts, int B, int restarts, int cap, uint64_t seed, int64_t pair0,
-                   const long long *pair0_dev, int32_t *boot, void *stream);
+                   const vo_pair_key *keys, int32_t *boot, void *stream);
 int pnp_ransac_ref_impl(vo_ctx *ctx, const float *xyz, const float *uv, const int32_t *n_pts, int n_fixed, int B, int cap,
                         const double *K_h, const int32_t *boot_idx, int restarts, int iters, float thr_px, double confidence,
                         int min_inliers, int refine_iters, double *rt, double *rvec_tvec, double *T_rel, int32_t *n_inl,

@@ -21,16 +21,15 @@ struct IntrD {
 };
 
 // ---------------------------------------------------------------- hypothesis table
-// pair0_dev (optional): the pair offset read from device memory — a CUDA graph of the keyframe loop replays with a fresh offset
+// keys (optional): per-pair generator keys read from device memory (common.cuh: vo_pair_key); NULL = (seed, pair0 + b)
 __global__ void hypotheses_kernel(const int32_t *__restrict__ n_pts, int B, int H, uint64_t seed, int64_t pair0,
-                                  const long long *__restrict__ pair0_dev, int32_t *__restrict__ hyp) {
+                                  const vo_pair_key *__restrict__ keys, int32_t *__restrict__ hyp) {
     const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (gid >= (long long)B * H) return;
     const int b = (int)(gid / H), h = (int)(gid % H);
     const int n = n_pts[b];
     int32_t idx[4] = {-1, -1, -1, -1};
-    if (pair0_dev) pair0 = (int64_t)*pair0_dev;
-    if (n >= 4) draw_hypothesis(seed, pair0 + b, h, n, idx);
+    if (n >= 4) draw_hypothesis(keys ? keys[b].seed : seed, keys ? keys[b].pair : pair0 + b, h, n, idx);
     reinterpret_cast<int4 *>(hyp)[gid] = make_int4(idx[0], idx[1], idx[2], idx[3]);
 }
 
@@ -682,7 +681,7 @@ refit_kernel(const float *__restrict__ xyz, const float *__restrict__ uv, const 
 }  // namespace vo
 
 namespace vo {
-int hypotheses_impl(vo_ctx *ctx, const int32_t *n_pts, int B, int H, uint64_t seed, int64_t pair0, const long long *pair0_dev,
+int hypotheses_impl(vo_ctx *ctx, const int32_t *n_pts, int B, int H, uint64_t seed, int64_t pair0, const vo_pair_key *keys,
                     int32_t *hyp, void *stream) {
     VO_REQUIRE(ctx && n_pts && hyp, "vo_hypotheses: null argument");
     VO_REQUIRE(B >= 0 && H >= 0, "vo_hypotheses: negative size");
@@ -690,7 +689,7 @@ int hypotheses_impl(vo_ctx *ctx, const int32_t *n_pts, int B, int H, uint64_t se
     const long long total = (long long)B * H;
     if (total == 0) return VO_OK;
     VO_PROF(ctx, (cudaStream_t)stream, VO_STAGE_HYP);
-    hypotheses_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n_pts, B, H, seed, pair0, pair0_dev, hyp);
+    hypotheses_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n_pts, B, H, seed, pair0, keys, hyp);
     VO_LAUNCH_CHECK(ctx);
     VO_PROF(ctx, (cudaStream_t)stream, -1);
     return VO_OK;
@@ -1108,28 +1107,28 @@ ref_select_refit_kernel(const float *__restrict__ xyz, const float *__restrict__
 
 // ---------------------------------------------------------------- bootstrap rows
 // boot[b][r][i] = draw_bootstrap(seed, pair0 + b, r, i, n_pts[b]) for i < n_pts[b] (pnp_math.cuh: keyed like the hypotheses,
-// a pure function of the pair, not of its batch position), -1 for the padding i >= n_pts[b].
+// a pure function of the pair, not of its batch position), -1 for the padding i >= n_pts[b].  keys (optional) replaces
+// (seed, pair0 + b) by (keys[b].seed, keys[b].pair).
 __global__ void bootstrap_kernel(const int32_t *__restrict__ n_pts, int B, int restarts, int cap, uint64_t seed, int64_t pair0,
-                                 const long long *__restrict__ pair0_dev, int32_t *__restrict__ boot) {
+                                 const vo_pair_key *__restrict__ keys, int32_t *__restrict__ boot) {
     const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (gid >= (long long)B * restarts * cap) return;
     const int i = (int)(gid % cap), r = (int)((gid / cap) % restarts), b = (int)(gid / ((long long)cap * restarts));
     const int n = n_pts[b];
-    if (pair0_dev) pair0 = (int64_t)*pair0_dev;
-    boot[gid] = i < n ? draw_bootstrap(seed, pair0 + b, r, i, n) : -1;
+    boot[gid] = i < n ? draw_bootstrap(keys ? keys[b].seed : seed, keys ? keys[b].pair : pair0 + b, r, i, n) : -1;
 }
 
 }  // namespace
 
 int bootstrap_impl(vo_ctx *ctx, const int32_t *n_pts, int B, int restarts, int cap, uint64_t seed, int64_t pair0,
-                   const long long *pair0_dev, int32_t *boot, void *stream) {
+                   const vo_pair_key *keys, int32_t *boot, void *stream) {
     VO_REQUIRE(ctx && n_pts && boot, "vo_bootstrap: null argument");
     VO_REQUIRE(B >= 0 && restarts >= 0 && cap >= 0, "vo_bootstrap: negative size");
     const long long total = (long long)B * restarts * cap;
     if (total == 0) return VO_OK;
     VO_PROF(ctx, (cudaStream_t)stream, VO_STAGE_HYP);
     bootstrap_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n_pts, B, restarts, cap, seed, pair0,
-                                                                                      pair0_dev, boot);
+                                                                                      keys, boot);
     VO_LAUNCH_CHECK(ctx);
     VO_PROF(ctx, (cudaStream_t)stream, -1);
     return VO_OK;
