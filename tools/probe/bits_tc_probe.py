@@ -1,5 +1,4 @@
-"""Tensor-core Hamming pass at the c2 shape (B pairs of N x N 256-bit descriptors): time per call, and with VO_TC_DEBUG /
-VO_TC_TRACE set in the environment the kernel's own cycle accounting (stderr)."""
+"""Tensor-core Hamming pass at the c2 shape (B pairs of N x N 256-bit descriptors): time per call."""
 import os
 import sys
 
@@ -18,8 +17,6 @@ for norm in (ops.VO_NORM_HAMMING_TC, ops.VO_NORM_HAMMING):
     for _ in range(2):
         ops.match_u8(ref, cur, norm, ops.VO_MODE_MUTUAL, 0.0)
     torch.cuda.synchronize()
-    if os.environ.get("VO_TC_DEBUG") or os.environ.get("VO_TC_TRACE"):
-        break
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(10):

@@ -1,4 +1,4 @@
-"""Every kernel family of libvo_b200.so at small shapes, for compute-sanitizer (tools/sanitize.sh):
+"""Every kernel family of libvo_b200.so at small shapes, the case list that tests/test_gpu_small_shapes.py runs:
 all matcher precisions x acceptance rules (float and byte), raw k-NN output, ragged counts, the whole pipeline with
 pruned / sorted / unpruned scoring, dense back-projection, the device-resident keyframe loop, the ORB / SIFT front-ends.
 Usage: python tools/sanitize_cases.py [group ...]   groups: match_f32 match_u8 pipeline geometry seq orb sift conv"""

@@ -1,5 +1,4 @@
-"""Tuning helper (GPU box): time the tcgen05 matcher alone on c3-shaped input, with optional cycle accounting
-(VO_TC_DEBUG=1 prints one line per launch for CTA (0,0,0))."""
+"""Tuning helper (GPU box): time the tcgen05 matcher alone on c3-shaped input."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch

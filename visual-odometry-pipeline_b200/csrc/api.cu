@@ -69,6 +69,19 @@ int pick_split(vo_ctx *ctx, int B, int row_blocks, int col_tiles, int min_tiles_
     return n_split;
 }
 
+int ensure_encode(vo_ctx *ctx) {
+    if (ctx->encode_tiled) return VO_OK;
+    void *fn = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    VO_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
+    if (qres != cudaDriverEntryPointSuccess || !fn) {
+        set_error("cuTensorMapEncodeTiled is not available from this driver");
+        return VO_ERR_UNSUPPORTED;
+    }
+    ctx->encode_tiled = fn;
+    return VO_OK;
+}
+
 }  // namespace vo
 
 extern "C" int vo_abi_version(void) { return VO_ABI_VERSION; }

@@ -10,8 +10,8 @@ COMMON=(-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompi
         -Xptxas -v --expt-relaxed-constexpr)
 # pnp / orb / sift: no implicit FMA contraction, so the device rounds like the host restatements the parity tests use
 # (explicit fused operations, where OpenCV itself fuses, are spelled out with __fmaf_rn)
-# VO_TC_DBG=1 bash build.sh: the tensor-core matcher with its cycle counters compiled in (VO_TC_DEBUG / VO_TC_TRACE at run time)
-declare -A EXTRA=( [pnp]="-fmad=false" [orb]="-fmad=false" [sift]="-fmad=false" [match_f32_tc]="-DVO_TC_DBG=${VO_TC_DBG:-0} ${VO_TC_EXTRA:-}" )
+# VO_TC_EXTRA: extra nvcc flags for the tensor-core matcher, e.g. -DVO_TC_PERSIST_MAX_TILES=<n>
+declare -A EXTRA=( [pnp]="-fmad=false" [orb]="-fmad=false" [sift]="-fmad=false" [match_f32_tc]="${VO_TC_EXTRA:-}" )
 pids=()
 for src in api match_finalize match_u8 match_f32_simt match_f32_tc geometry pnp sequence conv_tc r2d2_net orb sift; do
   (

@@ -95,6 +95,7 @@ struct __align__(16) vo_row_partial {
 
 // ---- context ---------------------------------------------------------------
 #define VO_WS_SLOTS 10   /* = vo::WS_SLOTS (static_assert below) */
+#define VO_TC_PERSIST_KERNELS 6   /* persistent tensor-core matcher kernels: passes 16, 8, 9 x metric */
 struct vo_ctx {
     int device;
     int sm_count;
@@ -102,8 +103,8 @@ struct vo_ctx {
     // growable workspace regions (device)
     void *ws[VO_WS_SLOTS];
     size_t ws_bytes[VO_WS_SLOTS];
-    int tc_ready;  // tcgen05 path initialised (driver entry point resolved)
-    void *encode_tiled;  // PFN_cuTensorMapEncodeTiled
+    void *encode_tiled;  // PFN_encodeTiled, resolved by ensure_encode()
+    int tc_max_clusters[VO_TC_PERSIST_KERNELS];  // resident clusters of each persistent matcher kernel (0: not asked yet)
     void *prof;          // vo::Profiler* when profiling was ever enabled
     int prof_on;
     // bumped by every workspace (re)allocation: a CUDA graph that baked in ws pointers is stale once it differs from the
@@ -144,6 +145,8 @@ int match_bits_tc(vo_ctx *ctx, const uint8_t *ref, const uint8_t *cur, int B, in
                   const int32_t *n_cur, int need_cols, int need_second, vo_row_partial **part_out, int *n_split_out,
                   unsigned long long *colkey, cudaStream_t st);
 int pick_split(vo_ctx *ctx, int B, int row_blocks, int col_tiles, int min_tiles_per_split);
+// resolves cuTensorMapEncodeTiled into ctx->encode_tiled (once per context) for the TMA descriptors of the tcgen05 kernels
+int ensure_encode(vo_ctx *ctx);
 // Generator key of one pair: hypotheses and bootstrap rows of pair b are drawn from (keys[b].seed, keys[b].pair).  The
 // *_impl entries take an optional device array keys[B]; NULL means (seed, pair0 + b).  The keyframe loop passes one key per
 // sequence (its own seed, its history slot - 1), written on the device, so a captured graph replays with fresh keys.

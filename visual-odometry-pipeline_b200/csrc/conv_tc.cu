@@ -208,23 +208,6 @@ tf32_split_kernel(const float *__restrict__ x, size_t n4, float *__restrict__ hi
     }
 }
 
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                    const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-int ensure_encode(vo_ctx *ctx) {
-    if (ctx->encode_tiled) return VO_OK;
-    void *fn = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    VO_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-    if (qres != cudaDriverEntryPointSuccess || !fn) {
-        set_error("cuTensorMapEncodeTiled is not available from this driver");
-        return VO_ERR_UNSUPPORTED;
-    }
-    ctx->encode_tiled = fn;
-    return VO_OK;
-}
-
 }  // namespace
 
 // activation map: NHWC [H][W][C] viewed as a 3-D tensor (C, W, H), box {32, 128, 1}

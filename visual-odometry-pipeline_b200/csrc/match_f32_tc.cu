@@ -38,9 +38,6 @@
 #include <cuda_fp16.h>
 #include <stdlib.h>
 
-#ifndef VO_TC_DBG
-#define VO_TC_DBG 0
-#endif
 // Work items (row-block pair x column split x frame pair) with at most this many column tiles run on the persistent form of the
 // fp16 / fp8 passes: at 11 tiles (2k x 2k) the per-CTA set-up and drain is as long as the tiles, at 105 (20k x 20k) it is 2 %
 // and the plain form's steady state is 6 % faster (B200: 2k +9 %, 5k +5 % / +2 %, 20k -6 % persistent vs plain).
@@ -469,7 +466,7 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
                     const int32_t *__restrict__ n_ref, const int32_t *__restrict__ n_cur,
                     const float *__restrict__ row_norm, const float *__restrict__ col_norm, int n_split,
                     vo_row_partial *__restrict__ part, unsigned long long *__restrict__ colkey,
-                    long long *__restrict__ dbg, int pair_group, int row_elems, int lgrid_x, int n_pairs) {
+                    int pair_group, int row_elems, int lgrid_x, int n_pairs) {
     extern __shared__ uint8_t smem_raw[];
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     uint8_t *smem = smem_raw + (base - smem_u32(smem_raw));
@@ -529,17 +526,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
     };
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t crank = cluster_rank();
-    // optional cycle accounting of CTA (0,0,0) for bring-up / tuning (dbg == nullptr in production)
-    // (compiled in with -DVO_TC_DBG=1 only — VO_TC_DEBUG / VO_TC_TRACE at run time then; the counters cost a dozen registers
-    // that the persistent fp16 / fp8 epilogue cannot spare.  Persistent kernels: CTA 0, over all its items.)
-    const bool dbg_on = VO_TC_DBG && dbg != nullptr && rblock == 0 && blockIdx.y == 0 && b == 0;
-    const long long t_kernel0 = dbg_on ? clock64() : 0;
-    // VO_TC_TRACE: every CTA leaves (clock64 at entry, clock64 at exit, SM id) behind: idle time between CTAs of one SM
-    const bool trace_on = VO_TC_DBG && dbg != nullptr && dbg[15] == 1;
-    const long long t_trace0 = (trace_on && threadIdx.x == 0) ? clock64() : 0;
-#define TC_DBG_BEGIN() const long long _t0 = dbg_on ? clock64() : 0
-#define TC_DBG_END(slot) do { if (dbg_on) dbg_acc[slot] += clock64() - _t0; } while (0)
-    long long dbg_acc[4] = {0, 0, 0, 0};
 
     // single-pass L2: one extra box per tile carries -|b|^2 (three tf32 pieces), multiplied by a column block of ones in A
     constexpr bool F16 = Cfg::F16;
@@ -581,7 +567,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
     cluster_sync_all();  // the peer's barriers exist before anything multicasts into this CTA
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    if (dbg_on && threadIdx.x == 0) dbg[14] = clock64() - t_kernel0;   // set-up: barriers, TMEM, cluster rendezvous
 
     auto tile_of = [&](int lt) { return t_begin + lt; };
 
@@ -596,7 +581,7 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
                 for (int item = 0; item < ITEMS; ++item, ++it) {
                     const int stage = it % STAGES;
                     const uint32_t phase = (uint32_t)(it / STAGES) & 1u;
-                    { TC_DBG_BEGIN(); mbar_wait(bar_empty(stage), phase ^ 1u); TC_DBG_END(0); }  // both CTAs consumed the slot
+                    mbar_wait(bar_empty(stage), phase ^ 1u);  // both CTAs consumed the slot
                     const bool is_ext = EXT && item == NKB;  // map_b_lo is the extension map in that mode
                     mbar_expect_tx(bar_full(stage), is_ext ? BN * TC_EXT_K * 4 : BLOCK_BYTES);  // bytes arrive by multicast, whoever issues
                     if ((uint32_t)(it & 1) == crank) {
@@ -608,7 +593,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
                 }
             }
             }
-            if (dbg_on) dbg[4] = dbg_acc[0];
         }
     } else if (warp == TC_WARP_MMA) {
         // ===================== MMA issuer =====================
@@ -616,29 +600,22 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
         // constant upper word plus (smem address >> 4): one integer add per MMA, nothing else on the issue path.
         {
             uint32_t stage = 0, phase = 0, a_phase = 0;
-            long long mma_wait_full = 0, mma_wait_tempty = 0, mma_wait_a = 0;
             int gt = 0;  // tiles issued so far, over all items: accumulator buffer and its phase
             for (int w = w_first; w < w_end; w += w_step) {
             const Item I = item_at(w);
             if (I.n_tiles == 0) continue;
-            { const long long _t0 = dbg_on ? clock64() : 0;
-              mbar_wait(bar_a, a_phase);  // this item's A is in tensor memory
-              if (dbg_on) mma_wait_a += clock64() - _t0; }
+            mbar_wait(bar_a, a_phase);  // this item's A is in tensor memory
             a_phase ^= 1u;
             tc_fence_after();
             for (int lt = 0; lt < I.n_tiles; ++lt, ++gt) {
                 const int buf = gt & 1;
                 const uint32_t use = (uint32_t)(gt >> 1);
-                { const long long _t0 = dbg_on ? clock64() : 0;
-                  mbar_wait(bar_tempty(buf), (use & 1u) ^ 1u);  // epilogue has drained this accumulator
-                  if (dbg_on) mma_wait_tempty += clock64() - _t0; }
+                mbar_wait(bar_tempty(buf), (use & 1u) ^ 1u);  // epilogue has drained this accumulator
                 tc_fence_after();
                 const uint32_t d_tmem = tmem_base + (uint32_t)(buf * BN);
 #pragma unroll
                 for (int item = 0; item < ITEMS; ++item) {
-                    { const long long _t0 = dbg_on ? clock64() : 0;
-                      mbar_wait(bar_full(stage), phase);
-                      if (dbg_on) mma_wait_full += clock64() - _t0; }
+                    mbar_wait(bar_full(stage), phase);
                     tc_fence_after();
                     if (elect_one()) {
                         const int kb = THREE ? (item >> 1) : item;       // compile-time after unrolling
@@ -681,7 +658,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
                 }
             }
             }
-            if (dbg_on && lane == 0) { dbg[1] = mma_wait_full; dbg[2] = mma_wait_tempty; dbg[3] = clock64() - t_kernel0; dbg[11] = gt; dbg[12] = mma_wait_a; }
         }
     } else {
         if constexpr (Cfg::F16) {
@@ -691,7 +667,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
         // at once, and only then folds them into its row's top-2: the accumulator is blocked for one TMEM read, not
         // for the fold (with two 8-warp groups the fold time of a tile sat on the critical path of its buffer).
         constexpr int QW = BN / 4;
-        const bool edbg = VO_TC_DBG >= 2 && dbg_on;   // the epilogue counters cost registers the fp16 / fp8 epilogue spills for
         static_assert(QW == 48, "three 16-column reads per thread");
         const int cq = warp >> 2;
         const int q = warp & 3;
@@ -714,7 +689,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
         // once per item (pair, split, row block; the next item for the hand-over) is decoded again from w where it is used.
         int gt = 0;             // tiles consumed so far, over all items
         bool a_stored = false;  // the current item's A went in during the previous item's last tile
-        long long t_between = edbg ? clock64() : 0;
         for (int w = w_first; w < w_end; w += w_step) {
             int M, n_t, tile0;
             bool row_ok, partial_rows;
@@ -736,7 +710,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
             }
             float s1 = -INFINITY, s2 = -INFINITY, thr = -INFINITY;
             int32_t i1 = -1, i2 = -1;
-            if (edbg) dbg_acc[3] += clock64() - t_between;   // between the tile loops of consecutive items
             // One tile: wait for its accumulator (unless the hand-over below already did), read it, fold it.
             auto tile = [&](int lt, bool waited) {
                 const int buf = gt & 1;
@@ -744,10 +717,9 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
                 const int col0 = (tile0 + lt) * BN + cq * QW;
                 const bool full_tile = (tile0 + lt) * BN + BN <= M;
                 if (!waited) {
-                    { const long long _t0 = edbg ? clock64() : 0; mbar_wait(bar_tfull(buf), use & 1u); if (edbg) dbg_acc[0] += clock64() - _t0; }
+                    mbar_wait(bar_tfull(buf), use & 1u);
                     tc_fence_after();
                 }
-                const long long _tc0 = edbg ? clock64() : 0;
                 const uint32_t taddr = lane_base + (uint32_t)(buf * BN + cq * QW);
                 // 48 columns per thread through 32 registers (four groups of 8): columns 0..31 are read; as the first two groups
                 // are folded, columns 32..47 are read into their registers (the reads fly during the next group's fold), and
@@ -769,8 +741,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
                 tc_ld_wait8(g1);
                 tc_ld_wait8(g2);
                 tc_ld_wait8(g3);
-                if (edbg) dbg_acc[1] += clock64() - _tc0;
-                const long long _tm0 = edbg ? clock64() : 0;
 #define TC_FOLD8(BUF, J0, MASKC, MASKR)                                                                                    \
     {                                                                                                                      \
         float v[8];                                                                                                        \
@@ -795,7 +765,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
 #undef TC_FOLD48
 #undef TC_FOLD8
                 srow2[cq * TC_BM + rr] = Cfg::TOP1 ? s1 : s2;
-                if (edbg) dbg_acc[2] += clock64() - _tm0;
                 ++gt;
             };
             // all tiles but the last in a plain loop (the loop of the one-item-per-CTA kernel, and compiled like it); the last
@@ -815,7 +784,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
                 }
                 tile(n_t - 1, waited);
             }
-            if (edbg) t_between = clock64();
             if (METRIC == VO_METRIC_L2) {  // the deferred row norm (-inf stays -inf)
                 s1 = __fsub_rn(s1, na); s2 = __fsub_rn(s2, na);
             }
@@ -842,7 +810,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
                 asm volatile("bar.sync 1, 512;" ::: "memory");
             }
         }
-        if (edbg && q == 0 && lane == 0 && cq < 2) { dbg[5 + cq] = dbg_acc[0]; dbg[7 + cq] = dbg_acc[1]; dbg[9 + cq] = dbg_acc[2]; if (cq == 1) dbg[13] = dbg_acc[3]; }
         } else if constexpr (Cfg::ALLWARP_COLS) {
         // ===================== split-fp16 epilogue: all 16 warps on every tile, with the column side =====================
         // Same idea as the fp16 single pass: lane quarter q x column quarter cq (32 columns per thread), the tile slice
@@ -889,9 +856,8 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
             uint32_t *tile_cb = scol_b + buf * 4 * BN;
             float *my_cv = tile_cv + q * BN + cq * QW;
             uint32_t *my_cb = tile_cb + q * BN + cq * QW;
-            { TC_DBG_BEGIN(); mbar_wait(bar_tfull(buf), use & 1u); TC_DBG_END(0); }
+            mbar_wait(bar_tfull(buf), use & 1u);
             tc_fence_after();
-            const long long _tc0 = dbg_on ? clock64() : 0;
             const uint32_t taddr = lane_base + (uint32_t)(buf * BN + cq * QW);
             uint32_t ra[16], rb[16];
             tc_ld16_issue(taddr, ra);
@@ -918,8 +884,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
             tc_ld_wait16(rb);
             tc_fence_before();  // the tile slice is in registers: hand the accumulator back before folding
             if (lane == 0) mbar_arrive(bar_tempty(buf));
-            if (dbg_on) dbg_acc[1] += clock64() - _tc0;
-            const long long _tm0 = dbg_on ? clock64() : 0;
 #define TC_FOLD16(BUF, J0, MASKC, MASKR)                                                                                   \
     _Pragma("unroll") for (int u = 0; u < 2; ++u) {                                                                        \
         float v[8];                                                                                                        \
@@ -964,9 +928,7 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
                 // no second barrier: tile lt+1 writes the other scratch buffer, and tile lt+2 cannot be written before
                 // the merging warp has arrived at the barrier of tile lt+1, i.e. after it has read this one
             }
-            if (dbg_on) dbg_acc[2] += clock64() - _tm0;
         }
-        if (dbg_on && q == 0 && lane == 0 && cq < 2) { dbg[5 + cq] = dbg_acc[0]; dbg[7 + cq] = dbg_acc[1]; dbg[9 + cq] = dbg_acc[2]; }
         if (METRIC == VO_METRIC_L2 && !COLS) {  // the deferred row norm (-inf stays -inf)
             s1 = __fsub_rn(s1, na); s2 = __fsub_rn(s2, na);
         }
@@ -1032,9 +994,8 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
             uint32_t *tile_cb = grp_cb + (use & 1u) * 4 * BN;
             float *my_cv = tile_cv + q * BN;
             uint32_t *my_cb = tile_cb + q * BN;
-            { TC_DBG_BEGIN(); mbar_wait(bar_tfull(g), use & 1u); TC_DBG_END(0); }
+            mbar_wait(bar_tfull(g), use & 1u);
             tc_fence_after();
-            const long long _tc0 = dbg_on ? clock64() : 0;
             const uint32_t taddr = lane_base + (uint32_t)(g * BN);
             // Three epilogue schedules.  3xTF32 is bound by the tensor pipe: plain load -> wait -> fold.  Single pass is
             // bound by the epilogue, whose cost per 8 columns was the TMEM read latency, so the read of the next
@@ -1104,8 +1065,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
             }
             tc_fence_before();  // this warp's share of the accumulator has been read: hand it back
             if (lane == 0) mbar_arrive(bar_tempty(g));
-            if (dbg_on) dbg_acc[1] += clock64() - _tc0;
-            const long long _tm0 = dbg_on ? clock64() : 0;
             if (COLS) group_bar(1 + g);
             if (COLS && (h * 4 + q) * 32 < BN) {  // one column per thread, merge the 4 lane quarters (ascending rows)
                 const int j = (h * 4 + q) * 32 + lane;
@@ -1127,9 +1086,7 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
             }
             // no second barrier: the next tile of this group writes the other scratch buffer, and the one after
             // next cannot start before every warp has passed the barrier above again
-            if (dbg_on) dbg_acc[2] += clock64() - _tm0;
         }
-        if (dbg_on && q == 0 && h == 0 && lane == 0) { dbg[5 + g] = dbg_acc[0]; dbg[7 + g] = dbg_acc[1]; dbg[9 + g] = dbg_acc[2]; }
         // four warps (2 groups x 2 column halves) saw disjoint columns of each row: four partials, merged by finalize
         if (METRIC == VO_METRIC_L2 && !COLS) {  // the deferred row norm (-inf stays -inf)
             s1 = __fsub_rn(s1, na); s2 = __fsub_rn(s2, na);
@@ -1143,7 +1100,6 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
         }  // !F16
     }
 
-    if (dbg_on && threadIdx.x == 0) dbg[0] = clock64() - t_kernel0;
     tc_fence_before();
     __syncthreads();
     cluster_sync_all();  // nobody leaves while the peer can still multicast into / arrive on this CTA
@@ -1151,17 +1107,7 @@ match_f32_tc_kernel(const __grid_constant__ CUtensorMap map_b_hi, const __grid_c
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)TC_TMEM_COLS)
                      : "memory");
     }
-    if (trace_on && threadIdx.x == 0) {
-        uint32_t smid;
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-        long long *t = dbg + 16 + 3 * ((size_t)(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x);
-        t[0] = t_trace0; t[1] = clock64(); t[2] = smid;
-    }
 }
-
-typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                    const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 // [rows][row_elems] fp32 (or fp16 when `half`), box = 128 B of k x box_rows rows, SWIZZLE_128B
 int make_map(vo_ctx *ctx, CUtensorMap *map, const void *ptr, long long rows, int box_rows, int row_elems = TC_D,
@@ -1188,33 +1134,17 @@ int launch_tc_kern(vo_ctx *ctx, dim3 grid, const CUtensorMap &bh, const CUtensor
                    const float *col_norm, int n_split, vo_row_partial *part, unsigned long long *colkey, cudaStream_t st,
                    int row_elems) {
     auto kern = match_f32_tc_kernel<PASSES, METRIC, COLS, PERSIST>;
-    long long *dbg = nullptr;
-    const size_t n_ctas = (size_t)grid.x * grid.y * grid.z;
-    const bool trace = getenv("VO_TC_TRACE") != nullptr;
-    if (VO_TC_DBG && (getenv("VO_TC_DEBUG") || trace)) {  // bring-up only: cycle accounting of CTA (0,0,0), printed after a sync
-        static long long *dbg_dev = nullptr;
-        static size_t dbg_cap = 0;
-        const size_t need = 16 + (trace ? 3 * n_ctas : 0);
-        if (dbg_cap < need) {
-            if (dbg_dev) VO_CUDA(cudaFree(dbg_dev));
-            VO_CUDA(cudaMalloc(&dbg_dev, need * sizeof(long long)));
-            dbg_cap = need;
-        }
-        VO_CUDA(cudaMemsetAsync(dbg_dev, 0, 16 * sizeof(long long), st));
-        if (trace) {
-            const long long one = 1;
-            VO_CUDA(cudaMemcpyAsync(dbg_dev + 15, &one, sizeof(one), cudaMemcpyHostToDevice, st));
-        }
-        dbg = dbg_dev;
-    }
     VO_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<PASSES>::SMEM_BYTES));
     // split fp16 with the column side: interleave as many pairs as keep their current-frame descriptors (hi + lo fp16) in L2
     int pair_group = 1;
     if (TcCfg<PASSES>::ALLWARP_COLS && COLS && !getenv("VO_TC_NO_INTERLEAVE"))
         pair_group = (int)max(1ll, min(8ll, (64ll << 20) / ((long long)m_stride * TC_D * 4)));
     dim3 launch_grid = grid;
-    if (PERSIST) {  // persistent: one cluster per SM pair (as many as can be resident), each walks the logical grid
-        static int max_clusters = 0;
+    if constexpr (PERSIST) {  // persistent: one cluster per SM pair (as many as can be resident), each walks the logical grid
+        // resident clusters: asked once per kernel and context, since devices (and MIG slices) differ in SM count
+        constexpr int slot = 2 * (PASSES == 16 ? 0 : PASSES - 7) + (METRIC == VO_METRIC_COSINE ? 1 : 0);
+        static_assert(slot >= 0 && slot < VO_TC_PERSIST_KERNELS, "persistent passes 16, 8, 9 x metric");
+        int &max_clusters = ctx->tc_max_clusters[slot];
         if (max_clusters == 0) {
             cudaLaunchConfig_t cfg = {};
             cfg.gridDim = dim3(TC_CLUSTER * 64);
@@ -1237,43 +1167,8 @@ int launch_tc_kern(vo_ctx *ctx, dim3 grid, const CUtensorMap &bh, const CUtensor
         launch_grid = dim3((unsigned)(clusters * TC_CLUSTER), 1, 1);
     }
     kern<<<launch_grid, TC_THREADS, TcCfg<PASSES>::SMEM_BYTES, st>>>(bh, bl, a_hi, a_lo, n_stride, m_stride, n_ref, n_cur, row_norm, col_norm,
-                                                  n_split, part, colkey, dbg, pair_group, row_elems, (int)grid.x, (int)grid.z);
+                                                  n_split, part, colkey, pair_group, row_elems, (int)grid.x, (int)grid.z);
     VO_LAUNCH_CHECK(ctx);
-    if (dbg && trace) {  // per SM: busy cycles of its CTAs and the idle cycles between one CTA's exit and the next one's entry
-        VO_CUDA(cudaStreamSynchronize(st));
-        long long *h = (long long *)malloc(3 * n_ctas * sizeof(long long));
-        VO_CUDA(cudaMemcpy(h, dbg + 16, 3 * n_ctas * sizeof(long long), cudaMemcpyDeviceToHost));
-        double busy = 0, gap = 0;
-        long long n_gap = 0, max_gap = 0;
-        for (int sm = 0; sm < 256; ++sm) {
-            long long last_end = -1;
-            for (;;) {  // next CTA of this SM in start order (selection scan: a few thousand CTAs)
-                long long best = -1;
-                size_t bi = 0;
-                for (size_t i = 0; i < n_ctas; ++i)
-                    if (h[3 * i + 2] == sm && (last_end < 0 || h[3 * i] >= last_end) && (best < 0 || h[3 * i] < best)) {
-                        best = h[3 * i];
-                        bi = i;
-                    }
-                if (best < 0) break;
-                if (last_end >= 0) { gap += (double)(best - last_end); ++n_gap; if (best - last_end > max_gap) max_gap = best - last_end; }
-                busy += (double)(h[3 * bi + 1] - h[3 * bi]);
-                last_end = h[3 * bi + 1];
-            }
-        }
-        fprintf(stderr, "[vo tc trace] passes=%d ctas=%zu mean_cta_cycles=%.0f mean_gap_cycles=%.0f max_gap=%lld gaps=%lld\n", PASSES,
-                n_ctas, busy / (double)n_ctas, n_gap ? gap / (double)n_gap : 0.0, max_gap, n_gap);
-        free(h);
-    } else if (dbg) {
-        long long h[16];
-        VO_CUDA(cudaStreamSynchronize(st));
-        VO_CUDA(cudaMemcpy(h, dbg, sizeof(h), cudaMemcpyDeviceToHost));
-        fprintf(stderr,
-                "[vo tc dbg] passes=%d tiles=%lld cta_cycles=%lld | mma: wait_full=%lld wait_tempty=%lld total=%lld | "
-                "producer wait_empty=%lld | epi g0: wait_tfull=%lld chunks=%lld merge=%lld | g1: wait_tfull=%lld chunks=%lld merge=%lld | "
-                "mma wait_a=%lld, epi between items=%lld | set-up %lld | launch grid %u\n",
-                PASSES, h[11], h[0], h[1], h[2], h[3], h[4], h[5], h[7], h[9], h[6], h[8], h[10], h[12], h[13], h[14], launch_grid.x);
-    }
     return VO_OK;
 }
 
@@ -1305,23 +1200,13 @@ int match_f32_tc(vo_ctx *ctx, const float *ref, const float *cur, int B, int n_s
         set_error("match_f32_tc: byte descriptors (32 or 128 per row) run the fp16 single pass (L2, no column arg-min) only");
         return VO_ERR_ARG;
     }
-    if (!ctx->tc_ready) {
-        void *fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        VO_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-        if (qres != cudaDriverEntryPointSuccess || !fn) {
-            set_error("cuTensorMapEncodeTiled is not available from this driver");
-            return VO_ERR_UNSUPPORTED;
-        }
-        ctx->encode_tiled = fn;
-        ctx->tc_ready = 1;
-    }
+    int rc = ensure_encode(ctx);
+    if (rc) return rc;
     if (passes == 16 && need_cols) passes = 1;  // the fp16 pass has no column arg-max: same results from the tf32 pass
     const long long rows_a = (long long)B * n_stride, rows_b = (long long)B * m_stride;
     const bool l2 = metric == VO_METRIC_L2;
     // workspace: A_hi | A_lo  and  B_hi | B_lo  and  row norms | column norms
     float *split_a, *split_b, *norms;
-    int rc;
     const bool f16 = passes == 16, h16 = passes == 16 || passes == 48, three = passes == 3 || passes == 48;
     const size_t esz = h16 ? sizeof(__half) : sizeof(float);
     const int row_elems = src_u8 ? src_u8 : TC_D;  // stored elements per descriptor row
@@ -1406,21 +1291,11 @@ int match_f32_tc(vo_ctx *ctx, const float *ref, const float *cur, int B, int n_s
 int match_bits_tc(vo_ctx *ctx, const uint8_t *ref, const uint8_t *cur, int B, int n_stride, int m_stride, const int32_t *n_ref,
                   const int32_t *n_cur, int need_cols, int need_second, vo_row_partial **part_out, int *n_split_out,
                   unsigned long long *colkey, cudaStream_t st) {
-    if (!ctx->tc_ready) {
-        void *fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        VO_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres));
-        if (qres != cudaDriverEntryPointSuccess || !fn) {
-            set_error("cuTensorMapEncodeTiled is not available from this driver");
-            return VO_ERR_UNSUPPORTED;
-        }
-        ctx->encode_tiled = fn;
-        ctx->tc_ready = 1;
-    }
+    int rc = ensure_encode(ctx);
+    if (rc) return rc;
     constexpr int KD = 256, BN = TcCfg<8>::BN;
     const long long rows_a = (long long)B * n_stride, rows_b = (long long)B * m_stride;
     uint8_t *a8, *b8;
-    int rc;
     // consecutive pairs of one frame sequence (cur = ref one frame on): every frame is expanded once (see match_f32_tc)
     const bool chained = n_stride == m_stride && B > 0 && !getenv("VO_NO_CHAIN_PREP") && cur == ref + (size_t)n_stride * 32;
     const long long rows_p = chained ? rows_a + n_stride : rows_a;

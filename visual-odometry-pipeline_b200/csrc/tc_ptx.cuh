@@ -5,6 +5,12 @@
 #include <cuda.h>  // CUtensorMap & enums only; cuTensorMapEncodeTiled is resolved at run time
 
 namespace vo {
+
+// cuTensorMapEncodeTiled as vo_ctx::encode_tiled holds it
+typedef CUresult (*PFN_encodeTiled)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
+                                    const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
+                                    CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
 namespace tc {
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
