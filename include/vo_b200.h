@@ -27,11 +27,12 @@
 extern "C" {
 #endif
 
-#define VO_ABI_VERSION 4   /* 2: vo_pipeline_args.u8_bytes, vo_pnp_ransac_ref, VO_NORM_HAMMING_TC, vo_orb_debug_read
+#define VO_ABI_VERSION 5   /* 2: vo_pipeline_args.u8_bytes, vo_pnp_ransac_ref, VO_NORM_HAMMING_TC, vo_orb_debug_read
                              3: vo_bootstrap, vo_pnp_ransac_ref_batch, VO_ST_BAD_INPUT, the pnp_mode / ref_* fields of
                                 vo_pipeline_args and vo_seq_config
                              4: vo_seq_config.n_seqs / seeds, vo_seq_push_all, vo_seq_read_at, vo_seq_frames_at, vo_seq_graph_captures,
-                                vo_workspace_generation */
+                                vo_workspace_generation
+                             5: vo_orb_extract_batch, vo_seq_push_all_dev, vo_seq_lost_frames_at */
 
 #if defined(__GNUC__)
 #define VO_API __attribute__((visibility("default")))
@@ -307,6 +308,13 @@ VO_API int vo_pipeline(vo_ctx *ctx, const vo_pipeline_args *args, void *stream);
  * launch.  The graph holds the vo_ctx workspace pointers; when any call on the same vo_ctx has reallocated a workspace
  * since capture, the next step re-captures.  vo_seq_graph_captures: how many times the loop captured its step (0 when
  * it launches plainly; one more for every re-capture).  n_seqs is at most 65535.
+ * Device-side counts (VERSION 5), so that S sequences go from images to poses with no host read per step:
+ *   vo_seq_push_all_dev: desc / kp / depth as vo_seq_push_all; n_kp_d device int32 [S][2] = (rows, flags), the layout
+ *   vo_orb_extract_batch writes; present_h host int32 [S] (non-zero: sequence q has a frame at this step); frame_id_h as
+ *   vo_seq_push_all.  The loop reads each present sequence's count on the device and clamps it to n_cap; a frame that was
+ *   clamped or whose flag word is non-zero lost rows and is counted per sequence.  Checks (the history of every present
+ *   sequence not full) come before anything is enqueued.
+ *   vo_seq_lost_frames_at: *out_h = the number of such frames of sequence q so far (synchronises `stream`).
  */
 typedef struct vo_seq vo_seq;
 typedef struct vo_seq_config {
@@ -348,6 +356,9 @@ VO_API int vo_seq_push_all(vo_seq *seq, const void *desc, const float *kp, const
 VO_API int vo_seq_frames_at(const vo_seq *seq, int q);
 VO_API int vo_seq_read_at(vo_seq *seq, int q, int first, int count, double *poses_h, int32_t *info_h, void *stream);
 VO_API int vo_seq_graph_captures(const vo_seq *seq);
+VO_API int vo_seq_push_all_dev(vo_seq *seq, const void *desc, const float *kp, const int32_t *n_kp_d, const int32_t *present_h,
+                        const float *depth, const int32_t *frame_id_h, void *stream);
+VO_API int vo_seq_lost_frames_at(vo_seq *seq, int q, int32_t *out_h, void *stream);
 
 /*
  * "Same" 2-D convolution on the tensor cores (3xTF32 implicit GEMM; TMA zero fill is the padding): the layer type of
@@ -462,6 +473,13 @@ VO_API int vo_pnp_ransac_ref_batch(vo_ctx *ctx, const float *xyz, const float *u
  *   aux float [cap][4] = (octave, angle in degrees, response, size), optional; count int32[2] = (keypoints written,
  *   overflow flag: a level kept more than its share of ties).  Order: level-major, then row-major (OpenCV's own
  *   order is unspecified: it depends on std::nth_element).
+ *   vo_orb_extract_batch (VERSION 5): S images in one call of the same 17 launches (BGR; 16 for gray).  images uint8
+ *   [S][H][W] (channels = 1) or [S][H][W][3], device or pinned host memory.  Outputs (device): kp float [S][out_rows][2],
+ *   desc uint8 [S][out_rows][32], aux float [S][out_rows][4] (optional), count int32 [S][2] = (rows written, flags): flag
+ *   bit 0 = a level kept more tied keypoints than it holds (vo_orb_extract's overflow), bit 1 = rows past out_rows were
+ *   dropped.  Image s's rows are a prefix of what vo_orb_extract returns for it, in the same order.  1 <= S <= 65535,
+ *   out_rows >= 1.  Scratch grows to the largest S seen (growing synchronises the device).  vo_orb_extract is the S = 1
+ *   call with out_rows = vo_orb_capacity().
  */
 typedef struct vo_orb_config {
     int H, W;
@@ -475,6 +493,8 @@ VO_API void vo_orb_destroy(vo_orb *orb);
 VO_API int vo_orb_capacity(const vo_orb *orb);
 VO_API int vo_orb_extract(vo_orb *orb, const uint8_t *image, int channels, float *kp, uint8_t *desc, float *aux,
                    int32_t *count, void *stream);
+VO_API int vo_orb_extract_batch(vo_orb *orb, const uint8_t *images, int S, int channels, int out_rows, float *kp, uint8_t *desc,
+                         float *aux, int32_t *count, void *stream);
 /* Diagnostic: copy one intermediate buffer of the last vo_orb_extract to host memory (synchronises; buffer ids in
  * csrc/orb.cu).  Used by tools/orb_bisect.py to compare the extractor stage by stage with the CPU restatement. */
 VO_API int vo_orb_debug_read(vo_orb *orb, int what, int level, void *host_dst, size_t cap_bytes, size_t *out_bytes);

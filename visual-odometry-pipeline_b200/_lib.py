@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("VO_B200_LIB") or os.path.join(_HERE, "libvo_b200.so")   # (override: A/B runs of two builds)
 
 # ---- constants mirrored from include/vo_b200.h ---------------------------------------------
-VO_ABI_VERSION = 4
+VO_ABI_VERSION = 5
 VO_OK, VO_ERR_ARG, VO_ERR_CUDA, VO_ERR_UNSUPPORTED = 0, -1, -2, -3
 VO_ST_OK, VO_ST_NO_MODEL, VO_ST_TOO_FEW_POINTS, VO_ST_KP_OUT_OF_IMAGE, VO_ST_BAD_INPUT = 0, 1, 2, 4, 8
 VO_NORM_HAMMING, VO_NORM_L2_U8, VO_NORM_HAMMING_TC = 0, 1, 2
@@ -139,6 +139,8 @@ PROTOTYPES = {
     "vo_seq_frames_at": (c_int, [c_void_p, c_int]),
     "vo_seq_read_at": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "vo_seq_graph_captures": (c_int, [c_void_p]),
+    "vo_seq_push_all_dev": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vo_seq_lost_frames_at": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
     "vo_conv2d": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_int,
                           c_void_p, c_void_p]),
     "vo_r2d2_create": (c_int, [c_void_p, ctypes.POINTER(R2d2Config), ctypes.POINTER(c_void_p)]),
@@ -150,6 +152,7 @@ PROTOTYPES = {
     "vo_orb_destroy": (None, [c_void_p]),
     "vo_orb_capacity": (c_int, [c_void_p]),
     "vo_orb_extract": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vo_orb_extract_batch": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vo_orb_debug_read": (c_int, [c_void_p, c_int, c_int, c_void_p, ctypes.c_size_t, ctypes.POINTER(ctypes.c_size_t)]),
     "vo_sift_create": (c_int, [c_void_p, ctypes.POINTER(SiftConfig), ctypes.POINTER(c_void_p)]),
     "vo_sift_destroy": (None, [c_void_p]),

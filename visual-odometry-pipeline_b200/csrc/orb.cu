@@ -15,6 +15,12 @@
 // Everything is HBM-bound integer / byte work: ~1.1 M pixels per 1241 x 376 frame over the 8 levels; the per-pixel
 // kernels cover all levels in one launch each (17 launches per BGR frame, 7 of them the resize cascade).
 //
+// Batch (vo_orb_extract_batch): every kernel also runs over S images, the image index being the last grid dimension, so
+// a call is 17 launches (BGR) whatever S is; vo_orb_extract is the S = 1 call.  Per-pixel buffers are level-major with
+// the S images of a level back to back (image s of level l at img_ofs + s * w * h): level 0 of the batch is then one
+// contiguous block and a gray batch arrives with one copy.  Keypoint lists, kept lists, angles and the 32-entry count
+// block are image-major.  Image s's output rows are a prefix (level-major, then row-major) of what it alone would give.
+//
 // The rBRIEF point pairs below are OpenCV's learned pattern (modules/features2d/src/orb.cpp, bit_pattern_31_,
 // Apache-2.0): data of the third-party library whose arithmetic the reference's plug-in runs.
 #include "common.cuh"
@@ -69,14 +75,17 @@ struct OrbLevel {
     int n_feat;          // retainBest target of this level
     int cand_cap;        // w * h / 4 + 1: a strict 3x3 maximum cannot be denser
     float scale;
-    size_t img_ofs;      // bytes into the pyramid / blurred / score buffers
-    size_t cand_ofs;     // entries into the candidate / survivor lists
+    size_t img_ofs;      // bytes into the pyramid / blurred / score buffers of image 0 (image s: + s * w * h)
+    size_t cand_ofs;     // entries into the candidate / survivor lists of one image
 };
 struct OrbLevels {
     OrbLevel l[ORB_MAX_LEVELS];
     int n;
     int total_rows;      // sum of the level heights: per-pixel kernels run over all levels in one launch
+    size_t cand_img;     // candidate / survivor entries of one image (image s starts at s * cand_img)
 };
+
+__device__ __forceinline__ size_t orb_img(const OrbLevel &lv, int s) { return lv.img_ofs + (size_t)s * lv.w * lv.h; }
 
 // blockIdx.y of an all-level launch -> (level, row inside it).  The grid is as wide as level 0.
 __device__ __forceinline__ bool orb_locate_row(const OrbLevels &L, int gy, int &lev, int &y) {
@@ -87,14 +96,20 @@ __device__ __forceinline__ bool orb_locate_row(const OrbLevels &L, int gy, int &
     return false;
 }
 
+// blockIdx.y: image (level 0 of the batch is contiguous, n_px bytes per image)
 __global__ void orb_gray_kernel(const uint8_t *__restrict__ bgr, uint8_t *__restrict__ gray, int n_px) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n_px) gray[i] = orb::bgr_to_gray(bgr[3 * i], bgr[3 * i + 1], bgr[3 * i + 2]);
+    const size_t o = (size_t)blockIdx.y * n_px + i;
+    if (i < n_px) gray[o] = orb::bgr_to_gray(bgr[3 * o], bgr[3 * o + 1], bgr[3 * o + 2]);
 }
 
+// blockIdx.z: image; src / dst point at image 0's level, the next source image starts W * H bytes on, the next
+// destination image dw * dh bytes on
 __global__ void orb_resize_kernel(const uint8_t *__restrict__ src, int W, int H, uint8_t *__restrict__ dst, int dw, int dh) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
     if (x >= dw) return;
+    src += (size_t)blockIdx.z * W * H;
+    dst += (size_t)blockIdx.z * dw * dh;
     int ox, cx, oy, cy;
     bool inx, iny;
     orb::linear_exact_coeff(x, dw, W, ox, cx, inx);
@@ -104,14 +119,15 @@ __global__ void orb_resize_kernel(const uint8_t *__restrict__ src, int W, int H,
                                                       src[(size_t)oy1 * W + ox], src[(size_t)oy1 * W + ox1], cx, inx, cy, iny);
 }
 
-// FAST-9/16 corner score of every pixel of every level (0 in the 3-pixel frame and for non-corners).
+// FAST-9/16 corner score of every pixel of every level (0 in the 3-pixel frame and for non-corners).  blockIdx.z: image
+// (also in every kernel below).
 __global__ void orb_fast_kernel(OrbLevels L, const uint8_t *__restrict__ pyr, int thr, uint8_t *__restrict__ score_all) {
     int lev, y;
     if (!orb_locate_row(L, blockIdx.y, lev, y)) return;
     const int w = L.l[lev].w, h = L.l[lev].h;
     const int x = blockIdx.x * blockDim.x + threadIdx.x;
     if (x >= w) return;
-    const uint8_t *img = pyr + L.l[lev].img_ofs;
+    const uint8_t *img = pyr + orb_img(L.l[lev], blockIdx.z);
     int s = 0;
     if (x >= 3 && x < w - 3 && y >= 3 && y < h - 3) {
         const uint8_t *p = img + (size_t)y * w + x;
@@ -129,7 +145,7 @@ __global__ void orb_fast_kernel(OrbLevels L, const uint8_t *__restrict__ pyr, in
             s = orb::fast_corner_score(v, ring, thr);
         }
     }
-    score_all[L.l[lev].img_ofs + (size_t)y * w + x] = (uint8_t)s;
+    score_all[orb_img(L.l[lev], blockIdx.z) + (size_t)y * w + x] = (uint8_t)s;
 }
 
 // Corners that are strict maxima of the score in their 3x3 neighbourhood and lie >= 31 pixels inside their level.
@@ -141,25 +157,28 @@ __global__ void orb_nms_kernel(OrbLevels L, const uint8_t *__restrict__ score_al
     const int w = lv.w, h = lv.h;
     const int x = blockIdx.x * blockDim.x + threadIdx.x;
     if (x < ORB_EDGE || x >= w - ORB_EDGE || y < ORB_EDGE || y >= h - ORB_EDGE) return;
-    const uint8_t *p = score_all + lv.img_ofs + (size_t)y * w + x;
+    const uint8_t *p = score_all + orb_img(lv, blockIdx.z) + (size_t)y * w + x;
     const int s = p[0];
     if (s == 0) return;
     if (s > p[-1] && s > p[1] && s > p[-w - 1] && s > p[-w] && s > p[-w + 1] && s > p[w - 1] && s > p[w] && s > p[w + 1]) {
-        const int i = atomicAdd(cand_count + lev, 1);
-        if (i < lv.cand_cap) { cand_xy[lv.cand_ofs + i] = (uint32_t)x | ((uint32_t)y << 16); cand_s[lv.cand_ofs + i] = (uint8_t)s; }
+        const int i = atomicAdd(cand_count + 32 * blockIdx.z + lev, 1);
+        const size_t c = blockIdx.z * L.cand_img + lv.cand_ofs + i;
+        if (i < lv.cand_cap) { cand_xy[c] = (uint32_t)x | ((uint32_t)y << 16); cand_s[c] = (uint8_t)s; }
     }
 }
 
-// KeyPointsFilter::retainBest(2 n) on the FAST score: the 2 n best plus every tie with the 2 n-th.  One CTA per level.
+// KeyPointsFilter::retainBest(2 n) on the FAST score: the 2 n best plus every tie with the 2 n-th.  One CTA per level
+// (blockIdx.x) and image (blockIdx.y).
 __global__ void __launch_bounds__(1024)
 orb_select_fast_kernel(OrbLevels L, const uint32_t *__restrict__ cand_xy, const uint8_t *__restrict__ cand_s,
                        const int32_t *__restrict__ cand_count, uint32_t *__restrict__ surv_xy, int32_t *__restrict__ surv_count) {
     __shared__ int hist[256];
     __shared__ int thr_s, out_s;
     const OrbLevel lv = L.l[blockIdx.x];
-    const int m = min(cand_count[blockIdx.x], lv.cand_cap), keep = 2 * lv.n_feat;
-    const uint32_t *xy = cand_xy + lv.cand_ofs;
-    const uint8_t *sc = cand_s + lv.cand_ofs;
+    const size_t c0 = blockIdx.y * L.cand_img + lv.cand_ofs;
+    const int m = min(cand_count[32 * blockIdx.y + blockIdx.x], lv.cand_cap), keep = 2 * lv.n_feat;
+    const uint32_t *xy = cand_xy + c0;
+    const uint8_t *sc = cand_s + c0;
     for (int i = threadIdx.x; i < 256; i += blockDim.x) hist[i] = 0;
     if (threadIdx.x == 0) { thr_s = 0; out_s = 0; }
     __syncthreads();
@@ -175,19 +194,20 @@ orb_select_fast_kernel(OrbLevels L, const uint32_t *__restrict__ cand_xy, const 
     }
     const int thr = (keep > 0) ? thr_s : 256;   // keep == 0: retainBest clears the list
     for (int i = threadIdx.x; i < m; i += blockDim.x)
-        if ((int)sc[i] >= thr) surv_xy[lv.cand_ofs + atomicAdd(&out_s, 1)] = xy[i];
+        if ((int)sc[i] >= thr) surv_xy[c0 + atomicAdd(&out_s, 1)] = xy[i];
     __syncthreads();
-    if (threadIdx.x == 0) surv_count[blockIdx.x] = out_s;
+    if (threadIdx.x == 0) surv_count[32 * blockIdx.y + blockIdx.x] = out_s;
 }
 
 // Harris response of every survivor (orb.cpp HarrisResponses, 7x7 block).
 __global__ void orb_harris_kernel(OrbLevels L, const uint8_t *__restrict__ pyr, const uint32_t *__restrict__ surv_xy,
                                   const int32_t *__restrict__ surv_count, float *__restrict__ resp) {
     const OrbLevel lv = L.l[blockIdx.y];
-    const int m = surv_count[blockIdx.y], w = lv.w;
-    const uint8_t *img = pyr + lv.img_ofs;
+    const int m = surv_count[32 * blockIdx.z + blockIdx.y], w = lv.w;
+    const uint8_t *img = pyr + orb_img(lv, blockIdx.z);
+    const size_t c0 = blockIdx.z * L.cand_img + lv.cand_ofs;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < m; i += gridDim.x * blockDim.x) {
-    const uint32_t xy = surv_xy[lv.cand_ofs + i];
+    const uint32_t xy = surv_xy[c0 + i];
     const int x = xy & 0xffff, y = xy >> 16;
     int a = 0, b = 0, c = 0;
     for (int dy = -3; dy <= 3; ++dy)
@@ -197,12 +217,13 @@ __global__ void orb_harris_kernel(OrbLevels L, const uint8_t *__restrict__ pyr, 
             const int iy = ((int)p[w] - (int)p[-w]) * 2 + ((int)p[w - 1] - (int)p[-w - 1]) + ((int)p[w + 1] - (int)p[-w + 1]);
             a += ix * ix; b += iy * iy; c += ix * iy;
         }
-    resp[lv.cand_ofs + i] = orb::harris_response(a, b, c);
+    resp[c0 + i] = orb::harris_response(a, b, c);
     }
 }
 
 // retainBest(n) on the Harris response: exact n-th largest by a 4-pass radix select over the ordered float bits, every
-// tie with it kept; the kept keypoints are then ranked by (y, x) and written in that order.  One CTA per level.
+// tie with it kept; the kept keypoints are then ranked by (y, x) and written in that order.  One CTA per level
+// (blockIdx.x) and image (blockIdx.y); counts[24] of the image's block is its overflow flag.
 __global__ void __launch_bounds__(1024)
 orb_select_harris_kernel(OrbLevels L, const uint32_t *__restrict__ surv_xy, const float *__restrict__ resp,
                          const int32_t *__restrict__ surv_count, uint32_t *__restrict__ fin_xy, float *__restrict__ fin_resp,
@@ -212,11 +233,12 @@ orb_select_harris_kernel(OrbLevels L, const uint32_t *__restrict__ surv_xy, cons
     __shared__ int want_s, out_s;
     __shared__ uint32_t kxy[ORB_FINAL_CAP];
     __shared__ float kresp[ORB_FINAL_CAP];
-    const int lev = blockIdx.x;
+    const int lev = blockIdx.x, img = blockIdx.y;
     const OrbLevel lv = L.l[lev];
-    const int m = surv_count[lev], keep = lv.n_feat;
-    const uint32_t *xy = surv_xy + lv.cand_ofs;
-    const float *r = resp + lv.cand_ofs;
+    const int m = surv_count[32 * img + lev], keep = lv.n_feat;
+    const size_t c0 = img * L.cand_img + lv.cand_ofs, f0 = ((size_t)img * L.n + lev) * ORB_FINAL_CAP;
+    const uint32_t *xy = surv_xy + c0;
+    const float *r = resp + c0;
     uint32_t thr_key = 0;   // keep everything
     if (m > keep && keep > 0) {
         if (threadIdx.x == 0) { prefix_s = 0; want_s = keep; }
@@ -254,34 +276,40 @@ orb_select_harris_kernel(OrbLevels L, const uint32_t *__restrict__ surv_xy, cons
     __syncthreads();
     const int n_out = min(out_s, ORB_FINAL_CAP);
     if (threadIdx.x == 0) {
-        fin_count[lev] = n_out;
-        if (out_s > ORB_FINAL_CAP) atomicExch(overflow, 1);
+        fin_count[32 * img + lev] = n_out;
+        if (out_s > ORB_FINAL_CAP) atomicExch(overflow + 32 * img, 1);
     }
     // rank by (y << 16 | x): keys are distinct, so rank = number of smaller keys
     for (int i = threadIdx.x; i < n_out; i += blockDim.x) {
         const uint32_t k = kxy[i];
         int rank = 0;
         for (int j = 0; j < n_out; ++j) rank += kxy[j] < k;
-        fin_xy[(size_t)lev * ORB_FINAL_CAP + rank] = k;
-        fin_resp[(size_t)lev * ORB_FINAL_CAP + rank] = kresp[i];
+        fin_xy[f0 + rank] = k;
+        fin_resp[f0 + rank] = kresp[i];
     }
 }
 
-// Orientation (intensity centroid, fastAtan2) and the keypoint record.  One thread per kept keypoint.
+// Orientation (intensity centroid, fastAtan2) and the keypoint record.  One thread per kept keypoint; rows at or past
+// out_rows are dropped.  count_out[img] = (rows written, flags: 1 = a level overflowed, 2 = rows were dropped).
 __global__ void orb_finish_kernel(OrbLevels L, const uint8_t *__restrict__ pyr, const uint32_t *__restrict__ fin_xy,
                                   const float *__restrict__ fin_resp, const int32_t *__restrict__ fin_count,
-                                  const int32_t *__restrict__ overflow, float *__restrict__ kp, float *__restrict__ aux,
-                                  float *__restrict__ angle_out, int32_t *__restrict__ count_out) {
-    const int lev = blockIdx.y;
+                                  const int32_t *__restrict__ overflow, int out_rows, float *__restrict__ kp,
+                                  float *__restrict__ aux, float *__restrict__ angle_out, int32_t *__restrict__ count_out) {
+    const int lev = blockIdx.y, img = blockIdx.z;
     const OrbLevel lv = L.l[lev];
+    fin_count += 32 * img;
     int base = 0, total = 0;
     for (int j = 0; j < L.n; ++j) { if (j < lev) base += fin_count[j]; total += fin_count[j]; }
-    if (lev == 0 && blockIdx.x == 0 && threadIdx.x == 0) { count_out[0] = total; count_out[1] = overflow[0]; }
-    const int n_lev = fin_count[lev], w = lv.w;
+    if (lev == 0 && blockIdx.x == 0 && threadIdx.x == 0) {
+        count_out[2 * img] = min(total, out_rows);
+        count_out[2 * img + 1] = overflow[32 * img] | (total > out_rows ? 2 : 0);
+    }
+    const int n_lev = min(fin_count[lev], out_rows - base), w = lv.w;
+    const size_t f0 = ((size_t)img * L.n + lev) * ORB_FINAL_CAP, o0 = (size_t)img * out_rows;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n_lev; i += gridDim.x * blockDim.x) {
-    const uint32_t xy = fin_xy[(size_t)lev * ORB_FINAL_CAP + i];
+    const uint32_t xy = fin_xy[f0 + i];
     const int x = xy & 0xffff, y = xy >> 16;
-    const uint8_t *c = pyr + lv.img_ofs + (size_t)y * w + x;
+    const uint8_t *c = pyr + orb_img(lv, img) + (size_t)y * w + x;
     int m01 = 0, m10 = 0;
     for (int u = -orb::HALF_PATCH; u <= orb::HALF_PATCH; ++u) m10 += u * (int)c[u];
     for (int v = 1; v <= orb::HALF_PATCH; ++v) {
@@ -295,14 +323,14 @@ __global__ void orb_finish_kernel(OrbLevels L, const uint8_t *__restrict__ pyr, 
         m01 += v * vsum;
     }
     const float ang = orb::fast_atan2((float)m01, (float)m10);
-    const int o = base + i;
+    const size_t o = o0 + base + i;
     kp[2 * o + 0] = __fmul_rn((float)x, lv.scale);
     kp[2 * o + 1] = __fmul_rn((float)y, lv.scale);
-    angle_out[o] = ang;
+    angle_out[(size_t)img * L.n * ORB_FINAL_CAP + base + i] = ang;
     if (aux) {
         aux[4 * o + 0] = (float)lev;
         aux[4 * o + 1] = ang;
-        aux[4 * o + 2] = fin_resp[(size_t)lev * ORB_FINAL_CAP + i];
+        aux[4 * o + 2] = fin_resp[f0 + i];
         aux[4 * o + 3] = __fmul_rn(31.0f, lv.scale);
     }
     }
@@ -318,11 +346,12 @@ __global__ void orb_blur_row_kernel(OrbLevels L, const uint8_t *__restrict__ pyr
     const int w = L.l[lev].w;
     const int x = blockIdx.x * blockDim.x + threadIdx.x;
     if (x >= w) return;
-    const uint8_t *img = pyr + L.l[lev].img_ofs;
+    const size_t ofs = orb_img(L.l[lev], blockIdx.z);
+    const uint8_t *img = pyr + ofs;
     uint8_t p[7];
 #pragma unroll
     for (int i = 0; i < 7; ++i) p[i] = img[(size_t)y * w + reflect101(x + i - 3, w)];
-    tmp_all[L.l[lev].img_ofs + (size_t)y * w + x] = orb::blur_row(g.k, p);
+    tmp_all[ofs + (size_t)y * w + x] = orb::blur_row(g.k, p);
 }
 __global__ void orb_blur_col_kernel(OrbLevels L, const float *__restrict__ tmp_all, GaussK g, uint8_t *__restrict__ blurred) {
     int lev, y;
@@ -330,28 +359,34 @@ __global__ void orb_blur_col_kernel(OrbLevels L, const float *__restrict__ tmp_a
     const int w = L.l[lev].w, h = L.l[lev].h;
     const int x = blockIdx.x * blockDim.x + threadIdx.x;
     if (x >= w) return;
-    const float *tmp = tmp_all + L.l[lev].img_ofs;
+    const size_t ofs = orb_img(L.l[lev], blockIdx.z);
+    const float *tmp = tmp_all + ofs;
     float c[7];
 #pragma unroll
     for (int i = 0; i < 7; ++i) c[i] = tmp[(size_t)reflect101(y + i - 3, h) * w + x];
-    blurred[L.l[lev].img_ofs + (size_t)y * w + x] = orb::blur_col(g.k, c);
+    blurred[ofs + (size_t)y * w + x] = orb::blur_col(g.k, c);
 }
 
-// rBRIEF: one warp per keypoint, lane = descriptor byte (8 point pairs = 16 pattern points).
+// rBRIEF: one warp per keypoint, lane = descriptor byte (8 point pairs = 16 pattern points).  Rows at or past out_rows
+// are dropped, as in orb_finish_kernel.
 __global__ void orb_desc_kernel(OrbLevels L, const uint8_t *__restrict__ blurred, const uint32_t *__restrict__ fin_xy,
-                                const int32_t *__restrict__ fin_count, const float *__restrict__ angle,
+                                const int32_t *__restrict__ fin_count, const float *__restrict__ angle, int out_rows,
                                 uint8_t *__restrict__ desc) {
-    const int lev = blockIdx.y, lane = threadIdx.x & 31;
+    const int lev = blockIdx.y, img = blockIdx.z, lane = threadIdx.x & 31;
     const OrbLevel lv = L.l[lev];
-    const int n_lev = fin_count[lev], w = lv.w;
+    fin_count += 32 * img;
     int base = 0;
     for (int j = 0; j < lev; ++j) base += fin_count[j];
+    const int n_lev = min(fin_count[lev], out_rows - base), w = lv.w;
+    const size_t f0 = ((size_t)img * L.n + lev) * ORB_FINAL_CAP;
+    angle += (size_t)img * L.n * ORB_FINAL_CAP + base;
+    desc += ((size_t)img * out_rows + base) * 32;
     for (int i = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n_lev; i += gridDim.x * (blockDim.x >> 5)) {
-    const uint32_t xy = fin_xy[(size_t)lev * ORB_FINAL_CAP + i];
+    const uint32_t xy = fin_xy[f0 + i];
     const int x = xy & 0xffff, y = xy >> 16;
-    const uint8_t *c = blurred + lv.img_ofs + (size_t)y * w + x;
+    const uint8_t *c = blurred + orb_img(lv, img) + (size_t)y * w + x;
     float ca, sb;
-    orb::angle_cos_sin(angle[base + i], ca, sb);
+    orb::angle_cos_sin(angle[i], ca, sb);
     int val = 0;
 #pragma unroll
     for (int b = 0; b < 8; ++b) {
@@ -361,7 +396,7 @@ __global__ void orb_desc_kernel(OrbLevels L, const uint8_t *__restrict__ blurred
         orb::rotate_pattern_point(pp[2], pp[3], ca, sb, ix1, iy1);
         val |= ((int)c[iy0 * w + ix0] < (int)c[iy1 * w + ix1]) << b;
     }
-    desc[(size_t)(base + i) * 32 + lane] = (uint8_t)val;
+    desc[(size_t)i * 32 + lane] = (uint8_t)val;
     }
 }
 
@@ -372,22 +407,67 @@ struct vo_orb {
     vo_ctx *ctx;
     int H, W, fast_thr;
     vo::OrbLevels L;
-    size_t pyr_bytes, cand_total;
+    int S_cap;         // images the scratch buffers hold (the largest batch seen so far)
     uint8_t *pyr, *blurred, *score, *cand_s;
     float *tmp, *resp, *fin_resp, *angle;
     uint32_t *cand_xy, *surv_xy, *fin_xy;
-    int32_t *counts;   // cand[8] | surv[8] | fin[8] | overflow
+    int32_t *counts;   // per image: cand[8] | surv[8] | fin[8] | overflow | unused[7]
     vo::GaussK g;
 };
+
+namespace vo {
+namespace {
+
+void orb_free(vo_orb *o) {
+    void **ptrs[] = {(void **)&o->pyr, (void **)&o->blurred, (void **)&o->score, (void **)&o->cand_s, (void **)&o->tmp,
+                     (void **)&o->resp, (void **)&o->fin_resp, (void **)&o->angle, (void **)&o->cand_xy,
+                     (void **)&o->surv_xy, (void **)&o->fin_xy, (void **)&o->counts};
+    for (void **p : ptrs) {
+        if (*p) cudaFree(*p);
+        *p = nullptr;
+    }
+    o->S_cap = 0;
+}
+
+// Scratch for S images: level bases of the level-major pixel buffers follow from S, so they are set here.  Growing
+// drains the device first (work queued on any stream may still use the old blocks), as ws_get does.
+int orb_reserve(vo_orb *o, int S) {
+    if (S <= o->S_cap) return VO_OK;
+    cudaSetDevice(o->ctx->device);
+    if (o->S_cap) VO_CUDA(cudaDeviceSynchronize());
+    orb_free(o);
+    OrbLevels &L = o->L;
+    size_t img_ofs = 0;
+    for (int l = 0; l < L.n; ++l) {
+        L.l[l].img_ofs = img_ofs;
+        img_ofs += ((size_t)S * L.l[l].w * L.l[l].h + 255) & ~(size_t)255;
+    }
+    const size_t cand = (size_t)S * L.cand_img, fin = (size_t)S * L.n * ORB_FINAL_CAP;
+    cudaError_t e = cudaSuccess;
+    auto alloc = [&](void **p, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(p, bytes ? bytes : 16); };
+    alloc((void **)&o->pyr, img_ofs); alloc((void **)&o->blurred, img_ofs); alloc((void **)&o->score, img_ofs);
+    alloc((void **)&o->tmp, img_ofs * sizeof(float));
+    alloc((void **)&o->cand_xy, cand * 4); alloc((void **)&o->cand_s, cand); alloc((void **)&o->surv_xy, cand * 4);
+    alloc((void **)&o->resp, cand * 4);
+    alloc((void **)&o->fin_xy, fin * 4); alloc((void **)&o->fin_resp, fin * 4); alloc((void **)&o->angle, fin * 4);
+    alloc((void **)&o->counts, sizeof(int32_t) * 32 * S);
+    if (e != cudaSuccess) {
+        orb_free(o);
+        set_error("ORB scratch for %d images: cudaMalloc -> %s", S, cudaGetErrorString(e));
+        return VO_ERR_CUDA;
+    }
+    o->S_cap = S;
+    return VO_OK;
+}
+
+}  // namespace
+}  // namespace vo
 
 extern "C" void vo_orb_destroy(vo_orb *o) {
     if (!o) return;
     cudaSetDevice(o->ctx->device);
     cudaDeviceSynchronize();
-    void *ptrs[] = {o->pyr, o->blurred, o->score, o->cand_s, o->tmp, o->resp, o->fin_resp, o->angle, o->cand_xy, o->surv_xy,
-                    o->fin_xy, o->counts};
-    for (void *p : ptrs)
-        if (p) cudaFree(p);
+    vo::orb_free(o);
     delete o;
 }
 
@@ -410,7 +490,7 @@ extern "C" int vo_orb_create(vo_ctx *ctx, const vo_orb_config *cfg, vo_orb **out
     const float factor = (float)(1.0 / sf);
     float nd = cfg->nfeatures * (1 - factor) / (1 - (float)pow((double)factor, (double)cfg->nlevels));
     int sum = 0;
-    size_t img_ofs = 0, cand_ofs = 0;
+    size_t cand_ofs = 0;
     o->L.n = cfg->nlevels;
     for (int l = 0; l < cfg->nlevels; ++l) {
         OrbLevel &lv = o->L.l[l];
@@ -421,8 +501,7 @@ extern "C" int vo_orb_create(vo_ctx *ctx, const vo_orb_config *cfg, vo_orb **out
         if (l < cfg->nlevels - 1) { lv.n_feat = (int)lrintf(nd); sum += lv.n_feat; nd *= factor; }
         else lv.n_feat = cfg->nfeatures - sum > 0 ? cfg->nfeatures - sum : 0;
         lv.cand_cap = lv.w * lv.h / 4 + 1;
-        lv.img_ofs = img_ofs; lv.cand_ofs = cand_ofs;
-        img_ofs += ((size_t)lv.w * lv.h + 255) & ~(size_t)255;
+        lv.cand_ofs = cand_ofs;
         cand_ofs += ((size_t)lv.cand_cap + 63) & ~(size_t)63;
     }
     for (int l = 0; l < cfg->nlevels; ++l)
@@ -432,31 +511,21 @@ extern "C" int vo_orb_create(vo_ctx *ctx, const vo_orb_config *cfg, vo_orb **out
             delete o;
             return VO_ERR_ARG;
         }
-    o->pyr_bytes = img_ofs; o->cand_total = cand_ofs;
+    o->L.cand_img = cand_ofs;
     o->L.total_rows = 0;
     for (int l = 0; l < cfg->nlevels; ++l) o->L.total_rows += o->L.l[l].h;
     orb::gaussian_kernel(o->g.k);
-    const size_t fin = (size_t)cfg->nlevels * ORB_FINAL_CAP;
-    cudaError_t e = cudaSuccess;
-    auto alloc = [&](void **p, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(p, bytes ? bytes : 16); };
-    cudaSetDevice(ctx->device);
-    alloc((void **)&o->pyr, img_ofs); alloc((void **)&o->blurred, img_ofs); alloc((void **)&o->score, img_ofs);
-    alloc((void **)&o->tmp, img_ofs * sizeof(float));
-    alloc((void **)&o->cand_xy, cand_ofs * 4); alloc((void **)&o->cand_s, cand_ofs); alloc((void **)&o->surv_xy, cand_ofs * 4);
-    alloc((void **)&o->resp, cand_ofs * 4);
-    alloc((void **)&o->fin_xy, fin * 4); alloc((void **)&o->fin_resp, fin * 4); alloc((void **)&o->angle, fin * 4);
-    alloc((void **)&o->counts, sizeof(int32_t) * 32);
-    if (e != cudaSuccess) {
-        set_error("vo_orb_create: cudaMalloc -> %s", cudaGetErrorString(e));
+    const int rc = orb_reserve(o, 1);
+    if (rc) {
         vo_orb_destroy(o);
-        return VO_ERR_CUDA;
+        return rc;
     }
     *out = o;
     return VO_OK;
 }
 
 // Diagnostic read-back of the extractor's intermediate buffers (tools/orb_bisect.py compares them stage by stage with
-// the CPU restatement).  Synchronises the device.  what: 0 level geometry (int32 {w, h, n_feat, cand_cap} per level),
+// the CPU restatement), of image 0 of the last call.  Synchronises the device.  what: 0 level geometry (int32 {w, h, n_feat, cand_cap} per level),
 // 1 pyramid level, 2 FAST score map, 3 blurred level, 4 candidate xy (u32), 5 candidate score (u8), 6 survivor xy (u32),
 // 7 survivor Harris response (f32), 8 kept xy (u32), 9 kept response (f32), 10 counts (int32[32]), 11 angles (f32, all levels).
 extern "C" int vo_orb_debug_read(vo_orb *o, int what, int level, void *host_dst, size_t cap_bytes, size_t *out_bytes) {
@@ -497,31 +566,35 @@ extern "C" int vo_orb_debug_read(vo_orb *o, int what, int level, void *host_dst,
     return VO_OK;
 }
 
-extern "C" int vo_orb_extract(vo_orb *o, const uint8_t *image, int channels, float *kp, uint8_t *desc, float *aux,
-                              int32_t *count, void *stream) {
-    using namespace vo;
-    VO_REQUIRE(o && image && kp && desc && count, "vo_orb_extract: null argument");
-    VO_REQUIRE(channels == 1 || channels == 3, "vo_orb_extract: image must have 1 (gray) or 3 (BGR) channels, got %d", channels);
+namespace vo {
+namespace {
+
+// The one launch sequence of the extractor: S images, out_rows output rows per image.  17 launches for BGR, 16 for gray
+// (level 0 arrives by one copy), whatever S is.
+int orb_run(vo_orb *o, const uint8_t *images, int S, int channels, int out_rows, float *kp, uint8_t *desc, float *aux,
+            int32_t *count, void *stream) {
     vo_ctx *ctx = o->ctx;
     cudaStream_t st = (cudaStream_t)stream;
+    int rc = orb_reserve(o, S);
+    if (rc) return rc;
     const OrbLevels &L = o->L;
     int32_t *cand_count = o->counts, *surv_count = o->counts + 8, *fin_count = o->counts + 16, *overflow = o->counts + 24;
-    VO_CUDA(cudaMemsetAsync(o->counts, 0, sizeof(int32_t) * 32, st));
+    VO_CUDA(cudaMemsetAsync(o->counts, 0, sizeof(int32_t) * 32 * S, st));
     const int n_px = o->W * o->H;
     if (channels == 3) {
-        VO_LAUNCH(orb_gray_kernel, ceil_div(n_px, 256), 256, st, image, o->pyr, n_px);
+        VO_LAUNCH(orb_gray_kernel, dim3(ceil_div(n_px, 256), S), 256, st, images, o->pyr, n_px);
         VO_LAUNCH_CHECK(ctx);
-    } else {
-        VO_CUDA(cudaMemcpyAsync(o->pyr, image, (size_t)n_px, cudaMemcpyDefault, st));
+    } else {   // level 0 of the batch is contiguous (L.l[0].img_ofs == 0)
+        VO_CUDA(cudaMemcpyAsync(o->pyr, images, (size_t)S * n_px, cudaMemcpyDefault, st));
     }
     for (int l = 1; l < L.n; ++l) {   // every level is resized from the previous one
         const OrbLevel &lv = L.l[l], &pv = L.l[l - 1];
-        VO_LAUNCH(orb_resize_kernel, dim3(ceil_div(lv.w, 128), lv.h), 128, st, o->pyr + pv.img_ofs, pv.w, pv.h,
+        VO_LAUNCH(orb_resize_kernel, dim3(ceil_div(lv.w, 128), lv.h, S), 128, st, o->pyr + pv.img_ofs, pv.w, pv.h,
                   o->pyr + lv.img_ofs, lv.w, lv.h);
         VO_LAUNCH_CHECK(ctx);
     }
     // per-pixel work of all levels in one launch each (levels too small for the 31-pixel border yield no candidate)
-    const dim3 grid_all(ceil_div(L.l[0].w, 128), L.total_rows);
+    const dim3 grid_all(ceil_div(L.l[0].w, 128), L.total_rows, S);
     VO_LAUNCH(orb_fast_kernel, grid_all, 128, st, L, o->pyr, o->fast_thr, o->score);
     VO_LAUNCH_CHECK(ctx);
     VO_LAUNCH(orb_nms_kernel, grid_all, 128, st, L, o->score, o->cand_xy, o->cand_s, cand_count);
@@ -530,17 +603,38 @@ extern "C" int vo_orb_extract(vo_orb *o, const uint8_t *image, int channels, flo
     VO_LAUNCH_CHECK(ctx);
     VO_LAUNCH(orb_blur_col_kernel, grid_all, 128, st, L, o->tmp, o->g, o->blurred);
     VO_LAUNCH_CHECK(ctx);
-    VO_LAUNCH_BAR(orb_select_fast_kernel, L.n, 1024, st, L, o->cand_xy, o->cand_s, cand_count, o->surv_xy, surv_count);
+    VO_LAUNCH_BAR(orb_select_fast_kernel, dim3(L.n, S), 1024, st, L, o->cand_xy, o->cand_s, cand_count, o->surv_xy, surv_count);
     VO_LAUNCH_CHECK(ctx);
     // keypoint-list kernels: a few CTAs per level striding over lists whose lengths only the device knows
-    VO_LAUNCH(orb_harris_kernel, dim3(8, L.n), 256, st, L, o->pyr, o->surv_xy, surv_count, o->resp);
+    VO_LAUNCH(orb_harris_kernel, dim3(8, L.n, S), 256, st, L, o->pyr, o->surv_xy, surv_count, o->resp);
     VO_LAUNCH_CHECK(ctx);
-    VO_LAUNCH_BAR(orb_select_harris_kernel, L.n, 1024, st, L, o->surv_xy, o->resp, surv_count, o->fin_xy, o->fin_resp, fin_count, overflow);
+    VO_LAUNCH_BAR(orb_select_harris_kernel, dim3(L.n, S), 1024, st, L, o->surv_xy, o->resp, surv_count, o->fin_xy, o->fin_resp,
+                  fin_count, overflow);
     VO_LAUNCH_CHECK(ctx);
-    VO_LAUNCH(orb_finish_kernel, dim3(4, L.n), 128, st, L, o->pyr, o->fin_xy, o->fin_resp, fin_count,
-              overflow, kp, aux, o->angle, count);
+    VO_LAUNCH(orb_finish_kernel, dim3(4, L.n, S), 128, st, L, o->pyr, o->fin_xy, o->fin_resp, fin_count, overflow, out_rows,
+              kp, aux, o->angle, count);
     VO_LAUNCH_CHECK(ctx);
-    VO_LAUNCH(orb_desc_kernel, dim3(16, L.n), 256, st, L, o->blurred, o->fin_xy, fin_count, o->angle, desc);
+    VO_LAUNCH(orb_desc_kernel, dim3(16, L.n, S), 256, st, L, o->blurred, o->fin_xy, fin_count, o->angle, out_rows, desc);
     VO_LAUNCH_CHECK(ctx);
     return VO_OK;
+}
+
+}  // namespace
+}  // namespace vo
+
+extern "C" int vo_orb_extract(vo_orb *o, const uint8_t *image, int channels, float *kp, uint8_t *desc, float *aux,
+                              int32_t *count, void *stream) {
+    VO_REQUIRE(o && image && kp && desc && count, "vo_orb_extract: null argument");
+    VO_REQUIRE(channels == 1 || channels == 3, "vo_orb_extract: image must have 1 (gray) or 3 (BGR) channels, got %d", channels);
+    return vo::orb_run(o, image, 1, channels, vo_orb_capacity(o), kp, desc, aux, count, stream);
+}
+
+extern "C" int vo_orb_extract_batch(vo_orb *o, const uint8_t *images, int S, int channels, int out_rows, float *kp,
+                                    uint8_t *desc, float *aux, int32_t *count, void *stream) {
+    VO_REQUIRE(o && images && kp && desc && count, "vo_orb_extract_batch: null argument");
+    VO_REQUIRE(channels == 1 || channels == 3, "vo_orb_extract_batch: images must have 1 (gray) or 3 (BGR) channels, got %d",
+               channels);
+    VO_REQUIRE(S >= 1 && S <= 65535, "vo_orb_extract_batch: %d images outside [1, 65535]", S);
+    VO_REQUIRE(out_rows >= 1, "vo_orb_extract_batch: out_rows %d must be >= 1", out_rows);
+    return vo::orb_run(o, images, S, channels, out_rows, kp, desc, aux, count, stream);
 }

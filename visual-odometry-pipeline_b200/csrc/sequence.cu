@@ -10,7 +10,8 @@
 //   promote_kernel
 // begin_kernel (one thread per sequence) writes the per-sequence state and the counts the pipeline reads: a sequence with no
 // frame at this step (n_kp < 0) or at its first frame gets count 0 on both sides, so it costs no matches, and the policy
-// skips it.  The generator key of sequence q is (seeds[q], slot_q - 1) (common.cuh: vo_pair_key), what a single loop created
+// skips it.  With device-side counts (vo_seq_push_all_dev) begin_kernel also reads each present sequence's count from the
+// extractor's [S][2] (rows, flags) array, clamps it to n_cap and counts the frames that lost rows.  The generator key of sequence q is (seeds[q], slot_q - 1) (common.cuh: vo_pair_key), what a single loop created
 // with seed = seeds[q] draws, so each sequence's poses equal that loop's bit for bit.  S = 1 is vo_seq_push's loop.
 // With VO_SEQ_GRAPH=1 (Mode T only), once a step has run the pipeline plainly (which sizes every workspace: nothing may
 // allocate during capture), everything after begin_kernel is ONE CUDA-graph launch: the pipeline's ~16 kernels, the policy
@@ -52,6 +53,7 @@ struct vo_seq {
     vo::vo_pair_key *keys; // [S]
     double *T_rel, *rt;    // [S][16], [S][12]
     int32_t *out4;         // [4][S]: n_matches, n_corr, n_inl, status
+    int32_t *lost;         // [S]: frames whose device-side count was clamped to n_cap or came with a non-zero flag word
     double *poses;         // [S][max_frames][16]
     int32_t *info;         // [S][max_frames][6]
     int32_t *step_h;       // host [3][S] staging of step_in (pageable: the copy has read it when cudaMemcpyAsync returns)
@@ -67,18 +69,27 @@ struct vo_seq {
 namespace vo {
 namespace {
 
-__global__ void seq_begin_kernel(vo_seq_state *sts, int S, const int32_t *__restrict__ step_in, int32_t *__restrict__ n_eff,
+// n_kp_d: NULL (counts come from step_in) or the device int32 [S][2] (rows, flags) array of vo_seq_push_all_dev, read for
+// the present sequences (step_in[q] == 0).
+__global__ void seq_begin_kernel(vo_seq_state *sts, int S, const int32_t *__restrict__ step_in, const int32_t *__restrict__ n_kp_d,
+                                 int n_cap, int32_t *__restrict__ lost, int32_t *__restrict__ n_eff,
                                  vo_pair_key *__restrict__ keys, double *poses, int32_t *info, int max_frames) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= S) return;
     vo_seq_state *st = sts + q;
-    const int n_kp = step_in[q], frame_id = step_in[S + q], slot = step_in[2 * S + q];
+    int n_kp = step_in[q];
+    const int frame_id = step_in[S + q], slot = step_in[2 * S + q];
     st->active = 0;
     n_eff[q] = 0;
     n_eff[S + q] = 0;
     if (n_kp < 0) {  // no frame of this sequence at this step: nothing of it is touched
         st->promote = 0;
         return;
+    }
+    if (n_kp_d) {
+        const int n = n_kp_d[2 * q], flags = n_kp_d[2 * q + 1];
+        n_kp = min(max(n, 0), n_cap);
+        if (n > n_cap || flags != 0) lost[q]++;
     }
     st->cur_n = n_kp;
     st->cur_id = frame_id;
@@ -221,12 +232,13 @@ extern "C" int vo_seq_create(vo_ctx *ctx, const vo_seq_config *cfg, vo_seq **out
     const size_t nd = round16(s->nd * S), nk = round16(s->nk * S), nz = round16(s->nz * S);
     const size_t mf = (size_t)cfg->max_frames;
     // one allocation: key desc | cur desc | key kp | cur kp | key depth | cur depth | state | step inputs | counts | keys |
-    // outputs | history
+    // outputs | lost-frame counters | history
     const size_t off_kd = 0, off_cd = off_kd + nd, off_kk = off_cd + nd, off_ck = off_kk + nk, off_kz = off_ck + nk,
                  off_cz = off_kz + nz, off_st = off_cz + nz, off_in = off_st + round16(sizeof(vo_seq_state) * S),
                  off_ne = off_in + round16(sizeof(int32_t) * 3 * S), off_keys = off_ne + round16(sizeof(int32_t) * 2 * S),
                  off_T = off_keys + round16(sizeof(vo_pair_key) * S), off_rt = off_T + sizeof(double) * 16 * S,
-                 off_o4 = off_rt + sizeof(double) * 12 * S, off_poses = off_o4 + round16(sizeof(int32_t) * 4 * S),
+                 off_o4 = off_rt + sizeof(double) * 12 * S, off_lost = off_o4 + round16(sizeof(int32_t) * 4 * S),
+                 off_poses = off_lost + round16(sizeof(int32_t) * S),
                  off_info = off_poses + sizeof(double) * 16 * mf * S, total = off_info + round16(sizeof(int32_t) * 6 * mf * S);
     char *base = nullptr;
     cudaError_t e = cudaMalloc(&base, total);
@@ -247,6 +259,7 @@ extern "C" int vo_seq_create(vo_ctx *ctx, const vo_seq_config *cfg, vo_seq **out
     s->keys = (vo_pair_key *)(base + off_keys);
     s->T_rel = (double *)(base + off_T); s->rt = (double *)(base + off_rt);
     s->out4 = (int32_t *)(base + off_o4);
+    s->lost = (int32_t *)(base + off_lost);
     s->poses = (double *)(base + off_poses); s->info = (int32_t *)(base + off_info);
     *out = s;
     return VO_OK;
@@ -270,8 +283,9 @@ namespace vo {
 namespace {
 
 // One step.  desc / kp / depth: `rows` keypoint rows of every sequence's slot, sequence-major with stride n_cap (vo_seq_push
-// copies only the n_kp rows of its one sequence).  All checks come before anything is enqueued.
-int seq_step(vo_seq *seq, const void *desc, const float *kp, const int32_t *n_kp_h, const float *depth,
+// copies only the n_kp rows of its one sequence).  n_kp_d: NULL, or device counts (then n_kp_h[q] is 0 for a present
+// sequence, -1 for an absent one).  All checks come before anything is enqueued.
+int seq_step(vo_seq *seq, const void *desc, const float *kp, const int32_t *n_kp_h, const int32_t *n_kp_d, const float *depth,
              const int32_t *frame_id_h, size_t rows, void *stream, const char *who) {
     const vo_seq_config &c = seq->cfg;
     const int S = seq->S;
@@ -296,8 +310,8 @@ int seq_step(vo_seq *seq, const void *desc, const float *kp, const int32_t *n_kp
     VO_CUDA(cudaMemcpyAsync(seq->cur_depth, depth, seq->nz * S, cudaMemcpyDefault, st));
     VO_CUDA(cudaMemcpyAsync(seq->step_in, seq->step_h, sizeof(int32_t) * 3 * S, cudaMemcpyHostToDevice, st));
     const int threads = S < 64 ? 32 : 64, blocks = ceil_div(S, threads);
-    seq_begin_kernel<<<blocks, threads, 0, st>>>(seq->st, S, seq->step_in, seq->n_eff, seq->keys, seq->poses, seq->info,
-                                                 c.max_frames);
+    seq_begin_kernel<<<blocks, threads, 0, st>>>(seq->st, S, seq->step_in, n_kp_d, c.n_cap, seq->lost, seq->n_eff, seq->keys,
+                                                 seq->poses, seq->info, c.max_frames);
     VO_LAUNCH_CHECK(ctx);
     // everything after begin_kernel: identical launches for every step (per-step values are read from device memory)
     auto body = [&](bool run_pipeline) -> int {
@@ -383,14 +397,37 @@ extern "C" int vo_seq_push(vo_seq *seq, const void *desc, const float *kp, int n
     VO_REQUIRE(seq->S == 1, "vo_seq_push: the loop holds %d sequences; push them with vo_seq_push_all", seq->S);
     VO_REQUIRE(n_kp >= 0, "vo_seq_push: negative keypoint count %d", n_kp);
     const int32_t n = n_kp, id = frame_id;
-    return seq_step(seq, desc, kp, &n, depth, &id, (size_t)n_kp, stream, "vo_seq_push");
+    return seq_step(seq, desc, kp, &n, nullptr, depth, &id, (size_t)n_kp, stream, "vo_seq_push");
 }
 
 extern "C" int vo_seq_push_all(vo_seq *seq, const void *desc, const float *kp, const int32_t *n_kp_h, const float *depth,
                                const int32_t *frame_id_h, void *stream) {
     using namespace vo;
     VO_REQUIRE(seq && desc && kp && n_kp_h && depth && frame_id_h, "vo_seq_push_all: null argument");
-    return seq_step(seq, desc, kp, n_kp_h, depth, frame_id_h, (size_t)seq->S * seq->cfg.n_cap, stream, "vo_seq_push_all");
+    return seq_step(seq, desc, kp, n_kp_h, nullptr, depth, frame_id_h, (size_t)seq->S * seq->cfg.n_cap, stream, "vo_seq_push_all");
+}
+
+extern "C" int vo_seq_push_all_dev(vo_seq *seq, const void *desc, const float *kp, const int32_t *n_kp_d, const int32_t *present_h,
+                                   const float *depth, const int32_t *frame_id_h, void *stream) {
+    using namespace vo;
+    VO_REQUIRE(seq && desc && kp && n_kp_d && present_h && depth && frame_id_h, "vo_seq_push_all_dev: null argument");
+    int32_t *pres = (int32_t *)malloc(sizeof(int32_t) * seq->S);
+    VO_REQUIRE(pres, "vo_seq_push_all_dev: out of host memory");
+    for (int q = 0; q < seq->S; ++q) pres[q] = present_h[q] ? 0 : -1;
+    const int rc = seq_step(seq, desc, kp, pres, n_kp_d, depth, frame_id_h, (size_t)seq->S * seq->cfg.n_cap, stream,
+                            "vo_seq_push_all_dev");
+    free(pres);
+    return rc;
+}
+
+extern "C" int vo_seq_lost_frames_at(vo_seq *seq, int q, int32_t *out_h, void *stream) {
+    using namespace vo;
+    VO_REQUIRE(seq && out_h, "vo_seq_lost_frames_at: null argument");
+    VO_REQUIRE(q >= 0 && q < seq->S, "vo_seq_lost_frames_at: sequence %d outside [0, %d)", q, seq->S);
+    cudaStream_t st = (cudaStream_t)stream;
+    VO_CUDA(cudaMemcpyAsync(out_h, seq->lost + q, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    VO_CUDA(cudaStreamSynchronize(st));
+    return VO_OK;
 }
 
 extern "C" int vo_seq_read_at(vo_seq *seq, int q, int first, int count, double *poses_h, int32_t *info_h, void *stream) {

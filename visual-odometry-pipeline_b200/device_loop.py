@@ -188,6 +188,7 @@ class MultiDeviceLoop:
     B = S pairs (each sequence's current frame against its own keyframe) followed by the per-sequence policy and promotion on
     the device.  Sequence q draws from (seeds[q], its frame slot - 1), so `poses(q)` equals, bit for bit, what
     `DeviceLoop(seed=seeds[q])` gives for the same frames.  A sequence may start late, end early or skip steps (n_kp < 0).
+    `push_images` starts a step from the S camera images instead (batched ORB on the device, no host read per step).
 
     Options are DeviceLoop's (seed is the default seed base: seeds = seed + q when `seeds` is None)."""
 
@@ -252,6 +253,55 @@ class MultiDeviceLoop:
             stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
             check(self.ctx.lib.vo_seq_push_all(self.handle, _ptr(desc_a), _ptr(kp_a), _ptr(n_kp), _ptr(depth_a),
                                                _ptr(frame_no), stream), "vo_seq_push_all")
+
+    def push_images(self, images, depth, frame_no, present=None, nfeatures=500):
+        """One step of every sequence from its image: images uint8 torch tensor (S, H, W) gray or (S, H, W, 3) BGR, on the
+        device or pinned; depth (S, H, W) float32 (torch, device or pinned, or numpy); frame_no (S,) or one int; present
+        (S,) truthy where a sequence has a frame at this step (default: all).  ORB (cv2.ORB_create(nfeatures) semantics)
+        runs on all S images in one batched call (OrbExtractor.extract_batch with rows = n_cap) and the keypoint counts
+        reach the loop on the device (vo_seq_push_all_dev): the call only enqueues work.  The images of absent sequences
+        are extracted too (the batch has a fixed shape) and their results ignored.  A frame with more keypoints than n_cap
+        keeps its first n_cap rows (level-major, then row-major) and counts in lost_frames(q).  The loop holds the
+        images and depth until poses() synchronises; do not write into them before then.  Byte-descriptor loops with
+        kp_stride 2 only; nfeatures is read when the extractor is created, at the first call."""
+        c, S = self.cfg, self.n_seqs
+        if c.desc_is_f32 or c.kp_stride != 2:
+            raise ValueError("MultiDeviceLoop.push_images: ORB images need a byte-descriptor loop with kp_stride 2")
+        present = np.ones(S, np.int32) if present is None else np.ascontiguousarray(present, dtype=bool).astype(np.int32)
+        frame_no = np.ascontiguousarray(np.broadcast_to(np.asarray(frame_no), (S,)), dtype=np.int32)
+        if present.shape != (S,):
+            raise ValueError(f"MultiDeviceLoop.push_images: present {present.shape} must be ({S},)")
+        if not isinstance(images, torch.Tensor) or images.shape[0] != S:
+            raise ValueError(f"MultiDeviceLoop.push_images: images must be a torch tensor of {S} images")
+        if isinstance(depth, torch.Tensor):
+            depth_a = depth.to(torch.float32).contiguous()
+        else:
+            depth_a = np.ascontiguousarray(depth, dtype=np.float32)
+        if tuple(depth_a.shape) != (S, c.H, c.W):
+            raise ValueError(f"MultiDeviceLoop.push_images: depth {tuple(depth_a.shape)} != {(S, c.H, c.W)}")
+        if getattr(self, "_extractor", None) is None:
+            from .orb_frontend import OrbExtractor
+            self._extractor = OrbExtractor(c.H, c.W, nfeatures=nfeatures, device=self.device)
+        kp, desc, _, count = self._extractor.extract_batch(images, rows=c.n_cap)
+        # the kernels read pinned images and depth asynchronously: hold them (a dropped pinned tensor's block is handed to
+        # the next pin_memory() and overwritten) until poses() has synchronised; kp / desc / count are device tensors of
+        # this stream, ordered by it
+        self._keep.append((images, depth_a))
+        with torch.cuda.device(self.device):
+            stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
+            check(self.ctx.lib.vo_seq_push_all_dev(self.handle, _ptr(desc), _ptr(kp), _ptr(count), _ptr(present),
+                                                   _ptr(depth_a), _ptr(frame_no), stream), "vo_seq_push_all_dev")
+
+    def lost_frames(self, q):
+        """Frames of sequence q pushed by push_images (or vo_seq_push_all_dev) that lost keypoint rows: more keypoints than
+        n_cap, or an extractor flag (a pyramid level overflowed).  Synchronises the stream."""
+        if not 0 <= int(q) < self.n_seqs:
+            raise IndexError(f"MultiDeviceLoop: sequence {q} outside [0, {self.n_seqs})")
+        out = np.zeros(1, np.int32)
+        with torch.cuda.device(self.device):
+            stream = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
+            check(self.ctx.lib.vo_seq_lost_frames_at(self.handle, int(q), _ptr(out), stream), "vo_seq_lost_frames_at")
+        return int(out[0])
 
     def frames(self, q):
         """Frames pushed to sequence q."""
