@@ -27,12 +27,13 @@
 extern "C" {
 #endif
 
-#define VO_ABI_VERSION 5   /* 2: vo_pipeline_args.u8_bytes, vo_pnp_ransac_ref, VO_NORM_HAMMING_TC, vo_orb_debug_read
+#define VO_ABI_VERSION 6   /* 2: vo_pipeline_args.u8_bytes, vo_pnp_ransac_ref, VO_NORM_HAMMING_TC, vo_orb_debug_read
                              3: vo_bootstrap, vo_pnp_ransac_ref_batch, VO_ST_BAD_INPUT, the pnp_mode / ref_* fields of
                                 vo_pipeline_args and vo_seq_config
                              4: vo_seq_config.n_seqs / seeds, vo_seq_push_all, vo_seq_read_at, vo_seq_frames_at, vo_seq_graph_captures,
                                 vo_workspace_generation
-                             5: vo_orb_extract_batch, vo_seq_push_all_dev, vo_seq_lost_frames_at */
+                             5: vo_orb_extract_batch, vo_seq_push_all_dev, vo_seq_lost_frames_at
+                             6: vo_sift_extract_batch */
 
 #if defined(__GNUC__)
 #define VO_API __attribute__((visibility("default")))
@@ -509,6 +510,17 @@ VO_API int vo_orb_debug_read(vo_orb *orb, int what, int level, void *host_dst, s
  *   aux float [cap][4] = (size, angle in degrees, response, packed octave word), optional; count int32[2] =
  *   (keypoints written, raw candidates found: more than max_keypoints means the list was cut).  Rows are in OpenCV's
  *   order (sorted by x, y, ...; duplicates removed).
+ *   vo_sift_extract_batch (VERSION 6): S images in one call of the same launches as vo_sift_extract for that shape,
+ *   whatever S is.  images uint8 [S][H][W] (channels = 1) or [S][H][W][3] BGR, device or pinned host memory.  Outputs
+ *   (device): kp float [S][out_rows][2], desc float [S][out_rows][128], aux float [S][out_rows][4] (optional), count
+ *   int32 [S][2] = (rows written, flags) -- the layout vo_seq_push_all_dev reads: flag bit 0 = the raw list passed
+ *   max_keypoints (vo_sift_extract's count[1] > max_keypoints; which keypoints survive is then unspecified), bit 1 =
+ *   rows past out_rows were dropped.  Image s's rows are a prefix of what vo_sift_extract returns for it, bit for bit
+ *   (only the first min(unique, out_rows) descriptors are computed).  1 <= S <= 65535, out_rows >= 1; arguments are
+ *   checked before anything is enqueued.  Scratch is per image and grows to the largest S seen (growing synchronises
+ *   the device): about 117 MB per 1241 x 376 image (9 octaves of 6 Gaussian and 5 DoG fp32 planes on the doubled
+ *   image, plus the blur-temp plane), ~7.5 GB at S = 64.  vo_sift_extract is the S = 1 call with out_rows =
+ *   max_keypoints.
  */
 typedef struct vo_sift_config {
     int H, W;
@@ -520,6 +532,8 @@ VO_API void vo_sift_destroy(vo_sift *sift);
 VO_API int vo_sift_capacity(const vo_sift *sift);
 VO_API int vo_sift_extract(vo_sift *sift, const uint8_t *image, int channels, float *kp, float *desc, float *aux,
                     int32_t *count, void *stream);
+VO_API int vo_sift_extract_batch(vo_sift *sift, const uint8_t *images, int S, int channels, int out_rows, float *kp,
+                          float *desc, float *aux, int32_t *count, void *stream);
 
 #ifdef __cplusplus
 }

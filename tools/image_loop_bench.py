@@ -1,16 +1,19 @@
 #!/usr/bin/env python
-"""S camera streams from images to poses: the batched ORB front-end (OrbExtractor.extract_batch) and the keyframe loop fed
-from it (MultiDeviceLoop.push_images: one batched extraction and one vo_pipeline(B = S) per step, keypoint counts on the
-device) against the one-stream path (OrbExtractor.extract per image; DeviceLoop.push_image, S loops run one after another
-on the same stream).  KITTI-shaped BGR frames (1241 x 376: a window panning 5 pixels per frame over a seeded texture, 8
-distinct sequences) and depth maps in pinned host memory, ORB 500 (cv2.ORB_create() defaults), Hamming + mutual, Mode T.
-Prints one JSON line per S with medians of --reps timed runs, launches per step, whether the last sequence equals its
-single loop bit for bit, and the GPU's name and power limit read in the same call.
+"""S camera streams from images to poses: the batched front-end (OrbExtractor / SiftExtractor.extract_batch) and the
+keyframe loop fed from it (MultiDeviceLoop.push_images: one batched extraction and one vo_pipeline(B = S) per step,
+keypoint counts on the device) against the one-stream path (extract per image; DeviceLoop.push_image, S loops run one after
+another on the same stream).  KITTI-shaped BGR frames (1241 x 376: a window panning 5 pixels per frame over a seeded
+texture, 8 distinct sequences) and depth maps in pinned host memory, Mode T.  --frontend orb: ORB 500 (cv2.ORB_create()
+defaults), Hamming + mutual, n_cap 1024.  --frontend sift: cv2.SIFT_create() defaults, L2 + ratio 0.85 on the default
+F16X1 pass, n_cap 8192 (above any frame's raw count, so the single loops' extractors never overflow); the record also
+gives the device memory the extractor's scratch takes at that S (cudaMemGetInfo before and after, less what torch's
+allocator took).  Prints one JSON line per S with medians of --reps timed runs, launches per step, whether the last
+sequence equals its single loop bit for bit, and the GPU's name and power limit read in the same call.
 
 One pinned step carries 1.40 MB of BGR image and 1.87 MB of depth per sequence: at S = 64, 209 MB, so the host-to-device
 copies alone bound a step from below (DESIGN 5 measured 55.4 GB/s pinned).
 
-  python tools/image_loop_bench.py [--s 1,4,16,64] [--frames 20] [--out profiles/image_loop_r05.json]
+  python tools/image_loop_bench.py [--frontend orb|sift] [--s 1,4,16,64] [--frames 20] [--out profiles/image_loop_r05.json]
 """
 import argparse
 import json
@@ -26,8 +29,11 @@ sys.path.insert(0, ROOT)
 
 H, W = 376, 1241
 N_BASE = 8
-OPTS = dict(kind="orb", norm_or_metric=0, mode=1, precision=0)
-N_CAP = 1024
+FRONTENDS = {
+    "orb": dict(opts=dict(kind="orb", norm_or_metric=0, mode=1, precision=0), n_cap=1024, workload="orb500_hamming_mutual_modeT"),
+    "sift": dict(opts=dict(kind="sift", norm_or_metric=0, mode=0, match_param=0.85), n_cap=8192,
+                 workload="sift_l2_ratio0.85_f16x1_modeT"),
+}
 
 
 def gpu_info():
@@ -52,6 +58,7 @@ def texture_frames(seed, n):
 
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument("--frontend", choices=sorted(FRONTENDS), default="orb")
     ap.add_argument("--s", default="1,4,16,64")
     ap.add_argument("--frames", type=int, default=20)
     ap.add_argument("--reps", type=int, default=5)
@@ -62,7 +69,11 @@ def main():
     from vo_b200 import ops, synthetic
     from vo_b200.device_loop import DeviceLoop, MultiDeviceLoop
     from vo_b200.orb_frontend import OrbExtractor
+    from vo_b200.sift_frontend import SiftExtractor
     assert torch.cuda.is_available(), "image_loop_bench needs a CUDA device"
+    fe = FRONTENDS[args.frontend]
+    OPTS, N_CAP = fe["opts"], fe["n_cap"]
+    sift = args.frontend == "sift"
     s_list = [int(x) for x in args.s.split(",")]
     F, S_max = args.frames, max(s_list)
     K = synthetic.KITTI_K
@@ -73,7 +84,19 @@ def main():
         for q in range(S_max):
             images[i, q] = torch.from_numpy(np.ascontiguousarray(bases[q % N_BASE][i]))
     depth = torch.full((S_max, H, W), 10.0, dtype=torch.float32).pin_memory()
-    orb = OrbExtractor(H, W)
+    ext = SiftExtractor(H, W) if sift else OrbExtractor(H, W)
+    rows = N_CAP if sift else None                              # SIFT: as push_images asks (max_keypoints rows would be 16 MB each)
+
+    def scratch_mb(S):
+        """Device memory a fresh extractor's scratch takes once it has run S images."""
+        torch.cuda.synchronize()
+        free0, res0 = torch.cuda.mem_get_info()[0], torch.cuda.memory_reserved()
+        e = SiftExtractor(H, W) if sift else OrbExtractor(H, W)
+        e.extract_batch(images[1, :S], rows=rows)
+        torch.cuda.synchronize()
+        free1, res1 = torch.cuda.mem_get_info()[0], torch.cuda.memory_reserved()
+        e.close()
+        return ((free0 - free1) - (res1 - res0)) / 1e6
 
     def timed(fn, reps):
         out = []
@@ -121,31 +144,40 @@ def main():
     run_single(1)                                               # warm every shape and the workspaces
     for S in s_list:
         resident = images[1, :S].cuda()
-        orb.extract_batch(images[1, :S]); orb.extract_batch(resident)
-        t_batch_pinned = timed(lambda: [orb.extract_batch(images[i % F, :S]) for i in range(10)], args.reps) / (10 * S)
-        t_batch_resident = timed(lambda: [orb.extract_batch(resident) for _ in range(10)], args.reps) / (10 * S)
-        t_each_pinned = timed(lambda: [orb.extract(images[1, q]) for q in range(S)], args.reps) / S
-        t_each_resident = timed(lambda: [orb.extract(resident[q]) for q in range(S)], args.reps) / S
+        ext.extract_batch(images[1, :S], rows=rows); ext.extract_batch(resident, rows=rows)
+        t_batch_pinned = timed(lambda: [ext.extract_batch(images[i % F, :S], rows=rows) for i in range(10)], args.reps) / (10 * S)
+        t_batch_resident = timed(lambda: [ext.extract_batch(resident, rows=rows) for _ in range(10)], args.reps) / (10 * S)
+        t_each_pinned = timed(lambda: [ext.extract(images[1, q]) for q in range(S)], args.reps) / S
+        t_each_resident = timed(lambda: [ext.extract(resident[q]) for q in range(S)], args.reps) / S
         l0 = ops.launch_count()
-        orb.extract_batch(images[1, :S])
+        count = ext.extract_batch(images[1, :S], rows=rows)[3]
         batch_launches = ops.launch_count() - l0
+        l0 = ops.launch_count()
+        ext.extract(images[1, 0])
+        extract_launches = ops.launch_count() - l0
+        kp_per_image = float(count[:, 0].float().mean())
         multi = [run_multi(S) for _ in range(args.reps)]
         t_multi = float(np.median([m[0] for m in multi]))
         single = [run_single(S) for _ in range(args.reps if S <= 16 else 1)]
         t_single = float(np.median([s[0] for s in single]))
         same = bool(np.array_equal(multi[0][1][0], single[0][1][0]) and np.array_equal(multi[0][1][1], single[0][1][1]))
         steps = F - 1
-        rec = dict(S=S, frames=F, frame="1241x376 BGR", nfeatures=500, n_cap=N_CAP, workload="orb500_hamming_mutual_modeT",
+        rec = dict(S=S, frames=F, frame="1241x376 BGR", frontend=args.frontend, n_cap=N_CAP, workload=fe["workload"],
                    extract_batch_us_per_image_pinned=1e6 * t_batch_pinned,
                    extract_batch_us_per_image_resident=1e6 * t_batch_resident,
                    extract_us_per_image_pinned=1e6 * t_each_pinned, extract_us_per_image_resident=1e6 * t_each_resident,
-                   extract_batch_launches_per_call=batch_launches,
+                   extract_batch_launches_per_call=batch_launches, extract_launches_per_call=extract_launches,
+                   keypoints_per_image=kp_per_image,
                    push_images_fps=S * steps / t_multi, push_images_ms_per_step=1e3 * t_multi / steps,
                    sequential_push_image_fps=S * steps / t_single, speedup=t_single / t_multi,
                    launches_per_step_push_images=multi[0][2], launches_per_step_sequential=single[0][2],
                    h2d_mb_per_step=S * (H * W * 3 + H * W * 4) / 1e6, equal_to_single=same,
                    keyframes_last_seq=int(multi[0][1][1][:, 5].sum()), matches_last_seq=float(multi[0][1][1][1:, 1].mean()),
                    **gpu_info())
+        if sift:
+            rec["scratch_mb"] = scratch_mb(S)
+        else:
+            rec["nfeatures"] = 500
         print(json.dumps(rec), flush=True)
         results.append(rec)
         del resident

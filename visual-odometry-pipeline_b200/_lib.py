@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("VO_B200_LIB") or os.path.join(_HERE, "libvo_b200.so")   # (override: A/B runs of two builds)
 
 # ---- constants mirrored from include/vo_b200.h ---------------------------------------------
-VO_ABI_VERSION = 5
+VO_ABI_VERSION = 6
 VO_OK, VO_ERR_ARG, VO_ERR_CUDA, VO_ERR_UNSUPPORTED = 0, -1, -2, -3
 VO_ST_OK, VO_ST_NO_MODEL, VO_ST_TOO_FEW_POINTS, VO_ST_KP_OUT_OF_IMAGE, VO_ST_BAD_INPUT = 0, 1, 2, 4, 8
 VO_NORM_HAMMING, VO_NORM_L2_U8, VO_NORM_HAMMING_TC = 0, 1, 2
@@ -158,6 +158,7 @@ PROTOTYPES = {
     "vo_sift_destroy": (None, [c_void_p]),
     "vo_sift_capacity": (c_int, [c_void_p]),
     "vo_sift_extract": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "vo_sift_extract_batch": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vo_profile_enable": (c_int, [c_void_p, c_int]),
     "vo_profile_collect": (c_int, [c_void_p, c_void_p, c_void_p]),
 }

@@ -13,6 +13,12 @@
 // Candidates (26-neighbour extrema of the DoG stack) are refined and tested by one thread each and given their
 // orientations by one warp each; the keypoint list is then sorted exactly as OpenCV's KeyPointsFilter::removeDuplicatedSorted does (rank by
 // counting), duplicates are dropped, and one warp per keypoint accumulates the 4 x 4 x 8 descriptor.
+//
+// Batch (vo_sift_extract_batch): every kernel also runs over S images, the image index being the last grid dimension
+// (blockIdx.z of the per-pixel kernels, blockIdx.y of the grid-stride ones), so a call issues the same launches whatever
+// S is; vo_sift_extract is the S = 1 call.  Scratch is image-major: image s has its own Gaussian, DoG and blur-temp
+// planes, its own candidate / keypoint / sorted / unique lists (max_keypoints entries each) and its own count block.
+// Batching changes indexing only: image s's output rows are a prefix of what it alone gives, bit for bit.
 #include "common.cuh"
 #include "orb_math.cuh"
 #include <math.h>
@@ -27,6 +33,9 @@ constexpr int SIFT_G = SIFT_LAYERS + 3;   // Gaussian images per octave
 constexpr int SIFT_D = SIFT_LAYERS + 2;   // DoG images per octave
 constexpr int SIFT_BORDER = 5;
 constexpr int SIFT_KMAX = 33;             // longest Gaussian kernel (sigma 3.09 -> 25 taps)
+// count block of one image: [0] raw keypoint records, [1] unique keypoints, [2 + o] candidates of octave o
+constexpr int SIFT_CNT = 16;
+static_assert(2 + SIFT_MAX_OCT <= SIFT_CNT, "one candidate counter per octave");
 
 struct SiftOct {
     int w, h;
@@ -51,10 +60,14 @@ __device__ __forceinline__ int reflect101i(int i, int n) {
     return i;
 }
 
-// gray (or BGR) u8 -> fp32, up-sampled x2 (cv2.resize INTER_LINEAR semantics: half-pixel centres, clamped edges)
-__global__ void sift_upsample_kernel(const uint8_t *__restrict__ img, int channels, int W, int H, float *__restrict__ out) {
+// gray (or BGR) u8 -> fp32, up-sampled x2 (cv2.resize INTER_LINEAR semantics: half-pixel centres, clamped edges).
+// blockIdx.z: image (input images back to back, output planes out_img floats apart)
+__global__ void sift_upsample_kernel(const uint8_t *__restrict__ img, int channels, int W, int H, float *__restrict__ out,
+                                     size_t out_img) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
     if (x >= 2 * W) return;
+    img += (size_t)blockIdx.z * W * H * channels;
+    out += blockIdx.z * out_img;
     const float fx = (x + 0.5f) * 0.5f - 0.5f, fy = (y + 0.5f) * 0.5f - 0.5f;
     int x0 = (int)floorf(fx), y0 = (int)floorf(fy);
     float wx = fx - x0, wy = fy - y0;
@@ -75,12 +88,16 @@ __global__ void sift_upsample_kernel(const uint8_t *__restrict__ img, int channe
 // 11, 13, 17, 21, 27): the unrolled loop lets all loads of a pixel issue before the first use, and interior pixels skip the
 // border reflection.  The products and the left-to-right sum are rounded one by one as before (-fmad=false): same bits as
 // the generic loop, which stays for other lengths.  (Generic loop on a B200: 18-50 us per 2482 x 752 layer, latency-bound;
-// the blur passes were 52 % of the front-end after the orientation kernel got its warps.)
+// the blur passes were 52 % of the front-end after the orientation kernel got its warps.)  blockIdx.z: image (source
+// planes src_img floats apart, destination planes dst_img).
 template <int N>
 __global__ void __launch_bounds__(128)
-sift_blur_row_kernel(const float *__restrict__ src, int w, int h, SiftKernels K, int ki, float *__restrict__ dst) {
+sift_blur_row_kernel(const float *__restrict__ src, size_t src_img, int w, int h, SiftKernels K, int ki, float *__restrict__ dst,
+                     size_t dst_img) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
     if (x >= w) return;
+    src += blockIdx.z * src_img;
+    dst += blockIdx.z * dst_img;
     const int n = N > 0 ? N : K.ksize[ki], r = n / 2;
     const float *row = src + (size_t)y * w;
     float s = 0.f;
@@ -97,9 +114,12 @@ sift_blur_row_kernel(const float *__restrict__ src, int w, int h, SiftKernels K,
 }
 template <int N>
 __global__ void __launch_bounds__(128)
-sift_blur_col_kernel(const float *__restrict__ src, int w, int h, SiftKernels K, int ki, float *__restrict__ dst) {
+sift_blur_col_kernel(const float *__restrict__ src, size_t src_img, int w, int h, SiftKernels K, int ki, float *__restrict__ dst,
+                     size_t dst_img) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
     if (x >= w) return;
+    src += blockIdx.z * src_img;
+    dst += blockIdx.z * dst_img;
     const int n = N > 0 ? N : K.ksize[ki], r = n / 2;
     float s = 0.f;
     if (N > 0 && y >= r && y + r < h) {
@@ -114,14 +134,18 @@ sift_blur_col_kernel(const float *__restrict__ src, int w, int h, SiftKernels K,
     }
     dst[(size_t)y * w + x] = s;
 }
-__global__ void sift_decimate_kernel(const float *__restrict__ src, int sw, float *__restrict__ dst, int w, int h) {
+// blockIdx.z: image (src and dst both in the Gaussian buffer, g_img floats per image)
+__global__ void sift_decimate_kernel(const float *__restrict__ src, int sw, float *__restrict__ dst, int w, int h, size_t g_img) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
-    if (x < w) dst[(size_t)y * w + x] = src[(size_t)(2 * y) * sw + 2 * x];
+    const size_t o = blockIdx.z * g_img;
+    if (x < w) dst[o + (size_t)y * w + x] = src[o + (size_t)(2 * y) * sw + 2 * x];
 }
-// the five DoG layers of one octave: grid.y = 5 * h
-__global__ void sift_dog_kernel(const float *__restrict__ g, int w, int h, float *__restrict__ d) {
+// the five DoG layers of one octave: grid.y = 5 * h, blockIdx.z: image
+__global__ void sift_dog_kernel(const float *__restrict__ g, size_t g_img, int w, int h, float *__restrict__ d, size_t d_img) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x;
     if (x >= w) return;
+    g += blockIdx.z * g_img;
+    d += blockIdx.z * d_img;
     const size_t i = (size_t)blockIdx.y * w + x;       // layer * h * w + y * w + x
     d[i] = g[i + (size_t)w * h] - g[i];
 }
@@ -150,11 +174,15 @@ struct SiftCand {
     int32_t r, c, layer, octave;
     float xc, xr, contr, size;
 };
-__global__ void sift_extrema_kernel(const float *__restrict__ dog, int w, int h, int octv, int threshold,
+// blockIdx.z: image (DoG planes d_img floats apart, cap candidates and a SIFT_CNT count block per image)
+__global__ void sift_extrema_kernel(const float *__restrict__ dog, size_t d_img, int w, int h, int octv, int threshold,
                                     SiftCand *__restrict__ cands, int32_t *__restrict__ n_cand, int cap) {
     const int c0 = blockIdx.x * blockDim.x + threadIdx.x;
     const int layer0 = 1 + blockIdx.y / h, r0 = blockIdx.y % h;
     if (c0 < SIFT_BORDER || c0 >= w - SIFT_BORDER || r0 < SIFT_BORDER || r0 >= h - SIFT_BORDER) return;
+    dog += blockIdx.z * d_img;
+    cands += (size_t)blockIdx.z * cap;
+    n_cand += SIFT_CNT * blockIdx.z;
     const size_t plane = (size_t)w * h;
     {
         const float *cur = dog + layer0 * plane, *prv = cur - plane, *nxt = cur + plane;
@@ -224,13 +252,19 @@ __global__ void sift_extrema_kernel(const float *__restrict__ dog, int w, int h,
 // calcOrientationHist + the peak loop of findScaleSpaceExtrema, one warp (= one CTA of 32 threads) per candidate: the rows of
 // the (2 r + 1)^2 window are dealt to the lanes, every lane accumulates its own 36-bin partial histogram in shared memory
 // (bin-major, lane-minor: no bank conflicts, no atomics), the 32 partials of a bin are summed in lane order, and lane 0
-// smooths, finds the peaks and appends one keypoint per peak: the result does not depend on scheduling.
+// smooths, finds the peaks and appends one keypoint per peak: the result does not depend on scheduling.  blockIdx.y:
+// image (Gaussian planes g_img floats apart; cap candidates, cap keypoints and a SIFT_CNT count block per image).
 __global__ void __launch_bounds__(32)
-sift_orient_kernel(const float *__restrict__ gauss, int w, int h, int octv, const SiftCand *__restrict__ cands,
-                   const int32_t *__restrict__ n_cand, int cand_cap, SiftKp *__restrict__ kps, int32_t *__restrict__ count, int cap) {
+sift_orient_kernel(const float *__restrict__ gauss, size_t g_img, int w, int h, int octv, const SiftCand *__restrict__ cands,
+                   const int32_t *__restrict__ n_cand, SiftKp *__restrict__ kps, int32_t *__restrict__ count, int cap) {
     __shared__ float part[36 * 32];
     __shared__ float temp[36 + 4];
-    const int n = min(n_cand[0], cand_cap), lane = threadIdx.x;
+    gauss += blockIdx.y * g_img;
+    cands += (size_t)blockIdx.y * cap;
+    kps += (size_t)blockIdx.y * cap;
+    n_cand += SIFT_CNT * blockIdx.y;
+    count += SIFT_CNT * blockIdx.y;
+    const int n = min(n_cand[0], cap), lane = threadIdx.x;
     const size_t plane = (size_t)w * h;
     const float oscale = (float)(1 << octv);
     for (int idx = blockIdx.x; idx < n; idx += gridDim.x) {
@@ -292,9 +326,11 @@ sift_orient_kernel(const float *__restrict__ gauss, int w, int h, int octv, cons
     }
 }
 
-// First octave is -1: halve coordinates and size and rewrite the octave byte (SIFT_Impl::detectAndCompute).
+// First octave is -1: halve coordinates and size and rewrite the octave byte (SIFT_Impl::detectAndCompute).  blockIdx.y:
+// image (also in the rank, unique and descriptor kernels below).
 __global__ void sift_rescale_kernel(SiftKp *__restrict__ kps, const int32_t *__restrict__ count, int cap) {
-    const int n = min(count[0], cap);
+    kps += (size_t)blockIdx.y * cap;
+    const int n = min(count[SIFT_CNT * blockIdx.y], cap);
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         SiftKp k = kps[i];
         k.x *= 0.5f; k.y *= 0.5f; k.size *= 0.5f;
@@ -320,7 +356,9 @@ constexpr int SIFT_RANK_T = 256;
 __global__ void __launch_bounds__(SIFT_RANK_T)
 sift_rank_kernel(const SiftKp *__restrict__ kps, const int32_t *__restrict__ count, int cap, SiftKp *__restrict__ sorted) {
     __shared__ SiftKp tile[SIFT_RANK_T];
-    const int n = min(count[0], cap);
+    kps += (size_t)blockIdx.y * cap;
+    sorted += (size_t)blockIdx.y * cap;
+    const int n = min(count[SIFT_CNT * blockIdx.y], cap);
     for (int i0 = blockIdx.x * SIFT_RANK_T; i0 < n; i0 += gridDim.x * SIFT_RANK_T) {   // block-uniform loop: barriers inside
         const int i = i0 + threadIdx.x;
         SiftKp k = kps[min(i, n - 1)];
@@ -336,12 +374,15 @@ sift_rank_kernel(const SiftKp *__restrict__ kps, const int32_t *__restrict__ cou
         if (i < n) sorted[rank] = k;
     }
 }
-// Drop records that repeat (x, y, size, angle) of their predecessor, keep the order.  One CTA; chunks of blockDim.
+// Drop records that repeat (x, y, size, angle) of their predecessor, keep the order.  One CTA per image; chunks of
+// blockDim.  count[1] of the image's block = unique keypoints.
 __global__ void __launch_bounds__(1024)
-sift_unique_kernel(const SiftKp *__restrict__ sorted, const int32_t *__restrict__ count, int cap, SiftKp *__restrict__ out,
-                   int32_t *__restrict__ out_count) {
+sift_unique_kernel(const SiftKp *__restrict__ sorted, int32_t *__restrict__ count, int cap, SiftKp *__restrict__ out) {
     __shared__ int scan[1024];
     __shared__ int base_s;
+    sorted += (size_t)blockIdx.y * cap;
+    out += (size_t)blockIdx.y * cap;
+    count += SIFT_CNT * blockIdx.y;
     const int n = min(count[0], cap);
     if (threadIdx.x == 0) base_s = 0;
     __syncthreads();
@@ -370,19 +411,32 @@ sift_unique_kernel(const SiftKp *__restrict__ sorted, const int32_t *__restrict_
         if (threadIdx.x == 0) base_s += scan[blockDim.x - 1];
         __syncthreads();
     }
-    if (threadIdx.x == 0) out_count[0] = base_s;
+    if (threadIdx.x == 0) count[1] = base_s;
 }
 
 // calcSIFTDescriptor, one warp (= one CTA of 32 threads) per keypoint.  The (2 r + 1)^2 samples are dealt to the lanes by
 // row; every lane accumulates its own 6 x 6 x 10 partial histogram in shared memory (bin-major, lane-minor: no bank
 // conflicts, no atomics), the 32 partials are summed in lane order, and lane 0 finishes (circular wrap, clipping,
-// normalisation): the result does not depend on scheduling.
+// normalisation): the result does not depend on scheduling.  Only the first out_rows keypoints of an image are written;
+// count_out (optional) [img] = (rows written, flags: 1 = the raw list passed cap, 2 = rows past out_rows were dropped).
 constexpr int SIFT_HIST = 6 * 6 * 10;
 __global__ void __launch_bounds__(32)
-sift_desc_kernel(SiftGeom G, const float *__restrict__ gauss, const SiftKp *__restrict__ kps, const int32_t *__restrict__ n_kp,
-                 float *__restrict__ kp_out, float *__restrict__ aux, float *__restrict__ desc) {
+sift_desc_kernel(SiftGeom G, const float *__restrict__ gauss, size_t g_img, const SiftKp *__restrict__ kps,
+                 const int32_t *__restrict__ counts, int cap, int out_rows, float *__restrict__ kp_out, float *__restrict__ aux,
+                 float *__restrict__ desc, int32_t *__restrict__ count_out) {
     __shared__ float part[SIFT_HIST * 32];
-    const int n = n_kp[0], lane = threadIdx.x;
+    const int img_i = blockIdx.y, lane = threadIdx.x;
+    gauss += img_i * g_img;
+    kps += (size_t)img_i * cap;
+    counts += SIFT_CNT * img_i;
+    kp_out += (size_t)img_i * out_rows * 2;
+    desc += (size_t)img_i * out_rows * 128;
+    if (aux) aux += (size_t)img_i * out_rows * 4;
+    const int n_unique = counts[1], n = min(n_unique, out_rows);
+    if (count_out && blockIdx.x == 0 && lane == 0) {
+        count_out[2 * img_i] = n;
+        count_out[2 * img_i + 1] = (counts[0] > cap ? 1 : 0) | (n_unique > out_rows ? 2 : 0);
+    }
     for (int idx = blockIdx.x; idx < n; idx += gridDim.x) {
         const SiftKp k = kps[idx];
         if (lane == 0) {
@@ -461,12 +515,14 @@ sift_desc_kernel(SiftGeom G, const float *__restrict__ gauss, const SiftKp *__re
     }
 }
 
-// row pass src -> tmp, column pass tmp -> dst with kernel ki; the unrolled instantiation when the length is one of the scale space's
-int sift_blur(vo_ctx *ctx, dim3 grid, cudaStream_t st, const float *src, int w, int h, const SiftKernels &K, int ki, float *tmp, float *dst) {
-#define VO_SIFT_BLUR(N)                                                                  \
-    VO_LAUNCH(sift_blur_row_kernel<N>, grid, 128, st, src, w, h, K, ki, tmp);            \
-    VO_LAUNCH_CHECK(ctx);                                                                \
-    VO_LAUNCH(sift_blur_col_kernel<N>, grid, 128, st, tmp, w, h, K, ki, dst)
+// row pass src -> tmp, column pass tmp -> dst with kernel ki; the unrolled instantiation when the length is one of the scale space's.
+// grid.z images: src and dst planes g_img floats apart, tmp planes t_img.
+int sift_blur(vo_ctx *ctx, dim3 grid, cudaStream_t st, const float *src, int w, int h, const SiftKernels &K, int ki, float *tmp,
+              float *dst, size_t g_img, size_t t_img) {
+#define VO_SIFT_BLUR(N)                                                                        \
+    VO_LAUNCH(sift_blur_row_kernel<N>, grid, 128, st, src, g_img, w, h, K, ki, tmp, t_img);    \
+    VO_LAUNCH_CHECK(ctx);                                                                      \
+    VO_LAUNCH(sift_blur_col_kernel<N>, grid, 128, st, tmp, t_img, w, h, K, ki, dst, g_img)
     switch (K.ksize[ki]) {
         case 11: VO_SIFT_BLUR(11); break;
         case 13: VO_SIFT_BLUR(13); break;
@@ -486,21 +542,60 @@ int sift_blur(vo_ctx *ctx, dim3 grid, cudaStream_t st, const float *src, int w, 
 struct vo_sift {
     vo_ctx *ctx;
     int H, W, cap;
+    int S_cap;            // images the scratch holds (the largest batch seen so far)
+    size_t g_img, d_img;  // floats of one image's Gaussian / DoG planes (all octaves)
     vo::SiftGeom G;
     vo::SiftKernels K;
     float *gauss, *dog, *tmp;
     vo::SiftKp *kps, *sorted, *uniq;
-    int32_t *counts;   // [0] raw count, [1] final count, [2] candidates of the octave in flight
+    int32_t *counts;      // per image: SIFT_CNT words ([0] raw count, [1] final count, [2 + o] candidates of octave o)
     vo::SiftCand *cands;
 };
+
+namespace vo {
+namespace {
+
+void sift_free(vo_sift *s) {
+    void **ptrs[] = {(void **)&s->gauss, (void **)&s->dog, (void **)&s->tmp, (void **)&s->kps, (void **)&s->sorted,
+                     (void **)&s->uniq, (void **)&s->counts, (void **)&s->cands};
+    for (void **p : ptrs) {
+        if (*p) cudaFree(*p);
+        *p = nullptr;
+    }
+    s->S_cap = 0;
+}
+
+// Scratch for S images (a KITTI-shaped 1241 x 376 image takes ~117 MB, nearly all of it the fp32 planes).  Growing
+// drains the device first (work queued on any stream may still use the old blocks), as ws_get does.
+int sift_reserve(vo_sift *s, int S) {
+    if (S <= s->S_cap) return VO_OK;
+    cudaSetDevice(s->ctx->device);
+    if (s->S_cap) VO_CUDA(cudaDeviceSynchronize());
+    sift_free(s);
+    const size_t n = (size_t)S, cap = (size_t)s->cap, t_img = (size_t)s->G.o[0].w * s->G.o[0].h;
+    cudaError_t e = cudaSuccess;
+    auto alloc = [&](void **p, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(p, bytes ? bytes : 16); };
+    alloc((void **)&s->gauss, n * s->g_img * 4); alloc((void **)&s->dog, n * s->d_img * 4); alloc((void **)&s->tmp, n * t_img * 4);
+    alloc((void **)&s->kps, sizeof(SiftKp) * n * cap); alloc((void **)&s->sorted, sizeof(SiftKp) * n * cap);
+    alloc((void **)&s->uniq, sizeof(SiftKp) * n * cap); alloc((void **)&s->counts, sizeof(int32_t) * SIFT_CNT * n);
+    alloc((void **)&s->cands, sizeof(SiftCand) * n * cap);
+    if (e != cudaSuccess) {
+        sift_free(s);
+        set_error("SIFT scratch for %d images: cudaMalloc -> %s", S, cudaGetErrorString(e));
+        return VO_ERR_CUDA;
+    }
+    s->S_cap = S;
+    return VO_OK;
+}
+
+}  // namespace
+}  // namespace vo
 
 extern "C" void vo_sift_destroy(vo_sift *s) {
     if (!s) return;
     cudaSetDevice(s->ctx->device);
     cudaDeviceSynchronize();
-    void *ptrs[] = {s->gauss, s->dog, s->tmp, s->kps, s->sorted, s->uniq, s->counts, s->cands};
-    for (void *p : ptrs)
-        if (p) cudaFree(p);
+    vo::sift_free(s);
     delete s;
 }
 extern "C" int vo_sift_capacity(const vo_sift *s) { return s ? s->cap : 0; }
@@ -527,6 +622,7 @@ extern "C" int vo_sift_create(vo_ctx *ctx, const vo_sift_config *cfg, vo_sift **
         w /= 2; h /= 2;
         if (w < 1 || h < 1) { s->G.n_oct = o + 1; break; }
     }
+    s->g_img = g_ofs; s->d_img = d_ofs;
     // Gaussian kernels: [0] the base blur, [i] the increment from layer i - 1 to layer i
     double sig[SIFT_G];
     sig[0] = sqrt(fmax(1.6 * 1.6 - 0.5 * 0.5 * 4, 0.01));
@@ -544,73 +640,101 @@ extern "C" int vo_sift_create(vo_ctx *ctx, const vo_sift_config *cfg, vo_sift **
         for (int j = 0; j < ks; ++j) { const double x = j - (ks - 1) * 0.5; e[j] = exp(-(x * x) / (2.0 * sig[i] * sig[i])); sum += e[j]; }
         for (int j = 0; j < ks; ++j) s->K.k[i][j] = (float)(e[j] / sum);
     }
-    cudaError_t e = cudaSuccess;
-    auto alloc = [&](void **p, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(p, bytes ? bytes : 16); };
-    cudaSetDevice(ctx->device);
-    alloc((void **)&s->gauss, g_ofs * 4); alloc((void **)&s->dog, d_ofs * 4); alloc((void **)&s->tmp, (size_t)bw * bh * 4);
-    alloc((void **)&s->kps, sizeof(SiftKp) * (size_t)s->cap); alloc((void **)&s->sorted, sizeof(SiftKp) * (size_t)s->cap);
-    alloc((void **)&s->uniq, sizeof(SiftKp) * (size_t)s->cap); alloc((void **)&s->counts, sizeof(int32_t) * 4);
-    alloc((void **)&s->cands, sizeof(SiftCand) * (size_t)s->cap);
-    if (e != cudaSuccess) {
-        set_error("vo_sift_create: cudaMalloc -> %s", cudaGetErrorString(e));
+    if (const int rc = sift_reserve(s, 1)) {
         vo_sift_destroy(s);
-        return VO_ERR_CUDA;
+        return rc;
     }
     *out = s;
     return VO_OK;
 }
 
-extern "C" int vo_sift_extract(vo_sift *s, const uint8_t *image, int channels, float *kp, float *desc, float *aux,
-                               int32_t *count, void *stream) {
-    using namespace vo;
-    VO_REQUIRE(s && image && kp && desc && count, "vo_sift_extract: null argument");
-    VO_REQUIRE(channels == 1 || channels == 3, "vo_sift_extract: image must have 1 (gray) or 3 (BGR) channels, got %d", channels);
+namespace vo {
+namespace {
+
+// CTAs per image of a grid-stride kernel: the one-image grid `one` spread over the batch, at least `least` per image
+int sift_ctas(int one, int S, int least) { return ceil_div(one, S) > least ? ceil_div(one, S) : least; }
+
+// The one launch sequence of the extractor: S images, out_rows output rows per image.  The launches depend on the image
+// shape only, not on S.  count (optional) [S][2] = (rows written, flags), written by the descriptor kernel.
+int sift_run(vo_sift *s, const uint8_t *images, int S, int channels, int out_rows, float *kp, float *desc, float *aux,
+             int32_t *count, void *stream) {
     vo_ctx *ctx = s->ctx;
     cudaStream_t st = (cudaStream_t)stream;
+    if (int rc = sift_reserve(s, S)) return rc;
     const SiftGeom &G = s->G;
-    VO_CUDA(cudaMemsetAsync(s->counts, 0, sizeof(int32_t) * 4, st));
+    const size_t g_img = s->g_img, d_img = s->d_img;
     const SiftOct &o0 = G.o[0];
+    const size_t t_img = (size_t)o0.w * o0.h;
+    // every image's count block, the per-octave candidate counters included, is zeroed here once
+    VO_CUDA(cudaMemsetAsync(s->counts, 0, sizeof(int32_t) * SIFT_CNT * S, st));
     float *g00 = s->gauss + o0.g_ofs;
     // base image: up-sample into layer 1's slot (free until it is computed), blur into layer 0
     float *scratch = g00 + (size_t)o0.w * o0.h;
-    VO_LAUNCH(sift_upsample_kernel, dim3(ceil_div(o0.w, 128), o0.h), 128, st, image, channels, s->W, s->H, scratch);
+    VO_LAUNCH(sift_upsample_kernel, dim3(ceil_div(o0.w, 128), o0.h, S), 128, st, images, channels, s->W, s->H, scratch, g_img);
     VO_LAUNCH_CHECK(ctx);
-    if (int rc = sift_blur(ctx, dim3(ceil_div(o0.w, 128), o0.h), st, scratch, o0.w, o0.h, s->K, 0, s->tmp, g00)) return rc;
+    if (int rc = sift_blur(ctx, dim3(ceil_div(o0.w, 128), o0.h, S), st, scratch, o0.w, o0.h, s->K, 0, s->tmp, g00, g_img, t_img))
+        return rc;
     const int threshold = (int)floor(0.5 * 0.04 / SIFT_LAYERS * 255);
+    const int per_img = sift_ctas(1184, S, 8);   // one-image grid: 8 CTAs per SM, striding
     for (int o = 0; o < G.n_oct; ++o) {
         const SiftOct &oc = G.o[o];
         const size_t plane = (size_t)oc.w * oc.h;
         float *g = s->gauss + oc.g_ofs, *d = s->dog + oc.d_ofs;
-        const dim3 grid(ceil_div(oc.w, 128), oc.h);
+        const dim3 grid(ceil_div(oc.w, 128), oc.h, S);
         if (o > 0) {
             const SiftOct &pv = G.o[o - 1];
-            VO_LAUNCH(sift_decimate_kernel, grid, 128, st, s->gauss + pv.g_ofs + (size_t)SIFT_LAYERS * pv.w * pv.h, pv.w, g, oc.w, oc.h);
+            VO_LAUNCH(sift_decimate_kernel, grid, 128, st, s->gauss + pv.g_ofs + (size_t)SIFT_LAYERS * pv.w * pv.h, pv.w, g, oc.w,
+                      oc.h, g_img);
             VO_LAUNCH_CHECK(ctx);
         }
         for (int i = 1; i < SIFT_G; ++i) {
-            if (int rc = sift_blur(ctx, grid, st, g + (i - 1) * plane, oc.w, oc.h, s->K, i, s->tmp, g + i * plane)) return rc;
+            if (int rc = sift_blur(ctx, grid, st, g + (i - 1) * plane, oc.w, oc.h, s->K, i, s->tmp, g + i * plane, g_img, t_img))
+                return rc;
         }
-        VO_LAUNCH(sift_dog_kernel, dim3(ceil_div(oc.w, 128), SIFT_D * oc.h), 128, st, g, oc.w, oc.h, d);
+        VO_LAUNCH(sift_dog_kernel, dim3(ceil_div(oc.w, 128), SIFT_D * oc.h, S), 128, st, g, g_img, oc.w, oc.h, d, d_img);
         VO_LAUNCH_CHECK(ctx);
         if (oc.w > 2 * SIFT_BORDER && oc.h > 2 * SIFT_BORDER) {
-            VO_CUDA(cudaMemsetAsync(s->counts + 2, 0, sizeof(int32_t), st));
-            VO_LAUNCH(sift_extrema_kernel, dim3(ceil_div(oc.w, 128), SIFT_LAYERS * oc.h), 128, st, d, oc.w, oc.h, o, threshold,
-                      s->cands, s->counts + 2, s->cap);
+            VO_LAUNCH(sift_extrema_kernel, dim3(ceil_div(oc.w, 128), SIFT_LAYERS * oc.h, S), 128, st, d, d_img, oc.w, oc.h, o,
+                      threshold, s->cands, s->counts + 2 + o, s->cap);
             VO_LAUNCH_CHECK(ctx);
-            VO_LAUNCH_BAR(sift_orient_kernel, 1184, 32, st, g, oc.w, oc.h, o, s->cands, s->counts + 2, s->cap, s->kps, s->counts, s->cap);
+            VO_LAUNCH_BAR(sift_orient_kernel, dim3(per_img, S), 32, st, g, g_img, oc.w, oc.h, o, s->cands, s->counts + 2 + o,
+                          s->kps, s->counts, s->cap);
             VO_LAUNCH_CHECK(ctx);
         }
     }
-    VO_LAUNCH(sift_rescale_kernel, 32, 256, st, s->kps, s->counts, s->cap);
+    VO_LAUNCH(sift_rescale_kernel, dim3(sift_ctas(32, S, 4), S), 256, st, s->kps, s->counts, s->cap);
     VO_LAUNCH_CHECK(ctx);
-    VO_LAUNCH_BAR(sift_rank_kernel, 64, SIFT_RANK_T, st, s->kps, s->counts, s->cap, s->sorted);
+    VO_LAUNCH_BAR(sift_rank_kernel, dim3(sift_ctas(64, S, 16), S), SIFT_RANK_T, st, s->kps, s->counts, s->cap, s->sorted);
     VO_LAUNCH_CHECK(ctx);
-    VO_LAUNCH_BAR(sift_unique_kernel, 1, 1024, st, s->sorted, s->counts, s->cap, s->uniq, s->counts + 1);
+    VO_LAUNCH_BAR(sift_unique_kernel, dim3(1, S), 1024, st, s->sorted, s->counts, s->cap, s->uniq);
     VO_LAUNCH_CHECK(ctx);
-    VO_LAUNCH_BAR(sift_desc_kernel, 1184, 32, st, G, s->gauss, s->uniq, s->counts + 1, kp, aux, desc);   // 8 CTAs per SM, striding
+    VO_LAUNCH_BAR(sift_desc_kernel, dim3(per_img, S), 32, st, G, s->gauss, g_img, s->uniq, s->counts, s->cap, out_rows, kp, aux,
+                  desc, count);
     VO_LAUNCH_CHECK(ctx);
+    return VO_OK;
+}
+
+}  // namespace
+}  // namespace vo
+
+extern "C" int vo_sift_extract(vo_sift *s, const uint8_t *image, int channels, float *kp, float *desc, float *aux,
+                               int32_t *count, void *stream) {
+    VO_REQUIRE(s && image && kp && desc && count, "vo_sift_extract: null argument");
+    VO_REQUIRE(channels == 1 || channels == 3, "vo_sift_extract: image must have 1 (gray) or 3 (BGR) channels, got %d", channels);
+    if (int rc = vo::sift_run(s, image, 1, channels, s->cap, kp, desc, aux, nullptr, stream)) return rc;
     // count[0] = keypoints written, count[1] = raw candidates found (> max_keypoints: the list was cut)
+    cudaStream_t st = (cudaStream_t)stream;
     VO_CUDA(cudaMemcpyAsync(count, s->counts + 1, sizeof(int32_t), cudaMemcpyDefault, st));
     VO_CUDA(cudaMemcpyAsync(count + 1, s->counts, sizeof(int32_t), cudaMemcpyDefault, st));
     return VO_OK;
+}
+
+extern "C" int vo_sift_extract_batch(vo_sift *s, const uint8_t *images, int S, int channels, int out_rows, float *kp, float *desc,
+                                     float *aux, int32_t *count, void *stream) {
+    VO_REQUIRE(s && images && kp && desc && count, "vo_sift_extract_batch: null argument");
+    VO_REQUIRE(channels == 1 || channels == 3, "vo_sift_extract_batch: images must have 1 (gray) or 3 (BGR) channels, got %d",
+               channels);
+    VO_REQUIRE(S >= 1 && S <= 65535, "vo_sift_extract_batch: %d images outside [1, 65535]", S);
+    VO_REQUIRE(out_rows >= 1, "vo_sift_extract_batch: out_rows %d must be >= 1", out_rows);
+    return vo::sift_run(s, images, S, channels, out_rows, kp, desc, aux, count, stream);
 }

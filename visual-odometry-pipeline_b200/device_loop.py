@@ -188,7 +188,7 @@ class MultiDeviceLoop:
     B = S pairs (each sequence's current frame against its own keyframe) followed by the per-sequence policy and promotion on
     the device.  Sequence q draws from (seeds[q], its frame slot - 1), so `poses(q)` equals, bit for bit, what
     `DeviceLoop(seed=seeds[q])` gives for the same frames.  A sequence may start late, end early or skip steps (n_kp < 0).
-    `push_images` starts a step from the S camera images instead (batched ORB on the device, no host read per step).
+    `push_images` starts a step from the S camera images instead (batched ORB or SIFT on the device, no host read per step).
 
     Options are DeviceLoop's (seed is the default seed base: seeds = seed + q when `seeds` is None)."""
 
@@ -254,19 +254,25 @@ class MultiDeviceLoop:
             check(self.ctx.lib.vo_seq_push_all(self.handle, _ptr(desc_a), _ptr(kp_a), _ptr(n_kp), _ptr(depth_a),
                                                _ptr(frame_no), stream), "vo_seq_push_all")
 
-    def push_images(self, images, depth, frame_no, present=None, nfeatures=500):
+    def push_images(self, images, depth, frame_no, present=None, nfeatures=500, max_keypoints=32768):
         """One step of every sequence from its image: images uint8 torch tensor (S, H, W) gray or (S, H, W, 3) BGR, on the
         device or pinned; depth (S, H, W) float32 (torch, device or pinned, or numpy); frame_no (S,) or one int; present
-        (S,) truthy where a sequence has a frame at this step (default: all).  ORB (cv2.ORB_create(nfeatures) semantics)
-        runs on all S images in one batched call (OrbExtractor.extract_batch with rows = n_cap) and the keypoint counts
+        (S,) truthy where a sequence has a frame at this step (default: all).  The front-end follows the loop's
+        descriptors, as in DeviceLoop.push_image: a byte-descriptor loop runs ORB (cv2.ORB_create(nfeatures) semantics,
+        OrbExtractor.extract_batch), a float-descriptor loop with kp_stride 2 runs SIFT (cv2.SIFT_create() semantics,
+        SiftExtractor.extract_batch), each on all S images in one batched call with rows = n_cap, and the keypoint counts
         reach the loop on the device (vo_seq_push_all_dev): the call only enqueues work.  The images of absent sequences
         are extracted too (the batch has a fixed shape) and their results ignored.  A frame with more keypoints than n_cap
-        keeps its first n_cap rows (level-major, then row-major) and counts in lost_frames(q).  The loop holds the
-        images and depth until poses() synchronises; do not write into them before then.  Byte-descriptor loops with
-        kp_stride 2 only; nfeatures is read when the extractor is created, at the first call."""
+        keeps its first n_cap rows and counts in lost_frames(q): for ORB level-major, then row-major; for SIFT in OpenCV's
+        order (sorted by x), so the left of the image is kept.  A SIFT frame whose raw list passes max_keypoints (the raw
+        candidate capacity per image) counts too.  SIFT descriptors are integers in 0..255 by construction, so the default
+        F16X1 pass gets no integer check here (it would cost a host read per step).  The loop holds the images and depth
+        until poses() synchronises; do not write into them before then.  nfeatures (ORB) and max_keypoints (SIFT) are
+        read when the extractor is created, at the first call.  R2D2 loops (kp_stride 3) are refused."""
         c, S = self.cfg, self.n_seqs
-        if c.desc_is_f32 or c.kp_stride != 2:
-            raise ValueError("MultiDeviceLoop.push_images: ORB images need a byte-descriptor loop with kp_stride 2")
+        if c.kp_stride != 2:
+            raise ValueError("MultiDeviceLoop.push_images: images need an ORB (byte-descriptor) or SIFT (float-descriptor) "
+                             "loop with kp_stride 2")
         present = np.ones(S, np.int32) if present is None else np.ascontiguousarray(present, dtype=bool).astype(np.int32)
         frame_no = np.ascontiguousarray(np.broadcast_to(np.asarray(frame_no), (S,)), dtype=np.int32)
         if present.shape != (S,):
@@ -280,8 +286,12 @@ class MultiDeviceLoop:
         if tuple(depth_a.shape) != (S, c.H, c.W):
             raise ValueError(f"MultiDeviceLoop.push_images: depth {tuple(depth_a.shape)} != {(S, c.H, c.W)}")
         if getattr(self, "_extractor", None) is None:
-            from .orb_frontend import OrbExtractor
-            self._extractor = OrbExtractor(c.H, c.W, nfeatures=nfeatures, device=self.device)
+            if c.desc_is_f32:
+                from .sift_frontend import SiftExtractor
+                self._extractor = SiftExtractor(c.H, c.W, max_keypoints=max_keypoints, device=self.device)
+            else:
+                from .orb_frontend import OrbExtractor
+                self._extractor = OrbExtractor(c.H, c.W, nfeatures=nfeatures, device=self.device)
         kp, desc, _, count = self._extractor.extract_batch(images, rows=c.n_cap)
         # the kernels read pinned images and depth asynchronously: hold them (a dropped pinned tensor's block is handed to
         # the next pin_memory() and overwritten) until poses() has synchronised; kp / desc / count are device tensors of
@@ -294,7 +304,8 @@ class MultiDeviceLoop:
 
     def lost_frames(self, q):
         """Frames of sequence q pushed by push_images (or vo_seq_push_all_dev) that lost keypoint rows: more keypoints than
-        n_cap, or an extractor flag (a pyramid level overflowed).  Synchronises the stream."""
+        n_cap, or an extractor flag (an ORB pyramid level overflowed, a SIFT raw list passed max_keypoints).  Synchronises
+        the stream."""
         if not 0 <= int(q) < self.n_seqs:
             raise IndexError(f"MultiDeviceLoop: sequence {q} outside [0, {self.n_seqs})")
         out = np.zeros(1, np.int32)

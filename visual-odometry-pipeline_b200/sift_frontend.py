@@ -17,7 +17,7 @@ class SiftExtractor:
     """sift = SiftExtractor(H, W); kp, desc, aux = sift.extract(image_uint8)   (image [H,W] gray or [H,W,3] BGR).
 
     kp [n,2] float32 = KeyPoint.pt, desc [n,128] float32 (0..255), aux [n,4] float32 = (size, angle, response, octave word);
-    rows in OpenCV's order (sorted by x, y, ...; duplicates removed)."""
+    rows in OpenCV's order (sorted by x, y, ...; duplicates removed).  extract_batch runs S images in one call."""
 
     def __init__(self, H, W, max_keypoints=32768, device=None):
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
@@ -49,6 +49,41 @@ class SiftExtractor:
         if raw > self.cap:
             raise VoError(f"vo_sift_extract: {raw} candidates exceed max_keypoints = {self.cap}")
         return self.kp[:n], self.desc[:n], self.aux[:n]
+
+    def extract_batch(self, images, rows=None):
+        """S images in one call of the same kernels as `extract` (vo_sift_extract_batch), with no host read: images uint8
+        torch tensor [S,H,W] (gray) or [S,H,W,3] (BGR), contiguous, on this device or in pinned host memory.  Returns device
+        tensors kp [S,rows,2], desc [S,rows,128], aux [S,rows,4] and count int32 [S,2] = (rows written, flags); image s's
+        first count[s,0] rows are, bit for bit, the first rows `extract` gives for it (the rest are unspecified).  Flag bit
+        0: the raw list passed max_keypoints (where `extract` raises; which keypoints survive is then unspecified); bit 1:
+        rows past `rows` were dropped (the first rows in OpenCV's order, i.e. the left of the image, are kept).  rows
+        defaults to max_keypoints.  Scratch grows to the largest S seen (~117 MB per 1241 x 376 image).  Pinned images are
+        read by the kernels after the call returns: keep them alive and unchanged until the stream has passed this call."""
+        if not isinstance(images, torch.Tensor):
+            raise ValueError("SiftExtractor.extract_batch: images must be a torch tensor")
+        if images.dtype != torch.uint8 or not images.is_contiguous() or not (images.is_cuda or images.is_pinned()):
+            raise ValueError("SiftExtractor.extract_batch: images must be contiguous uint8 on the device or in pinned host memory")
+        if images.is_cuda and images.device != self.device:
+            raise ValueError(f"SiftExtractor.extract_batch: images on {images.device}, extractor on {self.device}")
+        if (images.dim() not in (3, 4) or tuple(images.shape[1:3]) != (self.H, self.W)
+                or (images.dim() == 4 and images.shape[3] != 3) or not 1 <= images.shape[0] <= 65535):
+            raise ValueError(f"SiftExtractor.extract_batch: expected [S,{self.H},{self.W}] or [S,{self.H},{self.W},3] with "
+                             f"1 <= S <= 65535, got {tuple(images.shape)}")
+        S = int(images.shape[0])
+        rows = self.cap if rows is None else int(rows)
+        if rows < 1:
+            raise ValueError(f"SiftExtractor.extract_batch: rows {rows} must be >= 1")
+        kp = torch.empty((S, rows, 2), dtype=torch.float32, device=self.device)
+        desc = torch.empty((S, rows, 128), dtype=torch.float32, device=self.device)
+        aux = torch.empty((S, rows, 4), dtype=torch.float32, device=self.device)
+        count = torch.empty((S, 2), dtype=torch.int32, device=self.device)
+        p = lambda t: ctypes.c_void_p(t.data_ptr())  # noqa: E731
+        with torch.cuda.device(self.device):
+            check(self.ctx.lib.vo_sift_extract_batch(self.handle, p(images), S, 1 if images.dim() == 3 else 3, rows, p(kp),
+                                                     p(desc), p(aux), p(count),
+                                                     ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)),
+                  "vo_sift_extract_batch")
+        return kp, desc, aux, count
 
     def close(self):
         if self.handle:
