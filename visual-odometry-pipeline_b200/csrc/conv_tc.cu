@@ -282,6 +282,9 @@ extern "C" int vo_conv2d(vo_ctx *ctx, const float *x, int H, int W, int cin, con
     using namespace vo;
     VO_REQUIRE(ctx && x && w && scale && shift && out, "vo_conv2d: null argument");
     VO_REQUIRE(H > 0 && W > 0 && k >= 1 && k <= 7 && dil >= 1, "vo_conv2d: bad shape");
+    // the channel checks of conv_tc_launch, repeated here so that a refused call enqueues nothing (no split kernels)
+    VO_REQUIRE(cin % CV_KB == 0 && cin > 0, "vo_conv2d: C_in must be a multiple of 32 (got %d)", cin);
+    VO_REQUIRE(cout == 32 || cout == 64 || cout == 128, "vo_conv2d: C_out must be 32, 64 or 128 (got %d)", cout);
     cudaStream_t st = (cudaStream_t)stream;
     const size_t n_act = (size_t)H * W * cin, n_w = (size_t)cout * k * k * cin;
     float *ws;

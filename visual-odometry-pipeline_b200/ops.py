@@ -181,8 +181,17 @@ def conv2d(x, w, scale, shift, k, dil=1, relu=False):
     """vo_conv2d: x [H,W,Cin] NHWC, w [Cout,k,k,Cin], scale/shift [Cout] (all CUDA float32) -> [H,W,Cout]."""
     for t, name in ((x, "x"), (w, "w"), (scale, "scale"), (shift, "shift")):
         _chk(t, torch.float32, name)
+    if x.dim() != 3:
+        raise ValueError(f"conv2d: x must be [H,W,Cin], got shape {tuple(x.shape)}")
     H, W, cin = x.shape
-    cout = w.shape[0]
+    cout = w.shape[0] if w.dim() > 0 else 0
+    # the weight map is encoded from (C_out, k, C_in) alone: a tensor smaller than that would be read past its end
+    if tuple(w.shape) != (cout, int(k), int(k), cin):
+        raise ValueError(f"conv2d: w must be [Cout,k,k,Cin] = [{cout},{int(k)},{int(k)},{cin}], got {tuple(w.shape)}")
+    if tuple(scale.shape) != (cout,) or tuple(shift.shape) != (cout,):
+        raise ValueError(f"conv2d: scale and shift must be [{cout}], got {tuple(scale.shape)} and {tuple(shift.shape)}")
+    if not (w.device == scale.device == shift.device == x.device):
+        raise ValueError(f"conv2d: tensors on different devices ({x.device}, {w.device}, {scale.device}, {shift.device})")
     out = torch.empty((H, W, cout), dtype=torch.float32, device=x.device)
     ctx = context(x.device)
     with torch.cuda.device(x.device):
